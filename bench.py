@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the IBL bake hot path (BASELINE.json: prefiltered texel-samples/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one GGX-prefilter chain bake of one synthetic HDR environment map
 (BASELINE config 2: 512^2 faces, 8 levels, 1024 samples/texel, rgbe payload as
@@ -29,6 +29,12 @@ HBM copy bandwidth; `cpu_baseline` is the unmodified reference tools/ibl.cpp
       and peer stores).
   C3_one_process (N > 1)  config 3 again through the device-list entry point: rank 0 alone, after the
       other ranks have left, drives all N GPUs from one process (datum_ibl_multi_*), host buffers in and out.
+
+`--dump-outputs DIR` saves what the last of the K timed steps baked, so that two builds can be compared
+output for output: levels 1..7 of its chain (level 0 is the step's input), decoded from the rgbe words to
+float32 RGB, one (6, h, w, 3) array per level as DIR/c2_level<L>.npy (DIR/c2_rank<R>_level<L>.npy with
+N > 1), 6.3 MB per GPU and at most 64 MiB in all: with more than 10 GPUs a fixed, seeded sample of 10 ranks
+saves theirs.  The inputs are seeded, so the same arguments bake the same probe in every run.
 """
 
 import argparse
@@ -50,6 +56,7 @@ FLOP_PER_TEXEL_SAMPLE = 85.0                     # SURVEY.md §8d, itemised in D
 SH9_BYTES_PER_TEXEL = 16.0                       # SURVEY.md §8d: RGBA32F texel read once
 CPU_SAMPLE = (128, 8)                            # CPU legs: one 128^2-face bake with C2's EIGHT levels (the same roughness set) per thread
 SUSTAINED_SECONDS = 2.5
+DUMP_BYTES = 64 * 2**20                          # --dump-outputs, all ranks together
 
 METRIC = "prefiltered texel-samples/sec"
 UNIT = "texel-samples/s"
@@ -574,6 +581,27 @@ def config_c5(job, ctx, engine, stream):
     }
 
 
+def dump_ranks(world):
+    """The ranks whose chains --dump-outputs saves: all while they fit DUMP_BYTES, else a fixed, seeded sample."""
+    per_rank = sum(6 * (WIDTH >> level) ** 2 * 3 * 4 + 128 for level in range(1, LEVELS))   # float32 RGB + .npy header
+    keep = DUMP_BYTES // per_rank
+    return list(range(world)) if world <= keep else sorted(np.random.default_rng(0).choice(world, keep, replace=False).tolist())
+
+
+def dump_outputs(directory, chain, rank, world):
+    """Levels >= 1 of one baked C2 chain (uint32 rgbe words), decoded to float32 RGB, one .npy per level."""
+    import datum_b200
+    import oracle_lib
+
+    os.makedirs(directory, exist_ok=True)
+    offs = datum_b200.level_offsets(WIDTH, WIDTH, LEVELS)
+    prefix = "c2" if world == 1 else "c2_rank%d" % rank
+    for level in range(1, LEVELS):
+        side = WIDTH >> level
+        rgb = oracle_lib.rgbe_decode_array(chain[offs[level]:offs[level + 1]])[:, :3].reshape(6, side, side, 3)
+        np.save(os.path.join(directory, "%s_level%d.npy" % (prefix, level)), np.ascontiguousarray(rgb))
+
+
 def run_ours(args):
     job = Job()
     torch, world, rank, device = job.torch, job.world, job.rank, job.device
@@ -621,6 +649,9 @@ def run_ours(args):
     elapsed_ms = job.max_over_ranks(ev0.elapsed_time(ev1))
     launches = ctx.launch_count - launches_before
     dom_n, dom_ms, dom_ts = ctx.dominant_kernel_stats(reset=True)
+    if args.dump_outputs and rank in dump_ranks(world):
+        last = pool_dev[(args.warmup + args.steps - 1) % POOL].cpu().numpy().view(np.uint32)
+        dump_outputs(args.dump_outputs, last, rank, world)
 
     # ---- end to end through the reference-facing call: pinned host payload in, baked payload out
     def host_loop(payloads):
@@ -806,15 +837,19 @@ def main():
     parser = argparse.ArgumentParser()
     parser.add_argument("--gpus", type=int, default=1)
     parser.add_argument("--steps", type=int, default=None, help="timed steps (default 50; 10 for --impl reference, whose step is ~7 s of CPU work)")
-    parser.add_argument("--warmup", type=int, default=5)
+    parser.add_argument("--warmup", type=int, default=5, help="untimed steps before the timed ones (the GPU arm runs at least 3: first launches load modules and build sample tables)")
     parser.add_argument("--impl", choices=["ours", "reference"], default="ours")
     parser.add_argument("--skip-configs", action="store_true", help="only the C2 headline (development runs)")
     parser.add_argument("--configs-timeout", type=int, default=480, help="seconds the extra configurations may take before the line is printed without them")
+    parser.add_argument("--dump-outputs", metavar="DIR", default=None, help="save the chain levels the last timed step baked as DIR/*.npy (float32)")
     args = parser.parse_args()
     if args.steps is None:
         args.steps = 50 if args.impl == "ours" else 10
+    if args.steps < 1:
+        parser.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        parser.error("--dump-outputs saves the GPU bake; the reference arm has none")
     args.warmup = max(3, args.warmup) if args.impl == "ours" else max(0, args.warmup)
-    args.steps = max(1, args.steps)
 
     if args.impl == "reference":
         return run_reference_arm(args)

@@ -138,7 +138,13 @@ def _gpu_worker(rank, world, port, w, levels, samples, out_dir):
         dist.destroy_process_group()
 
 
-def _two_gpus_split_one_probe_over_nccl(tmp_path, ctx):
+# The NCCL leg needs two distinct GPUs (NCCL refuses two ranks on one device): it skips on a one-GPU box,
+# where the shared-probe machinery is covered by the IPC test below and by tests/test_multi_gpu.py (two
+# contexts on one GPU); every multi-GPU configuration is also run and parity-checked by `bench.py --gpus N`
+# (configs C3, C4, C5 of its JSON line).
+@pytest.mark.gpu
+@pytest.mark.skipif(not torch.cuda.is_available() or torch.cuda.device_count() < 2, reason="needs two GPUs (NCCL refuses two ranks on one device)")
+def test_two_gpus_split_one_probe_over_nccl(tmp_path, ctx):
     w, levels, samples = 256, 9, 256
     mp.spawn(_gpu_worker, args=(2, free_port(), w, levels, samples, str(tmp_path)), nprocs=2, join=True)
 
@@ -221,11 +227,3 @@ def test_two_processes_on_one_gpu_share_a_probe_through_ipc(tmp_path, ctx):
     sh0, sh1 = np.load(tmp_path / "ipc_sh_0.npy"), np.load(tmp_path / "ipc_sh_1.npy")
     assert np.array_equal(sh0, sh1)
     assert np.abs(sh0 - want_sh).max() <= 1e-4 * np.abs(want_sh).max()
-
-
-# The NCCL leg needs two distinct GPUs (NCCL refuses two ranks on one device): it is collected on boxes that
-# have them.  On a one-GPU box the shared-probe machinery is covered by the IPC test above and by
-# tests/test_multi_gpu.py (two contexts on one GPU); every multi-GPU configuration is also run and
-# parity-checked by `bench.py --gpus N` (configs C3, C4, C5 of its JSON line).
-if torch.cuda.is_available() and torch.cuda.device_count() >= 2:
-    test_two_gpus_split_one_probe_over_nccl = pytest.mark.gpu(_two_gpus_split_one_probe_over_nccl)

@@ -21,11 +21,11 @@ pytestmark = pytest.mark.gpu
 
 
 def device_lists():
+    """Lists of several distinct GPUs stay in the suite and skip on a box with fewer."""
+    gpus = torch.cuda.device_count() if torch.cuda.is_available() else 0
     lists = [[0, 0], [0, 0, 0]]
-    if torch.cuda.is_available() and torch.cuda.device_count() >= 2:
-        lists.append([0, 1])
-    if torch.cuda.is_available() and torch.cuda.device_count() >= 4:
-        lists.append([0, 1, 2, 3])
+    for devices in ([0, 1], [0, 1, 2, 3]):
+        lists.append(pytest.param(devices, marks=pytest.mark.skipif(gpus < len(devices), reason="needs %d GPUs" % len(devices))))
     return lists
 
 
