@@ -15,6 +15,7 @@ from .ibl import (  # noqa: F401
     IblError,
     FORMAT_RGBE,
     FORMAT_F32,
+    FORMAT_F16,
     default_context,
     image_datasize,
     image_maxlevels,

@@ -61,6 +61,9 @@ SIGNATURES = {
     "datum_ibl_measure_fp32x2_peak": (c_int, [c_void_p, ctypes.POINTER(ctypes.c_double)]),
     "datum_ibl_dominant_kernel_stats": (c_int, [c_void_p, c_int, ctypes.POINTER(c_int), ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double)]),
     "datum_ibl_last_prefilter_ms": (c_int, [c_void_p, ctypes.POINTER(c_float)]),
+    "datum_ibl_buildmips_cube_float": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
+    "datum_ibl_buildmips_cube_float_device": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "datum_ibl_prefilter_level_float_device": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
 }
 
 

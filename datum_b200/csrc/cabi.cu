@@ -10,6 +10,7 @@
 #include "ibl_math.cuh"
 #include "ibl_tables.h"
 #include "prefilter.h"
+#include "prefilter_f.h"
 #include "sh9.h"
 #include "luts.h"
 #include "resample.h"
@@ -131,6 +132,7 @@ struct datum_ibl_ctx
   void *host_stage = nullptr;     // pinned staging between the device and a caller's PAGEABLE payload
   size_t host_stage_bytes = 0;
   DeviceBuffer<uint4> records;    // quad records of the current source level
+  DeviceBuffer<unsigned char> float_records; // footprint records of the current source level of a float chain (prefilter_f.h)
   std::map<std::pair<int, int>, float*> frames; // source size -> per-texel frames of the destination level (ibl::launch_build_frames)
   size_t frames_bytes = 0, world_frames_bytes = 0;
   std::map<std::pair<int, int>, float*> world_frames; // destination size -> world-space T, B, N per texel (tail kernel; levels of at most kWorldFrameTexels)
@@ -353,6 +355,87 @@ namespace
     return 0;
   }
 
+  // folded frames and sector limits of the destination level of a ws x hs source (proj_usable sizes), kept
+  // per source size: geometry only
+  int level_frames(datum_ibl_ctx *ctx, int ws, int hs, float const **out)
+  {
+    int wd = ws >> 1, hd = hs >> 1;
+
+    auto found = ctx->frames.find(std::make_pair(ws, hs));
+    if (found == ctx->frames.end())
+    {
+      // a process that bakes many different sizes must not collect planes for ever: start over above 1 GiB
+      const size_t bytes = sizeof(float) * ibl::frame_floats(wd, hd);
+      if (ctx->frames_bytes + bytes > ((size_t)1 << 30) && !ctx->frames.empty())
+      {
+        cudaStreamSynchronize(ctx->stream);
+        for(auto &entry : ctx->frames)
+          cudaFree(entry.second);
+        ctx->frames.clear();
+        ctx->frames_bytes = 0;
+      }
+
+      float *built = nullptr;
+      cudaError_t err = cudaMalloc(&built, bytes);
+      if (err == cudaSuccess)
+      {
+        err = ibl::launch_build_frames(built, ws, hs, ctx->quats, ctx->stream);
+        if (err != cudaSuccess)
+          cudaFree(built);
+      }
+      if (err != cudaSuccess)
+        return fail_cuda("build_frames", err);
+      ctx->launches += 1;
+      ctx->frames_bytes += bytes;
+      found = ctx->frames.emplace(std::make_pair(ws, hs), built).first;
+    }
+
+    *out = found->second;
+    return 0;
+  }
+
+  // world-space frames of a wd x hd destination level (tail kernels), kept per size; null for levels above
+  // kWorldFrameTexels (the tail kernel then computes a frame per CTA)
+  int level_world_frames(datum_ibl_ctx *ctx, int wd, int hd, float const **out)
+  {
+    *out = nullptr;
+    const size_t kWorldFrameTexels = (size_t)1 << 20;
+    if ((size_t)6 * wd * hd > kWorldFrameTexels)
+      return 0;
+
+    auto found = ctx->world_frames.find(std::make_pair(wd, hd));
+    if (found == ctx->world_frames.end())
+    {
+      // the same bound as for the pair kernel's planes: start over above 256 MiB
+      const size_t bytes = sizeof(float) * (size_t)ibl::kWorldFrameFloats * 6 * wd * hd;
+      if (ctx->world_frames_bytes + bytes > ((size_t)1 << 28) && !ctx->world_frames.empty())
+      {
+        cudaStreamSynchronize(ctx->stream);
+        for(auto &entry : ctx->world_frames)
+          cudaFree(entry.second);
+        ctx->world_frames.clear();
+        ctx->world_frames_bytes = 0;
+      }
+
+      float *built = nullptr;
+      cudaError_t err = cudaMalloc(&built, bytes);
+      if (err == cudaSuccess)
+      {
+        err = ibl::launch_build_world_frames(built, wd, hd, ctx->quats, ctx->stream);
+        if (err != cudaSuccess)
+          cudaFree(built);
+      }
+      if (err != cudaSuccess)
+        return fail_cuda("build_world_frames", err);
+      ctx->launches += 1;
+      ctx->world_frames_bytes += bytes;
+      found = ctx->world_frames.emplace(std::make_pair(wd, hd), built).first;
+    }
+
+    *out = found->second;
+    return 0;
+  }
+
   // slabs of more than kTailTexels texels of a level at least a tile wide: denormal-mantissa kernels (prefilter_dn.cu)
   int run_level_dn(datum_ibl_ctx *ctx, uint32_t const *d_src, int ws, int hs, DeviceTable const &table, int row_begin, int row_end, uint32_t *d_dst_words, float *d_dst_f32, bool record_dominant, PeerTargets const &peers, Batch const &batch)
   {
@@ -371,38 +454,8 @@ namespace
 
     // frames of the destination level: geometry only, computed on first use of a source size
     float const *frames = nullptr;
-    if (ibl::proj_usable(ws, hs))
-    {
-      auto found = ctx->frames.find(std::make_pair(ws, hs));
-      if (found == ctx->frames.end())
-      {
-        // a process that bakes many different sizes must not collect planes for ever: start over above 1 GiB
-        const size_t bytes = sizeof(float) * ibl::frame_floats(wd, hd);
-        if (ctx->frames_bytes + bytes > ((size_t)1 << 30) && !ctx->frames.empty())
-        {
-          cudaStreamSynchronize(ctx->stream);
-          for(auto &entry : ctx->frames)
-            cudaFree(entry.second);
-          ctx->frames.clear();
-          ctx->frames_bytes = 0;
-        }
-
-        float *built = nullptr;
-        err = cudaMalloc(&built, bytes);
-        if (err == cudaSuccess)
-        {
-          err = ibl::launch_build_frames(built, ws, hs, ctx->quats, ctx->stream);
-          if (err != cudaSuccess)
-            cudaFree(built);
-        }
-        if (err != cudaSuccess)
-          return fail_cuda("build_frames", err);
-        ctx->launches += 1;
-        ctx->frames_bytes += bytes;
-        found = ctx->frames.emplace(std::make_pair(ws, hs), built).first;
-      }
-      frames = found->second;
-    }
+    if (ibl::proj_usable(ws, hs) && level_frames(ctx, ws, hs, &frames))
+      return 1;
 
     ibl::PrefilterDnParams p = {};
     p.frames = frames;
@@ -478,39 +531,8 @@ namespace
       // world-space frames of the destination level: geometry only, kept per size (small levels only:
       // this kernel runs slabs of at most kTailTexels texels, a bigger level is a shared probe's)
       float const *world_frames = nullptr;
-      const size_t kWorldFrameTexels = (size_t)1 << 20;
-      if ((size_t)6 * wd * hd <= kWorldFrameTexels)
-      {
-        auto found = ctx->world_frames.find(std::make_pair(wd, hd));
-        if (found == ctx->world_frames.end())
-        {
-          // the same bound as for the pair kernel's planes: start over above 256 MiB
-          const size_t bytes = sizeof(float) * (size_t)ibl::kWorldFrameFloats * 6 * wd * hd;
-          if (ctx->world_frames_bytes + bytes > ((size_t)1 << 28) && !ctx->world_frames.empty())
-          {
-            cudaStreamSynchronize(ctx->stream);
-            for(auto &entry : ctx->world_frames)
-              cudaFree(entry.second);
-            ctx->world_frames.clear();
-            ctx->world_frames_bytes = 0;
-          }
-
-          float *built = nullptr;
-          cudaError_t err = cudaMalloc(&built, bytes);
-          if (err == cudaSuccess)
-          {
-            err = ibl::launch_build_world_frames(built, wd, hd, ctx->quats, ctx->stream);
-            if (err != cudaSuccess)
-              cudaFree(built);
-          }
-          if (err != cudaSuccess)
-            return fail_cuda("build_world_frames", err);
-          ctx->launches += 1;
-          ctx->world_frames_bytes += bytes;
-          found = ctx->world_frames.emplace(std::make_pair(wd, hd), built).first;
-        }
-        world_frames = found->second;
-      }
+      if (level_world_frames(ctx, wd, hd, &world_frames))
+        return 1;
 
       ibl::PrefilterTailParams p = {};
       p.src = d_src;
@@ -935,6 +957,134 @@ namespace
 
 namespace
 {
+  // ---- float chains: RGBA16F / RGBA32F levels, no rgbe re-quantisation (prefilter_f.cu) ----
+
+  bool float_format(int format)
+  {
+    return format == DATUM_IBL_FORMAT_F32 || format == DATUM_IBL_FORMAT_F16;
+  }
+
+  // the input range of the float kernels holds up to this many samples (prefilter_f.h, kFloatChainMaxRadiance)
+  const int kFloatMaxSamples = 4096;
+
+  // one level of a float chain on the context's stream.  The pair kernel takes slabs above kTailTexels of
+  // levels at least a tile wide whose source it can address (proj_usable); everything else runs the tail kernel.
+  int run_level_float(datum_ibl_ctx *ctx, int format, void const *d_src, int ws, int hs, DeviceTable const &table, int row_begin, int row_end, void *d_dst, float *d_dst_f32, bool record_dominant)
+  {
+    int wd = ws >> 1, hd = hs >> 1;
+
+    if (ws < 2 || hs < 2)
+      return fail("prefilter: source level must be at least 2x2");
+    if (row_begin < 0 || row_end > 6 * hd || row_begin > row_end)
+      return fail("prefilter: row range outside the destination level");
+    if (row_begin == row_end)
+      return 0;
+
+    ibl::PrefilterFloatParams p = {};
+    p.format = format;
+    p.src = d_src;
+    p.table = table.d_banded;
+    p.table_proj = table.d_banded_proj;
+    for(int i = 0; i < 2; ++i)
+    {
+      p.table_sector[i] = table.d_sector[i];
+      p.sector_rho[i] = table.d_sector_rho[i];
+      p.sector_bands[i] = table.sector_bands[i];
+    }
+    p.table_count = table.count;
+    p.dst = d_dst;
+    p.dst_f32 = d_dst_f32;
+    p.wd = wd;
+    p.hd = hd;
+    p.row_begin = row_begin;
+    p.row_end = row_end;
+    p.geom = ibl::make_level_geom(ws, hs);
+    for(int f = 0; f < 6; ++f)
+      p.quats[f] = ctx->quats[f];
+    p.norm = ibl::float_chain_norm(table.total_weight);
+
+    const bool tail = (size_t)(row_end - row_begin) * wd <= (size_t)ibl::kTailTexels || wd < 8 || !ibl::proj_usable(ws, hs);
+    cudaError_t err = cudaSuccess;
+
+    if (tail)
+    {
+      if (level_world_frames(ctx, wd, hd, &p.world_frames))
+        return 1;
+    }
+    else
+    {
+      const size_t record_bytes = format == DATUM_IBL_FORMAT_F16 ? sizeof(ibl::F16Record) : sizeof(ibl::F32Record);
+      err = ctx->float_records.reserve((size_t)6 * ws * hs * record_bytes);
+      if (err == cudaSuccess)
+        err = ctx->queue_heads.reserve((size_t)ctx->sm_count + 1);
+      if (err != cudaSuccess)
+        return fail_cuda("cudaMalloc(float records)", err);
+
+      err = ibl::launch_build_float_records(format, d_src, ctx->float_records.ptr, ws, hs, ctx->queue_heads.ptr, ctx->sm_count + 1, ctx->sm_count, ctx->stream);
+      if (err != cudaSuccess)
+        return fail_cuda("build_float_records", err);
+      ctx->launches += 1;
+
+      if (level_frames(ctx, ws, hs, &p.frames))
+        return 1;
+      p.records = ctx->float_records.ptr;
+      p.counters = ctx->queue_heads.ptr;
+    }
+
+    int slot = record_dominant ? begin_dominant(ctx, (double)(row_end - row_begin) * wd * (double)table.samples) : -1;
+
+    err = tail ? ibl::launch_prefilter_float_tail(p, ctx->stream) : ibl::launch_prefilter_float(p, ctx->sm_count, ctx->stream);
+    if (err != cudaSuccess)
+      return fail_cuda(("prefilter_float (source " + std::to_string(ws) + "x" + std::to_string(hs) + ", rows " + std::to_string(row_begin) + ".." + std::to_string(row_end) + ")").c_str(), err);
+    ctx->launches += 1;
+
+    if (slot >= 0)
+      cudaEventRecord(ctx->ring_end[slot], ctx->stream);
+
+    return 0;
+  }
+
+  // tools/ibl.cpp:247-278 on a float chain: level L from level L-1 as stored in the chain
+  int run_chain_float(datum_ibl_ctx *ctx, int format, int width, int height, int levels, int samples, unsigned char *d_chain, float *d_f32)
+  {
+    std::vector<DeviceTable> *tables = nullptr;
+    if (get_tables(ctx, levels, samples, &tables))
+      return 1;
+
+    const size_t texel = (size_t)ibl::float_texel_bytes(format);
+
+    cudaEventRecord(ctx->ev_begin, ctx->stream);
+
+    unsigned char *src = d_chain;
+    unsigned char *dst = src + (size_t)width * height * 6 * texel;
+
+    for(int level = 1; level < levels; ++level)
+    {
+      int hd = height >> 1;
+
+      if (run_level_float(ctx, format, src, width, height, (*tables)[level], 0, 6 * hd, dst, d_f32, level == 1))
+        return 1;
+
+      size_t outcount = (size_t)(width >> 1) * hd * 6;
+
+      src += (size_t)width * height * 6 * texel;
+      dst += outcount * texel;
+      if (d_f32)
+        d_f32 += 3 * outcount;
+
+      width /= 2;
+      height /= 2;
+    }
+
+    cudaEventRecord(ctx->ev_end, ctx->stream);
+    ctx->timed = true;
+
+    return 0;
+  }
+}
+
+namespace
+{
   // Level 0 is already in ctx->chain (six-image ingest, equirect pack): send it home at once — it travels
   // under the level-1 kernels — then the chain with every level following as soon as it is complete.
   // `bits` receives the whole payload; pageable payloads go through the pinned staging.
@@ -1130,6 +1280,7 @@ extern "C"
     if (ctx->host_stage)
       cudaFreeHost(ctx->host_stage);
     ctx->records.release();
+    ctx->float_records.release();
     for(auto &entry : ctx->frames)
       cudaFree(entry.second);
     ctx->frames.clear();
@@ -1483,6 +1634,97 @@ extern "C"
     return run_level(ctx, d_src, ws, hs, (*tables)[level], row_begin, row_end, d_dst_words, d_dst_f32);
   }
 
+  int datum_ibl_buildmips_cube_float_device(datum_ibl_ctx *ctx, int format, int width, int height, int levels, int samples, void *d_chain, float *d_f32)
+  {
+    if (!ctx || !d_chain)
+      return fail("datum_ibl_buildmips_cube_float_device: null argument");
+    if (!float_format(format))
+      return fail("datum_ibl_buildmips_cube_float_device: unknown format " + std::to_string(format) + " (DATUM_IBL_FORMAT_F32 or DATUM_IBL_FORMAT_F16)");
+    if (!valid_chain(width, height, levels) || samples < 1 || samples > kFloatMaxSamples)
+      return fail("datum_ibl_buildmips_cube_float_device: bad width/height/levels/samples");
+    if (reinterpret_cast<uintptr_t>(d_chain) % ibl::float_texel_bytes(format) != 0 || reinterpret_cast<uintptr_t>(d_f32) % sizeof(float) != 0)
+      return fail("datum_ibl_buildmips_cube_float_device: misaligned chain or d_f32");
+
+    DeviceGuard guard(ctx->device);
+    return run_chain_float(ctx, format, width, height, levels, samples, static_cast<unsigned char*>(d_chain), d_f32);
+  }
+
+  int datum_ibl_buildmips_cube_float(datum_ibl_ctx *ctx, int format, int width, int height, int levels, int samples, void *chain)
+  {
+    if (!ctx || !chain)
+      return fail("datum_ibl_buildmips_cube_float: null argument");
+    if (!float_format(format))
+      return fail("datum_ibl_buildmips_cube_float: unknown format " + std::to_string(format) + " (DATUM_IBL_FORMAT_F32 or DATUM_IBL_FORMAT_F16)");
+    if (!valid_chain(width, height, levels) || samples < 1 || samples > kFloatMaxSamples)
+      return fail("datum_ibl_buildmips_cube_float: bad width/height/levels/samples");
+
+    DeviceGuard guard(ctx->device);
+
+    const size_t texel = (size_t)ibl::float_texel_bytes(format);
+    const size_t bytes = datum_ibl_chain_bytes(width, height, levels) / sizeof(uint32_t) * texel;
+    const size_t level0 = (size_t)width * height * 6 * texel;
+
+    cudaError_t err = ctx->staging.reserve(bytes);
+    if (err != cudaSuccess)
+      return fail_cuda("cudaMalloc(chain)", err);
+
+    // a pageable chain goes through the context's pinned staging
+    const bool pinned = host_is_pinned(chain);
+    if (!pinned && reserve_host_stage(ctx, bytes))
+      return 1;
+
+    unsigned char *host = pinned ? static_cast<unsigned char*>(chain) : static_cast<unsigned char*>(ctx->host_stage);
+
+    err = upload_host(ctx, ctx->staging.ptr, chain, level0, pinned, ctx->host_stage);
+    if (err != cudaSuccess)
+    {
+      cudaStreamSynchronize(ctx->stream);
+      return fail_cuda("cudaMemcpyAsync(level 0)", err);
+    }
+
+    int failed = run_chain_float(ctx, format, width, height, levels, samples, ctx->staging.ptr, nullptr);
+
+    if (!failed && bytes > level0)
+    {
+      err = cudaMemcpyAsync(host + level0, ctx->staging.ptr + level0, bytes - level0, cudaMemcpyDeviceToHost, ctx->stream);
+      if (err != cudaSuccess)
+        failed = fail_cuda("cudaMemcpyAsync(levels)", err);
+    }
+
+    // also after a failure: nothing may stay in flight that reads or writes the caller's chain
+    err = cudaStreamSynchronize(ctx->stream);
+    if (failed)
+      return 1;
+    if (err != cudaSuccess)
+      return fail_cuda("datum_ibl_buildmips_cube_float", err);
+
+    if (!pinned && bytes > level0)
+      copy_parallel(static_cast<unsigned char*>(chain) + level0, host + level0, bytes - level0);
+
+    return 0;
+  }
+
+  int datum_ibl_prefilter_level_float_device(datum_ibl_ctx *ctx, int format, void const *d_src, int ws, int hs, int level, int levels, int samples, int row_begin, int row_end, void *d_dst, float *d_dst_f32)
+  {
+    if (!ctx || !d_src || !d_dst)
+      return fail("datum_ibl_prefilter_level_float_device: null argument");
+    if (!float_format(format))
+      return fail("datum_ibl_prefilter_level_float_device: unknown format " + std::to_string(format) + " (DATUM_IBL_FORMAT_F32 or DATUM_IBL_FORMAT_F16)");
+    if (levels < 2 || levels > 16 || level < 1 || level >= levels || samples < 1 || samples > kFloatMaxSamples)
+      return fail("datum_ibl_prefilter_level_float_device: bad level/levels/samples");
+    const uintptr_t align = (uintptr_t)ibl::float_texel_bytes(format);
+    if (reinterpret_cast<uintptr_t>(d_src) % align != 0 || reinterpret_cast<uintptr_t>(d_dst) % align != 0 || reinterpret_cast<uintptr_t>(d_dst_f32) % sizeof(float) != 0)
+      return fail("datum_ibl_prefilter_level_float_device: misaligned source, destination or d_dst_f32");
+
+    DeviceGuard guard(ctx->device);
+
+    std::vector<DeviceTable> *tables = nullptr;
+    if (get_tables(ctx, levels, samples, &tables))
+      return 1;
+
+    return run_level_float(ctx, format, d_src, ws, hs, (*tables)[level], row_begin, row_end, d_dst, d_dst_f32, false);
+  }
+
   int datum_ibl_prefilter_level_peers(datum_ibl_ctx *ctx, uint32_t const *d_src, int ws, int hs, int level, int levels, int samples, int row_begin, int row_end, int rank, int world, uint32_t *const *d_dst_words, uint32_t *const *d_flags, uint32_t epoch)
   {
     if (!ctx || !d_src || !d_dst_words)
@@ -1675,7 +1917,7 @@ extern "C"
   {
     if (!ctx || !d_level0 || !d_partial)
       return fail("datum_ibl_sh9_partial_device: null argument");
-    if (width < 1 || height < 1 || (format != DATUM_IBL_FORMAT_RGBE && format != DATUM_IBL_FORMAT_F32))
+    if (width < 1 || height < 1 || (format != DATUM_IBL_FORMAT_RGBE && format != DATUM_IBL_FORMAT_F32 && format != DATUM_IBL_FORMAT_F16))
       return fail("datum_ibl_sh9_partial_device: bad width/height/format");
     if (row_begin < 0 || row_end > 6 * height || row_begin > row_end)
       return fail("datum_ibl_sh9_partial_device: row range outside the cube");
@@ -1689,7 +1931,7 @@ extern "C"
   {
     if (!ctx || !d_level0 || !d_slots)
       return fail("datum_ibl_sh9_partial_peers: null argument");
-    if (width < 1 || height < 1 || (format != DATUM_IBL_FORMAT_RGBE && format != DATUM_IBL_FORMAT_F32))
+    if (width < 1 || height < 1 || (format != DATUM_IBL_FORMAT_RGBE && format != DATUM_IBL_FORMAT_F32 && format != DATUM_IBL_FORMAT_F16))
       return fail("datum_ibl_sh9_partial_peers: bad width/height/format");
     if (row_begin < 0 || row_end > 6 * height || row_begin > row_end)
       return fail("datum_ibl_sh9_partial_peers: row range outside the cube");
@@ -1731,12 +1973,12 @@ extern "C"
   {
     if (!ctx || !level0 || !sh)
       return fail("datum_ibl_project_sh9: null argument");
-    if (width < 1 || height < 1 || (format != DATUM_IBL_FORMAT_RGBE && format != DATUM_IBL_FORMAT_F32))
+    if (width < 1 || height < 1 || (format != DATUM_IBL_FORMAT_RGBE && format != DATUM_IBL_FORMAT_F32 && format != DATUM_IBL_FORMAT_F16))
       return fail("datum_ibl_project_sh9: bad width/height/format");
 
     DeviceGuard guard(ctx->device);
 
-    size_t bytes = (size_t)6 * width * height * (format == DATUM_IBL_FORMAT_RGBE ? 4 : 16);
+    size_t bytes = (size_t)6 * width * height * (format == DATUM_IBL_FORMAT_RGBE ? 4 : (format == DATUM_IBL_FORMAT_F16 ? 8 : 16));
 
     cudaError_t err = ctx->staging.reserve(bytes + 28 * sizeof(double));
     if (err != cudaSuccess)

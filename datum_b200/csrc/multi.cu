@@ -384,7 +384,7 @@ extern "C"
   {
     if (!m || !level0 || !sh)
       return fail("datum_ibl_multi_project_sh9: null argument");
-    if (width < 1 || height < 1 || (format != DATUM_IBL_FORMAT_RGBE && format != DATUM_IBL_FORMAT_F32))
+    if (width < 1 || height < 1 || (format != DATUM_IBL_FORMAT_RGBE && format != DATUM_IBL_FORMAT_F32 && format != DATUM_IBL_FORMAT_F16))
       return fail("datum_ibl_multi_project_sh9: bad width/height/format");
 
     const int world = (int)m->devices.size();
@@ -392,7 +392,7 @@ extern "C"
     if (world == 1)
       return datum_ibl_project_sh9(m->ctx[0], level0, format, width, height, sh);
 
-    const size_t texel = format == DATUM_IBL_FORMAT_RGBE ? 4 : 16;
+    const size_t texel = format == DATUM_IBL_FORMAT_RGBE ? 4 : (format == DATUM_IBL_FORMAT_F16 ? 8 : 16);
     const size_t cube_bytes = (size_t)6 * width * height * texel;
     const int rows = 6 * height;
 

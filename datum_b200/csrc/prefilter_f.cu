@@ -1,0 +1,757 @@
+// datum_b200 — GGX prefilter of one level of a FLOAT cube chain, RGBA16F or RGBA32F (sm_100a).
+//
+// The same level arithmetic as prefilter_dn.cu (tools/ibl.cpp:160-187, 247-278 with the non-seamless
+// per-face bilinear Sampler of ibl.cpp:34-88), but a tap is read as the float value the chain stores
+// instead of through rgbe_decode, and a level is stored as floats: no 9-bit re-quantisation between
+// levels.  Two kernels:
+//
+//   * prefilter_float_pair_kernel: the projective pair kernel of prefilter_dn.cu (prefilter_dp_kernel,
+//     PROJ) with the same sector tables, frame planes, 8x4 tiles and per-SM tile queues.  A lane's
+//     footprint comes from a record of the source level (prefilter_f.h): RGBA16F texels verbatim (32 B)
+//     or rgb fp32 (48 B).  The rgbe tap decode is replaced by half -> fp32 conversion (F16) or nothing
+//     (F32); weights stay fp32, so every tap product is the reference's up to summation order.
+//   * prefilter_float_tail_kernel: one CTA per texel, lanes are samples (prefilter_tail_kernel), the four
+//     texels of a footprint read straight from the source level.  Small slabs, levels narrower than a
+//     tile, and every source the pair kernel cannot address (!proj_usable: odd sizes, faces above 2048^2).
+//
+// The device helpers below restate those of prefilter_dn.cu instead of sharing them: the rgbe kernels
+// are sensitive to everything compiled into their bodies (DESIGN.md §4.1), and they stay untouched.
+
+#include "prefilter.h"
+#include "prefilter_f.h"
+#include "ibl_math.cuh"
+
+#include <cuda_runtime.h>
+
+namespace ibl
+{
+  namespace
+  {
+    typedef unsigned long long f32x2;
+
+    __device__ __forceinline__ f32x2 pack2(float lo, float hi) { f32x2 r; asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi)); return r; }
+    __device__ __forceinline__ void unpack2(f32x2 a, float &lo, float &hi) { asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(a)); }
+    __device__ __forceinline__ f32x2 fma2(f32x2 a, f32x2 b, f32x2 c) { f32x2 d; asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c)); return d; }
+    __device__ __forceinline__ f32x2 mul2(f32x2 a, f32x2 b) { f32x2 d; asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
+    __device__ __forceinline__ f32x2 add2(f32x2 a, f32x2 b) { f32x2 d; asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
+    __device__ __forceinline__ f32x2 bcast2(float v) { return pack2(v, v); }
+
+    __device__ __forceinline__ f32x2 neg2(f32x2 a)
+    {
+      float lo, hi;
+      unpack2(a, lo, hi);
+      return pack2(-lo, -hi);
+    }
+
+    template<int FMT> struct RecordOf { typedef F32Record type; };
+    template<> struct RecordOf<kFloatFormatF16> { typedef F16Record type; };
+
+    // a record pointer the compiler cannot re-associate: the index goes into one IMAD.WIDE
+    template<typename R>
+    __device__ __forceinline__ R const *opaque(R const *ptr)
+    {
+      asm volatile("" : "+l"(ptr));
+      return ptr;
+    }
+
+    // ---- records --------------------------------------------------------------------------
+
+    template<int FMT>
+    __global__ void __launch_bounds__(256) build_float_records_kernel(void const *__restrict__ src, void *__restrict__ rec, int ws, int hs, int *__restrict__ counters, int ncounters)
+    {
+      // the prefilter launch that follows on the stream takes its tiles from these queues
+      if (blockIdx.x == 0)
+        for(int i = threadIdx.x; i < ncounters; i += blockDim.x)
+          counters[i] = 0;
+
+      const uint32_t level = 6u * (uint32_t)ws * (uint32_t)hs;
+
+      for(uint32_t idx = blockIdx.x * blockDim.x + threadIdx.x; idx < level; idx += gridDim.x * blockDim.x)
+      {
+        uint32_t i = idx % (uint32_t)ws;
+        uint32_t j = (idx / (uint32_t)ws) % (uint32_t)hs;
+        uint32_t right = (i + 1 < (uint32_t)ws) ? 1u : 0u;
+        uint32_t down = (j + 1 < (uint32_t)hs) ? (uint32_t)ws : 0u;
+        const uint32_t tap[4] = { idx, idx + right, idx + down, idx + down + right };
+
+        if (FMT == kFloatFormatF16)
+        {
+          uint2 const *s = reinterpret_cast<uint2 const*>(src);
+          uint2 t0 = __ldg(s + tap[0]), t1 = __ldg(s + tap[1]), t2 = __ldg(s + tap[2]), t3 = __ldg(s + tap[3]);
+          uint4 *r = reinterpret_cast<uint4*>(rec) + 2 * (size_t)idx;
+          r[0] = make_uint4(t0.x, t0.y, t1.x, t1.y);
+          r[1] = make_uint4(t2.x, t2.y, t3.x, t3.y);
+        }
+        else
+        {
+          float4 const *s = reinterpret_cast<float4 const*>(src);
+          float4 t0 = __ldg(s + tap[0]), t1 = __ldg(s + tap[1]), t2 = __ldg(s + tap[2]), t3 = __ldg(s + tap[3]);
+          float4 *r = reinterpret_cast<float4*>(rec) + 3 * (size_t)idx;
+          r[0] = make_float4(t0.x, t0.y, t0.z, t1.x);
+          r[1] = make_float4(t1.y, t1.z, t2.x, t2.y);
+          r[2] = make_float4(t2.z, t3.x, t3.y, t3.z);
+        }
+      }
+    }
+
+    // ---- taps -----------------------------------------------------------------------------
+
+    // the four texels' rgb of a footprint record: c[k][channel]
+    __device__ __forceinline__ void load_footprint(F16Record const *rec, float c[4][3])
+    {
+      uint4 const *q = reinterpret_cast<uint4 const*>(rec);
+      uint4 lo = __ldg(q), hi = __ldg(q + 1);
+      const uint32_t w[8] = { lo.x, lo.y, lo.z, lo.w, hi.x, hi.y, hi.z, hi.w };
+      #pragma unroll
+      for(int k = 0; k < 4; ++k)
+      {
+        c[k][0] = half_to_float(w[2*k] & 0xFFFFu);
+        c[k][1] = half_to_float(w[2*k] >> 16);
+        c[k][2] = half_to_float(w[2*k + 1] & 0xFFFFu);
+      }
+    }
+
+    __device__ __forceinline__ void load_footprint(F32Record const *rec, float c[4][3])
+    {
+      float4 const *q = reinterpret_cast<float4 const*>(rec);
+      float4 a = __ldg(q), b = __ldg(q + 1), d = __ldg(q + 2);
+      c[0][0] = a.x; c[0][1] = a.y; c[0][2] = a.z;
+      c[1][0] = a.w; c[1][1] = b.x; c[1][2] = b.y;
+      c[2][0] = b.z; c[2][1] = b.w; c[2][2] = d.x;
+      c[3][0] = d.y; c[3][1] = d.z; c[3][2] = d.w;
+    }
+
+    // one texel of the source level itself (tail kernel)
+    template<int FMT>
+    __device__ __forceinline__ void load_texel(void const *src, uint32_t idx, float c[3])
+    {
+      if (FMT == kFloatFormatF16)
+      {
+        uint2 t = __ldg(reinterpret_cast<uint2 const*>(src) + idx);
+        c[0] = half_to_float(t.x & 0xFFFFu);
+        c[1] = half_to_float(t.x >> 16);
+        c[2] = half_to_float(t.y & 0xFFFFu);
+      }
+      else
+      {
+        float4 t = __ldg(reinterpret_cast<float4 const*>(src) + idx);
+        c[0] = t.x; c[1] = t.y; c[2] = t.z;
+      }
+    }
+
+    struct Sums
+    {
+      f32x2 rg, bb;       // (r, g) and the b sums of the two samples of a pair
+    };
+
+    struct PairEntry
+    {
+      f32x2 lx, ly, lz, wh;   // each: (sample a, sample b)
+    };
+
+    template<bool SMEM_TABLE>
+    __device__ __forceinline__ PairEntry load_pair(float4 const *t)
+    {
+      ulonglong2 const *q = reinterpret_cast<ulonglong2 const*>(t);
+      ulonglong2 lo = SMEM_TABLE ? q[0] : __ldg(q);
+      ulonglong2 hi = SMEM_TABLE ? q[1] : __ldg(q + 1);
+      return PairEntry{ lo.x, lo.y, hi.x, hi.y };
+    }
+
+    struct Frame
+    {
+      Vec3f T, B, N;
+    };
+
+    __device__ __forceinline__ void direction_pair_proj(Frame const &t, PairEntry const &e, f32x2 &x, f32x2 &y, f32x2 &z)
+    {
+      x = fma2(e.lx, bcast2(t.T.x), fma2(e.ly, bcast2(t.B.x), bcast2(t.N.x)));
+      y = fma2(e.lx, bcast2(t.T.y), fma2(e.ly, bcast2(t.B.y), bcast2(t.N.y)));
+      z = fma2(e.lx, bcast2(t.T.z), fma2(e.ly, bcast2(t.B.z), bcast2(t.N.z)));
+    }
+
+    // idx = raw index bits of both samples (what `base` has been moved back by), du/dv = fraction - 0.5;
+    // the weights of footprint_weights_diff (ibl.cpp:40 times the sample weight), taps as floats
+    template<typename R>
+    __device__ __forceinline__ void gather_pair(R const *base, uint32_t idx_a, uint32_t idx_b, f32x2 du, f32x2 dv, PairEntry const &e, Sums &acc)
+    {
+      float ca[4][3], cb[4][3];
+      load_footprint(base + idx_a, ca);
+      load_footprint(base + idx_b, cb);
+
+      f32x2 u0 = add2(neg2(du), bcast2(0.5f));
+      f32x2 v0 = fma2(neg2(dv), e.lz, e.wh);
+      f32x2 v1 = fma2(dv, e.lz, e.wh);
+      f32x2 p00 = mul2(u0, v0);
+      f32x2 p01 = mul2(u0, v1);
+
+      float wa[4], wb[4];
+      unpack2(p00, wa[0], wb[0]);
+      unpack2(add2(v0, neg2(p00)), wa[1], wb[1]);
+      unpack2(p01, wa[2], wb[2]);
+      unpack2(add2(v1, neg2(p01)), wa[3], wb[3]);
+
+      #pragma unroll
+      for(int k = 0; k < 4; ++k)
+      {
+        acc.rg = fma2(pack2(ca[k][0], ca[k][1]), bcast2(wa[k]), acc.rg);
+        acc.rg = fma2(pack2(cb[k][0], cb[k][1]), bcast2(wb[k]), acc.rg);
+        acc.bb = fma2(pack2(ca[k][2], cb[k][2]), pack2(wa[k], wb[k]), acc.bb);
+      }
+    }
+
+    // frame rows face-local and folded; `base` = records of the texel's face, moved back by kMagicBits
+    template<typename R>
+    __device__ __forceinline__ void pair_same_face(PrefilterFloatParams const &p, Frame const &t, R const *base, PairEntry const &e, Sums &acc)
+    {
+      f32x2 la, lb, lm;
+      direction_pair_proj(t, e, la, lb, lm);
+
+      float ma, mb;
+      unpack2(lm, ma, mb);
+      f32x2 r = pack2(rcp_fast(ma), rcp_fast(mb));
+
+      f32x2 mu = fma2(la, r, bcast2(kMagic));
+      f32x2 mv = fma2(lb, r, bcast2(kMagic));
+      f32x2 niu = add2(neg2(mu), bcast2(kMagic));
+      f32x2 niv = add2(neg2(mv), bcast2(kMagic));
+      f32x2 du = fma2(la, r, niu);
+      f32x2 dv = fma2(lb, r, niv);
+
+      float ia, ib;
+      unpack2(fma2(niv, bcast2(p.geom.neg_ws), mu), ia, ib);
+
+      gather_pair(base, f2u(ia), f2u(ib), du, dv, e, acc);
+    }
+
+    // frame rows in world coordinates; `base` = records moved back by geom.bias_general
+    template<typename R>
+    __device__ __forceinline__ void pair_general(PrefilterFloatParams const &p, Frame const &t, R const *base, PairEntry const &e, Sums &acc)
+    {
+      f32x2 x, y, z;
+      direction_pair_proj(t, e, x, y, z);
+
+      float xa, xb, ya, yb, za, zb;
+      unpack2(x, xa, xb);
+      unpack2(y, ya, yb);
+      unpack2(z, za, zb);
+
+      float qua, qva, qub, qvb;
+      uint32_t fa, fb;
+      cube_select_unshrunk(xa, ya, za, qua, qva, fa);
+      cube_select_unshrunk(xb, yb, zb, qub, qvb, fb);
+
+      f32x2 qu = pack2(qua, qub), qv = pack2(qva, qvb);
+      f32x2 mu = fma2(qu, bcast2(p.geom.hw_shrunk), bcast2(p.geom.hwm_magic));
+      f32x2 mv = fma2(qv, bcast2(p.geom.hh_shrunk), bcast2(p.geom.hhm_magic));
+      f32x2 cu = add2(neg2(mu), bcast2(p.geom.hwm_magic));
+      f32x2 cv = add2(neg2(mv), bcast2(p.geom.hhm_magic));
+      f32x2 du = fma2(qu, bcast2(p.geom.hw_shrunk), cu);
+      f32x2 dv = fma2(qv, bcast2(p.geom.hh_shrunk), cv);
+
+      float ia, ib;
+      unpack2(fma2(cv, bcast2(p.geom.neg_ws), mu), ia, ib);
+
+      gather_pair(base, fa * p.geom.face_size + f2u(ia), fb * p.geom.face_size + f2u(ib), du, dv, e, acc);
+    }
+
+    // ---- tiles (prefilter_dn.cu: steal_tile, next_tile_plain, tile_texel) -------------------------------
+
+    __device__ __noinline__ int steal_tile(int *counters, int queues, int chunk, uint32_t smid, int lane)
+    {
+      const int own = (int)(smid % (uint32_t)queues);
+
+      for(int base = 1; base < queues; base += 32)
+      {
+        int i = base + lane;
+        int q = own + i;
+        if (q >= queues)
+          q -= queues;
+
+        bool holds = i < queues && *(volatile int const *)(counters + q) < chunk;
+
+        for(unsigned candidates = __ballot_sync(0xffffffffu, holds); candidates != 0u; candidates &= candidates - 1u)
+        {
+          int src = __ffs(candidates) - 1;
+          int k = -1;
+          if (lane == src)
+            k = atomicAdd(counters + q, 1);
+          k = __shfl_sync(0xffffffffu, k, src);
+
+          if (k < chunk)
+            return __shfl_sync(0xffffffffu, q, src) * chunk + k;
+        }
+      }
+
+      return -1;
+    }
+
+    __device__ __forceinline__ int next_tile_plain(PrefilterFloatParams const &p, uint32_t smid)
+    {
+      if ((int)smid < p.queues)
+      {
+        int k = atomicAdd(p.counters + smid, 1);
+        if (k < p.chunk)
+          return (int)smid * p.chunk + k;
+      }
+
+      int tile = p.queued + atomicAdd(p.counters + p.queues, 1);
+      return tile < p.tiles ? tile : -1;
+    }
+
+    __device__ __forceinline__ bool tile_texel(PrefilterFloatParams const &p, int tile, int lane, int &x, int &row)
+    {
+      int block = tile >> 4, in = tile & 15;
+      int bx = block % p.blocks_x, by = block / p.blocks_x;
+      x = (bx * 4 + (in & 3)) * 8 + (lane & 7);
+      row = p.row_begin + (by * 4 + (in >> 2)) * 4 + (lane >> 3);
+      return x < p.wd && row < p.row_end;
+    }
+
+    // ---- epilogue ---------------------------------------------------------------------------
+
+    template<int FMT>
+    __device__ __forceinline__ void store_texel(PrefilterFloatParams const &p, size_t o, float r, float g, float b)
+    {
+      if (FMT == kFloatFormatF16)
+      {
+        uint32_t hr = float_to_half_rn(r), hg = float_to_half_rn(g), hb = float_to_half_rn(b);
+        reinterpret_cast<uint2*>(p.dst)[o] = make_uint2(hg << 16 | hr, 0x3C00u << 16 | hb);
+        if (p.dst_f32)
+        {
+          p.dst_f32[3*o + 0] = r;
+          p.dst_f32[3*o + 1] = g;
+          p.dst_f32[3*o + 2] = b;
+        }
+      }
+      else
+      {
+        reinterpret_cast<float4*>(p.dst)[o] = make_float4(r, g, b, 1.0f);
+        if (p.dst_f32)
+        {
+          p.dst_f32[3*o + 0] = r;
+          p.dst_f32[3*o + 1] = g;
+          p.dst_f32[3*o + 2] = b;
+        }
+      }
+    }
+
+    // ---- the pair kernel ------------------------------------------------------------------------
+    //
+    // CTA = NW warps sharing one 8x4 tile; warp w reads azimuth sector w of every band of the sector table,
+    // its leading bands without face selection as long as they provably stay on the texel's face.
+    template<int FMT, int NW, int MINB, bool SMEM_TABLE, bool QUEUES>
+    __global__ void __launch_bounds__(32 * NW, MINB) prefilter_float_pair_kernel(PrefilterFloatParams p)
+    {
+      typedef typename RecordOf<FMT>::type R;
+
+      extern __shared__ float4 smem[];
+      constexpr int SECTORS = NW == 8 ? 1 : 0;
+      const int bands = p.sector_bands[SECTORS];
+      constexpr int BAND = kSectorShare * NW;
+      const int padded = bands * BAND;
+      float4 *s_table = smem;
+      float *s_red = reinterpret_cast<float*>(smem + (SMEM_TABLE ? padded : 0));
+      int *s_tile = reinterpret_cast<int*>(s_red + NW * 3 * 32);
+
+      const int tid = threadIdx.x;
+      const int lane = tid & 31;
+      const int warp = tid >> 5;
+
+      if (SMEM_TABLE)
+      {
+        for(int i = tid; i < padded; i += 32 * NW)
+          s_table[i] = __ldg(p.table_sector[SECTORS] + i);
+        __syncthreads();
+      }
+
+      float4 const *table = SMEM_TABLE ? s_table : p.table_sector[SECTORS];
+
+      uint32_t smid;
+      asm("mov.u32 %0, %%smid;" : "=r"(smid));
+
+      constexpr int PER = BAND / NW;
+      constexpr int PAIRS = PER / 2;
+      constexpr int BAND_UNROLL = PAIRS >= 2 ? 1 : 2;
+
+      R const *biased = opaque(reinterpret_cast<R const*>(p.records) - (size_t)kMagicBits);
+
+      for(int it = 0; ; ++it)
+      {
+        int tile;
+        if (QUEUES)
+        {
+          if (tid == 0)
+            *s_tile = next_tile_plain(p, smid);
+          __syncthreads();
+          tile = *s_tile;
+
+          if (tile < 0)
+          {
+            __syncthreads();
+            if (warp == 0)
+            {
+              int stolen = steal_tile(p.counters, p.queues, p.chunk, smid, lane);
+              if (lane == 0)
+                *s_tile = stolen;
+            }
+            __syncthreads();
+            tile = *s_tile;
+          }
+        }
+        else
+        {
+          tile = (int)blockIdx.x + it * (int)gridDim.x;
+          if (tile >= p.tiles)
+            tile = -1;
+        }
+
+        if (tile < 0)
+          break;
+
+        int x, row;
+        bool valid = tile_texel(p, tile, lane, x, row);
+
+        if (__ballot_sync(0xffffffffu, valid) == 0u)
+        {
+          if (QUEUES)
+            __syncthreads();
+          continue;
+        }
+
+        if (!valid) { x = p.wd >> 1; row = (p.row_begin / p.hd) * p.hd + (p.hd >> 1); }
+
+        int face = row / p.hd;
+
+        Frame st;
+        int n_same;
+        {
+          float const *f = p.frames + ((size_t)row * p.wd + x);
+          const size_t plane = (size_t)6 * p.hd * p.wd;
+          st.T = Vec3f{ __ldg(f + 0 * plane), __ldg(f + 1 * plane), __ldg(f + 2 * plane) };
+          st.B = Vec3f{ __ldg(f + 3 * plane), __ldg(f + 4 * plane), __ldg(f + 5 * plane) };
+          st.N = Vec3f{ __ldg(f + 6 * plane), __ldg(f + 7 * plane), __ldg(f + 8 * plane) };
+
+          // this warp's sector limit over the tile rows the slab's first row touches (prefilter_dp_kernel)
+          float limit;
+          {
+            const int tiles_x = (p.wd + 7) >> 3, tile_rows = (6 * p.hd + 3) >> 2;
+            const int top = __shfl_sync(0xffffffffu, row, 0), left = __shfl_sync(0xffffffffu, x, 0);
+            const int t0 = top >> 2, t1 = min((top + 3) >> 2, tile_rows - 1);
+            float const *tl = p.frames + 9 * plane + (left >> 3);
+            const size_t sector = (size_t)tile_rows * tiles_x;
+            const int first = NW == 8 ? warp : 2 * warp;
+
+            limit = fminf(__ldg(tl + first * sector + (size_t)t0 * tiles_x), __ldg(tl + first * sector + (size_t)t1 * tiles_x));
+            if (NW != 8)
+              limit = fminf(limit, fminf(__ldg(tl + (first + 1) * sector + (size_t)t0 * tiles_x), __ldg(tl + (first + 1) * sector + (size_t)t1 * tiles_x)));
+          }
+
+          float const *rho = p.sector_rho[SECTORS] + warp * bands;
+          int count = 0;
+          for(int base = 0; base < bands; base += 32)
+          {
+            int k = base + lane;
+            unsigned within = __ballot_sync(0xffffffffu, k < bands && __ldg(rho + k) <= limit);
+            count += __popc(within);
+            if (within != 0xffffffffu)
+              break;
+          }
+          n_same = count;
+        }
+
+        Sums acc;
+        acc.rg = 0ull;
+        acc.bb = 0ull;
+
+        float4 const *tw = table + warp * PER;
+
+        {
+          R const *base = opaque(biased + (size_t)face * p.geom.face_size);
+
+          #pragma unroll BAND_UNROLL
+          for(int band = 0; band < n_same; ++band)
+          {
+            #pragma unroll
+            for(int k = 0; k < PAIRS; ++k)
+              pair_same_face(p, st, base, load_pair<SMEM_TABLE>(tw + band * BAND + 2 * k), acc);
+          }
+        }
+
+        if (n_same < bands)
+        {
+          st.T = from_face_local(face, unfold_face_row(p.geom, st.T));
+          st.B = from_face_local(face, unfold_face_row(p.geom, st.B));
+          st.N = from_face_local(face, unfold_face_row(p.geom, st.N));
+
+          R const *general = opaque(biased + (size_t)(kMagicBits - p.geom.bias_general));
+
+          #pragma unroll BAND_UNROLL
+          for(int band = n_same; band < bands; ++band)
+          {
+            #pragma unroll
+            for(int k = 0; k < PAIRS; ++k)
+              pair_general(p, st, general, load_pair<SMEM_TABLE>(tw + band * BAND + 2 * k), acc);
+          }
+        }
+
+        // ---- reduction over the CTA's warps: s_red[(warp*3 + c)*32 + lane] ----
+        float a[4];
+        unpack2(acc.rg, a[0], a[1]);
+        unpack2(acc.bb, a[2], a[3]);
+        a[2] += a[3];
+
+        #pragma unroll
+        for(int c = 0; c < 3; ++c)
+          s_red[(warp * 3 + c) * 32 + lane] = a[c];
+
+        __syncthreads();
+
+        if (warp == 0)
+        {
+          float sum[3] = { 0.0f, 0.0f, 0.0f };
+          #pragma unroll
+          for(int w = 0; w < NW; ++w)
+          {
+            #pragma unroll
+            for(int c = 0; c < 3; ++c)
+              sum[c] += s_red[(w * 3 + c) * 32 + lane];
+          }
+
+          if (valid)
+            store_texel<FMT>(p, (size_t)row * p.wd + x, sum[0] * p.norm, sum[1] * p.norm, sum[2] * p.norm);
+        }
+
+        __syncthreads();
+      }
+    }
+
+    // ---- the tail kernel: one CTA per texel, lanes are samples (prefilter_tail_kernel) ----------------
+    template<int FMT, int NW, bool PROJ>
+    __global__ void __launch_bounds__(32 * NW) prefilter_float_tail_kernel(PrefilterFloatParams p)
+    {
+      __shared__ float s_red[NW][3];
+      __shared__ float s_frame[9];
+
+      const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+
+      const int texel = blockIdx.x;
+      const int row = p.row_begin + texel / p.wd;
+      const int x = texel - (texel / p.wd) * p.wd;
+      const int face = row / p.hd;
+      const int y = row - face * p.hd;
+
+      if (p.world_frames)
+      {
+        if (threadIdx.x < 9)
+          s_frame[threadIdx.x] = __ldg(p.world_frames + (size_t)threadIdx.x * ((size_t)6 * p.hd * p.wd) + ((size_t)row * p.wd + x));
+      }
+      else if (threadIdx.x == 0)
+      {
+        Vec3f n = texel_normal(p.quats[face], x, y, p.wd, p.hd);
+        Vec3f t, b;
+        tangent_frame(n, t, b);
+        s_frame[0] = t.x; s_frame[1] = t.y; s_frame[2] = t.z;
+        s_frame[3] = b.x; s_frame[4] = b.y; s_frame[5] = b.z;
+        s_frame[6] = n.x; s_frame[7] = n.y; s_frame[8] = n.z;
+      }
+
+      __syncthreads();
+
+      const Vec3f T = { s_frame[0], s_frame[1], s_frame[2] };
+      const Vec3f B = { s_frame[3], s_frame[4], s_frame[5] };
+      const Vec3f N = { s_frame[6], s_frame[7], s_frame[8] };
+
+      float acc[3] = { 0.0f, 0.0f, 0.0f };
+
+      for(int s = threadIdx.x; s < p.table_count; s += 32 * NW)
+      {
+        float4 e = __ldg((PROJ ? p.table_proj : p.table) + s);
+
+        float du, dv, w[4];
+        uint32_t idx;                 // top-left texel of the footprint; i <= ws-2, j <= hs-2
+
+        if (PROJ)
+        {
+          float Lx = fmaf(e.x, T.x, fmaf(e.y, B.x, N.x));
+          float Ly = fmaf(e.x, T.y, fmaf(e.y, B.y, N.y));
+          float Lz = fmaf(e.x, T.z, fmaf(e.y, B.z, N.z));
+
+          uint32_t f;
+          idx = cube_footprint_proj(p.geom, Lx, Ly, Lz, du, dv, f);
+          idx += f * p.geom.face_size - p.geom.bias_general;
+          footprint_weights_diff(du, dv, e.w, e.z, w);
+        }
+        else
+        {
+          float Lx = fmaf(e.z, N.x, fmaf(e.y, B.x, e.x * T.x));
+          float Ly = fmaf(e.z, N.y, fmaf(e.y, B.y, e.x * T.y));
+          float Lz = fmaf(e.z, N.z, fmaf(e.y, B.z, e.x * T.z));
+
+          idx = cube_footprint(p.geom, Lx, Ly, Lz, du, dv);
+          footprint_weights(du, dv, e.w, e.z, w);
+        }
+
+        const uint32_t tap[4] = { idx, idx + 1, idx + (uint32_t)p.geom.ws, idx + (uint32_t)p.geom.ws + 1 };
+        #pragma unroll
+        for(int k = 0; k < 4; ++k)
+        {
+          float c[3];
+          load_texel<FMT>(p.src, tap[k], c);
+          float_accumulate_tap(c[0], c[1], c[2], w[k], acc);
+        }
+      }
+
+      #pragma unroll
+      for(int c = 0; c < 3; ++c)
+      {
+        float v = acc[c];
+        #pragma unroll
+        for(int offset = 16; offset > 0; offset >>= 1)
+          v += __shfl_down_sync(0xffffffffu, v, offset);
+        if (lane == 0)
+          s_red[warp][c] = v;
+      }
+
+      __syncthreads();
+
+      if (threadIdx.x == 0)
+      {
+        float sum[3] = { 0.0f, 0.0f, 0.0f };
+        #pragma unroll
+        for(int w = 0; w < NW; ++w)
+        {
+          #pragma unroll
+          for(int c = 0; c < 3; ++c)
+            sum[c] += s_red[w][c];
+        }
+
+        store_texel<FMT>(p, (size_t)row * p.wd + x, sum[0] * p.norm, sum[1] * p.norm, sum[2] * p.norm);
+      }
+    }
+
+    // resident CTAs per SM for one kernel and dynamic shared-memory size (opt-in above 48 KB)
+    cudaError_t resident_ctas(void (*kernel)(PrefilterFloatParams), int threads, size_t smem, int *resident)
+    {
+      if (smem > 48 * 1024)
+      {
+        cudaError_t err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (err != cudaSuccess)
+          return err;
+      }
+
+      cudaError_t err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(resident, kernel, threads, smem);
+      if (err != cudaSuccess)
+        return err;
+      return *resident < 1 ? cudaErrorLaunchOutOfResources : cudaSuccess;
+    }
+
+    template<int FMT, int NW, int MINB, bool SMEM_TABLE, bool QUEUES>
+    cudaError_t launch_pair(PrefilterFloatParams p, int sm_count, cudaStream_t stream)
+    {
+      auto kernel = prefilter_float_pair_kernel<FMT, NW, MINB, SMEM_TABLE, QUEUES>;
+
+      int rows = p.row_end - p.row_begin;
+      int tiles_x = (p.wd + 7) / 8, tiles_y = (rows + 3) / 4;
+      p.blocks_x = (tiles_x + 3) / 4;
+      p.tiles = p.blocks_x * ((tiles_y + 3) / 4) * 16;
+
+      const int table_bands = p.sector_bands[NW == 8 ? 1 : 0];
+      size_t smem = (SMEM_TABLE ? (size_t)table_bands * kSectorShare * NW * sizeof(float4) : 0) + (size_t)NW * 3 * 32 * sizeof(float) + sizeof(int);
+
+      int resident = 0;
+      cudaError_t err = resident_ctas(kernel, 32 * NW, smem, &resident);
+      if (err != cudaSuccess)
+        return err;
+
+      int grid = p.tiles < sm_count * resident ? p.tiles : sm_count * resident;
+      if (grid < 1)
+        grid = 1;
+
+      // queues: 7/8 of the tiles in per-SM chunks, the rest in the common pool
+      p.queues = sm_count;
+      p.chunk = (p.tiles - p.tiles / 8) / sm_count;
+      p.queued = p.chunk * sm_count;
+
+      kernel<<<grid, 32 * NW, smem, stream>>>(p);
+      return cudaGetLastError();
+    }
+
+    template<int FMT>
+    cudaError_t launch_pair_for(PrefilterFloatParams const &p, int sm_count, cudaStream_t stream)
+    {
+      // the slab-size classes of launch_prefilter_dn: 4 warps per tile for the biggest slabs, 8 below;
+      // tile queues from kQueuedTexels up; a table beyond ~1100 entries is read through L1
+      const size_t texels = (size_t)(p.row_end - p.row_begin) * p.wd;
+      const bool big_table = p.table_count > 1100;
+      const size_t kQueuedTexels = 32u * 148u * 8u, kFourWarpTexels = 160000u;
+
+      if (texels >= kFourWarpTexels)
+        return big_table ? launch_pair<FMT, 4, 8, false, true>(p, sm_count, stream) : launch_pair<FMT, 4, 8, true, true>(p, sm_count, stream);
+      if (texels >= kQueuedTexels)
+        return big_table ? launch_pair<FMT, 8, 4, false, true>(p, sm_count, stream) : launch_pair<FMT, 8, 4, true, true>(p, sm_count, stream);
+      return big_table ? launch_pair<FMT, 8, 4, false, false>(p, sm_count, stream) : launch_pair<FMT, 8, 4, true, false>(p, sm_count, stream);
+    }
+
+    template<int FMT, bool PROJ>
+    cudaError_t launch_tail_for(PrefilterFloatParams const &p, int texels, cudaStream_t stream)
+    {
+      // warps per texel as in launch_prefilter_tail: cover the machine first, then depth
+      if (texels >= 4096 || p.table_count <= 128)
+        prefilter_float_tail_kernel<FMT, 4, PROJ><<<texels, 128, 0, stream>>>(p);
+      else if (texels >= 1024 || p.table_count <= 256)
+        prefilter_float_tail_kernel<FMT, 8, PROJ><<<texels, 256, 0, stream>>>(p);
+      else if (texels >= 256 || p.table_count <= 512)
+        prefilter_float_tail_kernel<FMT, 16, PROJ><<<texels, 512, 0, stream>>>(p);
+      else
+        prefilter_float_tail_kernel<FMT, 32, PROJ><<<texels, 1024, 0, stream>>>(p);
+      return cudaGetLastError();
+    }
+  }
+
+  cudaError_t launch_build_float_records(int format, void const *src, void *records, int ws, int hs, int *counters, int ncounters, int sm_count, cudaStream_t stream)
+  {
+    size_t level = (size_t)6 * ws * hs;
+    size_t blocks = (level + 255) / 256;
+    size_t cap = (size_t)sm_count * 8;
+    int grid = (int)(blocks < cap ? blocks : cap);
+    if (grid < 1)
+      grid = 1;
+
+    if (format == kFloatFormatF16)
+      build_float_records_kernel<kFloatFormatF16><<<grid, 256, 0, stream>>>(src, records, ws, hs, counters, ncounters);
+    else if (format == kFloatFormatF32)
+      build_float_records_kernel<kFloatFormatF32><<<grid, 256, 0, stream>>>(src, records, ws, hs, counters, ncounters);
+    else
+      return cudaErrorInvalidValue;
+    return cudaGetLastError();
+  }
+
+  cudaError_t launch_prefilter_float(PrefilterFloatParams const &p, int sm_count, cudaStream_t stream)
+  {
+    if (p.row_end <= p.row_begin || p.wd <= 0)
+      return cudaSuccess;
+    if (!proj_usable(p.geom.ws, p.geom.hs) || !p.frames || !p.table_sector[0] || !p.table_sector[1])
+      return cudaErrorInvalidValue;
+
+    if (p.format == kFloatFormatF16)
+      return launch_pair_for<kFloatFormatF16>(p, sm_count, stream);
+    if (p.format == kFloatFormatF32)
+      return launch_pair_for<kFloatFormatF32>(p, sm_count, stream);
+    return cudaErrorInvalidValue;
+  }
+
+  cudaError_t launch_prefilter_float_tail(PrefilterFloatParams const &p, cudaStream_t stream)
+  {
+    int texels = (p.row_end - p.row_begin) * p.wd;
+    if (texels <= 0)
+      return cudaSuccess;
+
+    const bool proj = proj_usable(p.geom.ws, p.geom.hs);
+    if (p.format == kFloatFormatF16)
+      return proj ? launch_tail_for<kFloatFormatF16, true>(p, texels, stream) : launch_tail_for<kFloatFormatF16, false>(p, texels, stream);
+    if (p.format == kFloatFormatF32)
+      return proj ? launch_tail_for<kFloatFormatF32, true>(p, texels, stream) : launch_tail_for<kFloatFormatF32, false>(p, texels, stream);
+    return cudaErrorInvalidValue;
+  }
+}

@@ -85,10 +85,18 @@ namespace ibl
       g = (float)((c >> 9) & 0x1FFu) * s;
       b = (float)((c >> 18) & 0x1FFu) * s;
     }
-    else
+    else if (FORMAT == 1)
     {
       float4 c = ldg_stream(reinterpret_cast<float4 const *>(level0) + idx, stream_policy);
       r = c.x; g = c.y; b = c.z;
+    }
+    else
+    {
+      // RGBA16F: one 8-byte load, the halves widened exactly
+      uint32_t lo, hi;
+      asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.v2.u32 {%0,%1}, [%2], %3;" : "=r"(lo), "=r"(hi) : "l"(reinterpret_cast<uint2 const *>(level0) + idx), "l"(stream_policy));
+      asm("{ .reg .b16 x, y; mov.b32 {x, y}, %2; cvt.f32.f16 %0, x; cvt.f32.f16 %1, y; }" : "=f"(r), "=f"(g) : "r"(lo));
+      asm("{ .reg .b16 x, y; mov.b32 {x, y}, %1; cvt.f32.f16 %0, x; }" : "=f"(b) : "r"(hi));
     }
   }
 
@@ -709,8 +717,10 @@ namespace ibl
 
       if (format == 0)
         sh9_partial_kernel<0><<<blocks, kSh9Threads, 0, stream>>>(level0, weights, w, h, row_begin, row_end, block_partials, done_counter, partial, peers);
-      else
+      else if (format == 1)
         sh9_partial_kernel<1><<<blocks, kSh9Threads, 0, stream>>>(level0, weights, w, h, row_begin, row_end, block_partials, done_counter, partial, peers);
+      else
+        sh9_partial_kernel<2><<<blocks, kSh9Threads, 0, stream>>>(level0, weights, w, h, row_begin, row_end, block_partials, done_counter, partial, peers);
 
       return cudaGetLastError();
     }
@@ -738,8 +748,10 @@ namespace ibl
 
     if (format == 0)
       sh9_columns_kernel<0><<<cubes, kSh9ColThreads, 0, stream>>>(level0, weights, w, h, row_begin, row_end, rows_per_item, block_partials, done_counter, partial, peers, probe_stride);
-    else
+    else if (format == 1)
       sh9_columns_kernel<1><<<cubes, kSh9ColThreads, 0, stream>>>(level0, weights, w, h, row_begin, row_end, rows_per_item, block_partials, done_counter, partial, peers, probe_stride);
+    else
+      sh9_columns_kernel<2><<<cubes, kSh9ColThreads, 0, stream>>>(level0, weights, w, h, row_begin, row_end, rows_per_item, block_partials, done_counter, partial, peers, probe_stride);
 
     return cudaGetLastError();
   }

@@ -25,6 +25,13 @@ from . import _lib
 
 FORMAT_RGBE = 0
 FORMAT_F32 = 1
+FORMAT_F16 = 2
+
+# bytes per texel of each format
+TEXEL_BYTES = {FORMAT_RGBE: 4, FORMAT_F32: 16, FORMAT_F16: 8}
+
+# element dtype of the float chain formats (4 channels per texel)
+_FLOAT_DTYPES = {FORMAT_F32: np.float32, FORMAT_F16: np.float16}
 
 
 class IblError(RuntimeError):
@@ -52,6 +59,35 @@ def level_offsets(width, height, levels, layers=6):
     for i in range(levels):
         offsets.append(offsets[-1] + (width >> i) * (height >> i) * layers)
     return offsets
+
+
+def float_chain_texels(width, height, levels):
+    """Texels of a float chain: the same levels as image_datasize, 4 channels each."""
+    return sum((width >> i) * (height >> i) * 6 for i in range(levels))
+
+
+def _texel_bytes(fmt):
+    if fmt not in TEXEL_BYTES:
+        raise ValueError("unknown texel format %r" % (fmt,))
+    return TEXEL_BYTES[fmt]
+
+
+def _float_dtype(fmt):
+    if fmt not in _FLOAT_DTYPES:
+        raise ValueError("unknown float chain format %r (FORMAT_F32 or FORMAT_F16)" % (fmt,))
+    return np.dtype(_FLOAT_DTYPES[fmt])
+
+
+def _check_dtype(buf, dtype, what):
+    """A numpy array or a torch tensor of exactly `dtype` (numpy dtype)."""
+    got = buf.dtype if isinstance(buf, np.ndarray) else getattr(buf, "dtype", None)
+    if isinstance(buf, np.ndarray):
+        ok = got == dtype
+    else:
+        import torch
+        ok = got == {np.dtype(np.float32): torch.float32, np.dtype(np.float16): torch.float16}[dtype]
+    if not ok:
+        raise ValueError("%s must hold %s texels, not %s" % (what, dtype.name, got))
 
 
 def _host_pointer(buf, min_bytes, what):
@@ -231,6 +267,45 @@ class IblContext:
         self._after_torch()
         self._check(self._lib.datum_ibl_prefilter_level_device(self._handle, src_ptr, ws, hs, level, levels, samples, row_begin, row_end, words_ptr, f32_ptr))
 
+    # ---- float chains (RGBA32F / RGBA16F): the same chain without rgbe re-quantisation ----
+
+    def buildmips_cube_float(self, fmt, width, height, levels, chain, samples=1024):
+        """Host float chain (numpy array or CPU torch tensor: float32 for FORMAT_F32, float16 for
+        FORMAT_F16, 4 channels per texel, the levels of image_datasize), level 0 pre-filled, levels >= 1
+        written in place.  Synchronous."""
+        if not (hasattr(chain, "is_cuda") and chain.is_cuda):
+            _check_dtype(chain, _float_dtype(fmt), "chain")
+        ptr = _host_pointer(chain, float_chain_texels(width, height, levels) * _texel_bytes(fmt), "chain")
+        self._check(self._lib.datum_ibl_buildmips_cube_float(self._handle, fmt, width, height, levels, samples, ptr))
+
+    def buildmips_cube_float_device(self, fmt, width, height, levels, d_chain, samples=1024, d_f32=None):
+        """The same chain on a device-resident CUDA tensor of the format's dtype; asynchronous on the
+        context's stream, ordered behind the work torch has queued on its current stream.  d_f32: optional
+        float32 CUDA tensor receiving the fp32 rgb of levels >= 1 before rounding."""
+        _check_dtype(d_chain, _float_dtype(fmt), "d_chain")
+        texels = float_chain_texels(width, height, levels)
+        chain_ptr = _device_pointer(d_chain, texels * _texel_bytes(fmt), "d_chain", self.device)
+        if d_f32 is not None:
+            _check_dtype(d_f32, np.dtype(np.float32), "d_f32")
+        f32_ptr = _device_pointer(d_f32, (texels - 6 * width * height) * 12, "d_f32", self.device)
+        self._after_torch()
+        self._check(self._lib.datum_ibl_buildmips_cube_float_device(self._handle, fmt, width, height, levels, samples, chain_ptr, f32_ptr))
+
+    def prefilter_level_float_device(self, fmt, d_src, ws, hs, level, levels, samples, row_begin, row_end, d_dst, d_dst_f32=None):
+        """One level of a float chain, rows [row_begin,row_end) of the 6*(hs/2) destination rows; CUDA
+        tensors of the format's dtype; asynchronous."""
+        dtype = _float_dtype(fmt)
+        _check_dtype(d_src, dtype, "d_src")
+        _check_dtype(d_dst, dtype, "d_dst")
+        if d_dst_f32 is not None:
+            _check_dtype(d_dst_f32, np.dtype(np.float32), "d_dst_f32")
+        out_texels = 6 * (ws >> 1) * (hs >> 1)
+        src_ptr = _device_pointer(d_src, 6 * ws * hs * _texel_bytes(fmt), "d_src", self.device)
+        dst_ptr = _device_pointer(d_dst, out_texels * _texel_bytes(fmt), "d_dst", self.device)
+        f32_ptr = _device_pointer(d_dst_f32, out_texels * 12, "d_dst_f32", self.device)
+        self._after_torch()
+        self._check(self._lib.datum_ibl_prefilter_level_float_device(self._handle, fmt, src_ptr, ws, hs, level, levels, samples, row_begin, row_end, dst_ptr, f32_ptr))
+
     # ---- SH9: data/project.comp:23-106 ----
 
     # ---- one probe shared by the GPUs of a node: peer-mapped payloads, NVLink stores from the kernel epilogue ----
@@ -275,7 +350,7 @@ class IblContext:
 
     def sh9_partial_device(self, d_level0, fmt, width, height, row_begin, row_end, d_partial):
         """28 partial sums (27 coefficients + weight) into a float64 CUDA tensor; asynchronous."""
-        texel_bytes = 4 if fmt == FORMAT_RGBE else 16
+        texel_bytes = TEXEL_BYTES.get(fmt, 16)   # an unknown format is rejected by the C ABI
         src_ptr = _device_pointer(d_level0, 6 * width * height * texel_bytes, "d_level0", self.device)
         out_ptr = _device_pointer(d_partial, 28 * 8, "d_partial", self.device)
         self._after_torch()
@@ -285,7 +360,7 @@ class IblContext:
         """sh9_partial_device whose 28 sums also go to row [rank] of every peer's (world x 28) float64 array
         (addresses by rank, peer_alloc / peer_open); with flag blocks and an epoch the launch signals the peers
         and the stream waits for theirs.  Asynchronous."""
-        texel_bytes = 4 if fmt == FORMAT_RGBE else 16
+        texel_bytes = TEXEL_BYTES.get(fmt, 16)   # an unknown format is rejected by the C ABI
         src_ptr = _device_pointer(d_level0, 6 * width * height * texel_bytes, "d_level0", self.device)
         self._after_torch()
         slots = (ctypes.c_void_p * world)(*slot_addresses)
@@ -303,7 +378,7 @@ class IblContext:
 
     def project_sh9(self, level0, fmt, width, height):
         """SH9 of a host level-0 cube (uint32 rgbe words or RGBA float32) -> float32 [9][3]."""
-        texel_bytes = 4 if fmt == FORMAT_RGBE else 16
+        texel_bytes = TEXEL_BYTES.get(fmt, 16)   # an unknown format is rejected by the C ABI
         ptr = _host_pointer(level0, 6 * width * height * texel_bytes, "level0")
         sh = np.zeros((9, 3), np.float32)
         self._check(self._lib.datum_ibl_project_sh9(self._handle, ptr, fmt, width, height, sh.ctypes.data))
@@ -441,7 +516,7 @@ class MultiContext:
 
     def project_sh9(self, level0, fmt, width, height):
         """IblContext.project_sh9 with the cube's rows split over the devices."""
-        texel_bytes = 4 if fmt == FORMAT_RGBE else 16
+        texel_bytes = TEXEL_BYTES.get(fmt, 16)   # an unknown format is rejected by the C ABI
         ptr = _host_pointer(level0, 6 * width * height * texel_bytes, "level0")
         sh = np.zeros((9, 3), np.float32)
         self._check(self._lib.datum_ibl_multi_project_sh9(self._handle, ptr, fmt, width, height, sh.ctypes.data))

@@ -36,9 +36,10 @@ extern "C" {
 
 typedef struct datum_ibl_ctx datum_ibl_ctx;
 
-/* texel formats of a level-0 image handed to the SH9 projection */
+/* texel formats of a level-0 image handed to the SH9 projection, and of float chains (F32, F16) */
 #define DATUM_IBL_FORMAT_RGBE 0 /* uint32 E5B9G9R9 words, src/math/color.h:154-172 */
 #define DATUM_IBL_FORMAT_F32 1  /* RGBA fp32, the layout of HDRImage::bits (tools/hdr.h:24) */
+#define DATUM_IBL_FORMAT_F16 2  /* RGBA IEEE binary16, 8 bytes per texel: VK_FORMAT_R16G16B16A16_SFLOAT */
 
 /* ---- lifetime ------------------------------------------------------------ */
 
@@ -295,6 +296,30 @@ int datum_ibl_dominant_kernel_stats(datum_ibl_ctx *ctx, int reset, int *launches
 
 /* milliseconds the device spent in the prefilter kernels of the last chain call (CUDA events) */
 int datum_ibl_last_prefilter_ms(datum_ibl_ctx *ctx, float *ms);
+
+/* ---- GGX prefilter of float chains: RGBA32F / RGBA16F, no rgbe re-quantisation ---------- */
+
+/*
+ * The chain of datum_ibl_buildmips_cube_ibl on a cube of float texels: `format` is DATUM_IBL_FORMAT_F32
+ * (16 bytes per texel) or DATUM_IBL_FORMAT_F16 (8 bytes).  Same layout (level-major, then face 0..5, then
+ * rows; the texel offsets of datum_ibl_chain_bytes' levels, texel size of the format), level 0 pre-filled.
+ * Level L is convolved from level L-1 as stored in the chain (binary16 widened to fp32) with the arithmetic
+ * of tools/ibl.cpp:160-187; input alpha is ignored, output alpha is 1.0.  F32 stores the fp32 result,
+ * F16 stores min(x, 65504) rounded to nearest-even.  Level-0 texels must be finite and non-negative; every
+ * binary16 value works, fp32 values up to 2^52 (4.5e15).  `samples` 1..4096.
+ * Host chain (pageable or pinned), synchronous.
+ */
+int datum_ibl_buildmips_cube_float(datum_ibl_ctx *ctx, int format, int width, int height, int levels, int samples, void *chain);
+
+/*
+ * The same on a device-resident chain (aligned to the texel size); asynchronous on the context's stream.
+ * `d_f32` (optional) receives the fp32 rgb of levels >= 1 before rounding, in the layout of
+ * datum_ibl_buildmips_cube_ibl_device's d_f32.
+ */
+int datum_ibl_buildmips_cube_float_device(datum_ibl_ctx *ctx, int format, int width, int height, int levels, int samples, void *d_chain, float *d_f32);
+
+/* One level of a float chain, rows [row_begin, row_end) of the destination; device pointers, asynchronous. */
+int datum_ibl_prefilter_level_float_device(datum_ibl_ctx *ctx, int format, void const *d_src, int ws, int hs, int level, int levels, int samples, int row_begin, int row_end, void *d_dst, float *d_dst_f32);
 
 #ifdef __cplusplus
 }
