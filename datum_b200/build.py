@@ -26,7 +26,7 @@ HOST_LIB = os.path.join(LIBDIR, "libdatum_ibl_host.so")
 CUDA_SOURCES = ["cabi.cu", "multi.cu", "prefilter_dn.cu", "prefilter_f.cu", "sh9.cu", "luts.cu", "resample.cu", "ibl_tables.cpp"]
 AB_DIR = os.path.join(ROOT, "tools", "ab")
 AB_LIB = os.path.join(AB_DIR, "libdatum_ibl_cuda_ab.so")
-CUDA_HEADERS = ["ibl_math.cuh", "ibl_tables.h", "prefilter.h", "prefilter_f.h", "sh9.h", "luts.h", "resample.h", "cabi_internal.h"]
+CUDA_HEADERS = ["ibl_math.cuh", "ibl_tables.h", "prefilter.h", "prefilter_f.h", "prefilter_pair.cuh", "sh9.h", "luts.h", "resample.h", "cabi_internal.h"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -436,6 +436,28 @@ namespace
     return 0;
   }
 
+  // the checks of a slab of destination rows of a ws x hs source level, both chains: 1 after fail(), else 0
+  int check_slab(int ws, int hs, int row_begin, int row_end)
+  {
+    if (ws < 2 || hs < 2)
+      return fail("prefilter: source level must be at least 2x2");
+    if (row_begin < 0 || row_end > 6 * (hs >> 1) || row_begin > row_end)
+      return fail("prefilter: row range outside the destination level");
+    return 0;
+  }
+
+  // the pair kernels' sector tables (PrefilterDnParams, PrefilterFloatParams)
+  template<typename P>
+  void set_sector_tables(P &p, DeviceTable const &table)
+  {
+    for(int i = 0; i < 2; ++i)
+    {
+      p.table_sector[i] = table.d_sector[i];
+      p.sector_rho[i] = table.d_sector_rho[i];
+      p.sector_bands[i] = table.sector_bands[i];
+    }
+  }
+
   // slabs of more than kTailTexels texels of a level at least a tile wide: denormal-mantissa kernels (prefilter_dn.cu)
   int run_level_dn(datum_ibl_ctx *ctx, uint32_t const *d_src, int ws, int hs, DeviceTable const &table, int row_begin, int row_end, uint32_t *d_dst_words, float *d_dst_f32, bool record_dominant, PeerTargets const &peers, Batch const &batch)
   {
@@ -466,12 +488,7 @@ namespace
     p.records = ctx->records.ptr;
     p.table = table.d_banded;
     p.table_pairs = table.d_pairs;
-    for(int i = 0; i < 2; ++i)
-    {
-      p.table_sector[i] = table.d_sector[i];
-      p.sector_rho[i] = table.d_sector_rho[i];
-      p.sector_bands[i] = table.sector_bands[i];
-    }
+    set_sector_tables(p, table);
     p.band_min_lz = table.d_band_min;
     p.table_count = table.count;
     p.bands = table.bands;
@@ -513,12 +530,8 @@ namespace
   {
     int wd = ws >> 1, hd = hs >> 1;
 
-    if (ws < 2 || hs < 2)
-      return fail("prefilter: source level must be at least 2x2");
-
-    if (row_begin < 0 || row_end > 6 * hd || row_begin > row_end)
-      return fail("prefilter: row range outside the destination level");
-
+    if (check_slab(ws, hs, row_begin, row_end))
+      return 1;
     if (row_begin == row_end)
       return 0;
 
@@ -973,10 +986,8 @@ namespace
   {
     int wd = ws >> 1, hd = hs >> 1;
 
-    if (ws < 2 || hs < 2)
-      return fail("prefilter: source level must be at least 2x2");
-    if (row_begin < 0 || row_end > 6 * hd || row_begin > row_end)
-      return fail("prefilter: row range outside the destination level");
+    if (check_slab(ws, hs, row_begin, row_end))
+      return 1;
     if (row_begin == row_end)
       return 0;
 
@@ -985,12 +996,7 @@ namespace
     p.src = d_src;
     p.table = table.d_banded;
     p.table_proj = table.d_banded_proj;
-    for(int i = 0; i < 2; ++i)
-    {
-      p.table_sector[i] = table.d_sector[i];
-      p.sector_rho[i] = table.d_sector_rho[i];
-      p.sector_bands[i] = table.sector_bands[i];
-    }
+    set_sector_tables(p, table);
     p.table_count = table.count;
     p.dst = d_dst;
     p.dst_f32 = d_dst_f32;

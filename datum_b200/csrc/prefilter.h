@@ -129,6 +129,56 @@ namespace ibl
   // slabs up to this many texels go to the tail kernel
   constexpr int kTailTexels = 6144;
 
+  // warps per texel of the tail kernels: enough CTAs to cover the machine first, then depth; never more lanes than samples
+  inline int tail_warps(int texels, int table_count)
+  {
+    if (texels >= 4096 || table_count <= 128)
+      return 4;
+    if (texels >= 1024 || table_count <= 256)
+      return 8;
+    if (texels >= 256 || table_count <= 512)
+      return 16;
+    return 32;
+  }
+
+  // Slab-size classes of the pair kernels: slabs of at least kQueuedTexels texels take their tiles from
+  // per-SM queues, and of at least kFourWarpTexels run 4 warps per tile instead of 8.  A sample table of more
+  // than kBigTableEntries entries (4096-sample bakes) would cost too much shared memory per CTA: it is read
+  // through L1.
+  constexpr size_t kQueuedTexels = 32u * 148u * 8u;
+  constexpr size_t kFourWarpTexels = 160000u;
+  constexpr int kBigTableEntries = 1100;
+
+  // Resident CTAs per SM of one kernel for one dynamic shared-memory size (opt-in above 48 KB), remembered
+  // per (kernel, device, size) and host thread.
+  cudaError_t resident_ctas(void const *kernel, int threads, size_t smem, int *resident);
+
+  // The launch shape of a tiled kernel over a slab (P: PrefilterDnParams or PrefilterFloatParams): 8x4 tiles
+  // numbered in 4x4 blocks (tile_texel), the slabs of `probes` probes one after the other; at most one CTA
+  // per resident slot; 7/8 of the tiles in per-SM chunks of the tile queues, the rest in the common pool that
+  // evens out the end of the launch.
+  template<typename P>
+  cudaError_t plan_tiles(P &p, void (*kernel)(P), int threads, size_t smem, int probes, int sm_count, int *grid)
+  {
+    int resident = 0;
+    cudaError_t err = resident_ctas((void const*)kernel, threads, smem, &resident);
+    if (err != cudaSuccess)
+      return err;
+
+    const int tiles_x = (p.wd + 7) / 8, tiles_y = (p.row_end - p.row_begin + 3) / 4;
+    p.blocks_x = (tiles_x + 3) / 4;
+    p.tiles = p.blocks_x * ((tiles_y + 3) / 4) * 16 * probes;
+
+    *grid = p.tiles < sm_count * resident ? p.tiles : sm_count * resident;
+    if (*grid < 1)
+      *grid = 1;
+
+    p.queues = sm_count;
+    p.chunk = (p.tiles - p.tiles / 8) / sm_count;
+    p.queued = p.chunk * sm_count;
+    return cudaSuccess;
+  }
+
   cudaError_t launch_prefilter_tail(PrefilterTailParams const &p, int sm_count, cudaStream_t stream);
 
   // variant 0 = pick by slab size and table size; 50..58 = one sample at a time, fixed <warps per tile,

@@ -35,6 +35,7 @@
 //     (build_frames_kernel) instead of computing them per tile.
 
 #include "prefilter.h"
+#include "prefilter_pair.cuh"
 #include "ibl_math.cuh"
 
 #include <cuda_runtime.h>
@@ -43,19 +44,8 @@
 
 namespace ibl
 {
-  typedef unsigned long long f32x2;
-
   namespace
   {
-    // packed two-wide fp32 (fma.rn.f32x2 -> SASS FFMA2/FMUL2/FADD2): same lanes as two scalar
-    // ops, one issue slot; every element is rounded exactly like the scalar form
-    __device__ __forceinline__ f32x2 pack2(float lo, float hi) { f32x2 r; asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi)); return r; }
-    __device__ __forceinline__ void unpack2(f32x2 a, float &lo, float &hi) { asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(a)); }
-    __device__ __forceinline__ f32x2 fma2(f32x2 a, f32x2 b, f32x2 c) { f32x2 d; asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c)); return d; }
-    __device__ __forceinline__ f32x2 mul2(f32x2 a, f32x2 b) { f32x2 d; asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
-    __device__ __forceinline__ f32x2 add2(f32x2 a, f32x2 b) { f32x2 d; asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
-    __device__ __forceinline__ f32x2 bcast2(float v) { return pack2(v, v); }
-
     // bits(w) + E * 2^23 == bits(w * 2^E).  The multiplier arrives as a kernel parameter: as a
     // literal the compiler lowers it to shift + add on the ALU pipe, the pipe this loop is short of.
     __device__ __forceinline__ float scale_by_exponent(float w, uint32_t e, uint32_t emul)
@@ -164,11 +154,6 @@ namespace ibl
     int face;
   };
 
-  struct Sums
-  {
-    f32x2 rg, bb;       // (r, g) and two partial b sums
-  };
-
   // weights of the 2x2 footprint (tools/ibl.cpp:40 as four products), exponents folded in, taps accumulated
   __device__ __forceinline__ void accumulate(uint4 rec, float du, float dv, float nl, float wh, uint32_t emul, Sums &acc)
   {
@@ -229,75 +214,6 @@ namespace ibl
     uint32_t idx = cube_footprint(p.geom, Lx, Ly, Lz, du, dv);
 
     accumulate(__ldg(p.records + idx), du, dv, e.z, e.w, p.exp_mul, acc);
-  }
-
-  // ---- tiles ----------------------------------------------------------------------------
-  //
-  // Tiles of 8x4 texels are numbered in 4x4-blocked order over the slab.  With QUEUES the first
-  // `queued` tiles are cut into one contiguous chunk per SM (queue index = %smid) and the rest form
-  // a common pool that evens out the tail: a group takes tiles from its SM's chunk, then from the pool.
-  //
-  // %smid values are not guaranteed to be contiguous, and under MPS limits, green contexts or a
-  // concurrent kernel an SM may host no CTA of this launch at all: once its own chunk and the pool are
-  // empty (next_tile_plain returns -1) a group therefore looks through every other chunk before it
-  // gives up, so every tile is computed whatever the placement of the CTAs.  The look is made by the 32
-  // lanes of the group's first warp side by side (148 dependent L2 reads by one thread cost ~20 us per
-  // call, measured as +5 % on a whole level; 5 rounds of 32 cost under 1 us), and only then: the common
-  // hand-out stays one thread and one or two atomics.  Called by all lanes of warp 0; every lane gets the tile.
-  // NOT inlined on purpose: with this code inside the kernel body ptxas schedules the sample loops ~1 % (512^2
-  // level) to ~3 % (256^2 level) slower although it only ever runs at the very end of a launch (measured A/B).
-  __device__ __noinline__ int steal_tile(int *counters, int queues, int chunk, uint32_t smid, int lane)
-  {
-    const int own = (int)(smid % (uint32_t)queues);
-
-    for(int base = 1; base < queues; base += 32)
-    {
-      int i = base + lane;
-      int q = own + i;
-      if (q >= queues)
-        q -= queues;
-
-      // a drained chunk costs one read; only chunks that still hold tiles are bumped
-      bool holds = i < queues && *(volatile int const *)(counters + q) < chunk;
-
-      for(unsigned candidates = __ballot_sync(0xffffffffu, holds); candidates != 0u; candidates &= candidates - 1u)
-      {
-        int src = __ffs(candidates) - 1;
-        int k = -1;
-        if (lane == src)
-          k = atomicAdd(counters + q, 1);
-        k = __shfl_sync(0xffffffffu, k, src);
-
-        if (k < chunk)
-          return __shfl_sync(0xffffffffu, q, src) * chunk + k;
-      }
-    }
-
-    return -1;
-  }
-
-  // the common hand-out, one thread: the SM's own chunk, then the pool; -1 when both are empty
-  __device__ __forceinline__ int next_tile_plain(PrefilterDnParams const &p, uint32_t smid)
-  {
-    if ((int)smid < p.queues)
-    {
-      int k = atomicAdd(p.counters + smid, 1);
-      if (k < p.chunk)
-        return (int)smid * p.chunk + k;
-    }
-
-    int tile = p.queued + atomicAdd(p.counters + p.queues, 1);
-    return tile < p.tiles ? tile : -1;
-  }
-
-  // tile number -> texel of this lane; false when the lane's texel is outside the slab
-  __device__ __forceinline__ bool tile_texel(PrefilterDnParams const &p, int tile, int lane, int &x, int &row)
-  {
-    int block = tile >> 4, in = tile & 15;
-    int bx = block % p.blocks_x, by = block / p.blocks_x;
-    x = (bx * 4 + (in & 3)) * 8 + (lane & 7);
-    row = p.row_begin + (by * 4 + (in >> 2)) * 4 + (lane >> 3);
-    return x < p.wd && row < p.row_end;
   }
 
   // ---- the kernel --------------------------------------------------------------------------
@@ -473,28 +389,13 @@ namespace ibl
         }
       }
 
-      // ---- reduction over the CTA's warps: s_red[(warp*3 + c)*32 + lane] ----
-      float a[4];
-      unpack2(acc.rg, a[0], a[1]);
-      unpack2(acc.bb, a[2], a[3]);
-      a[2] += a[3];
-
-      #pragma unroll
-      for(int c = 0; c < 3; ++c)
-        s_red[(warp * 3 + c) * 32 + lane] = a[c];
-
+      store_warp_sums(acc, s_red, warp, lane);
       __syncthreads();
 
       if (warp == 0)
       {
-        float sum[3] = { 0.0f, 0.0f, 0.0f };
-        #pragma unroll
-        for(int w = 0; w < NW; ++w)
-        {
-          #pragma unroll
-          for(int c = 0; c < 3; ++c)
-            sum[c] += s_red[(w * 3 + c) * 32 + lane];
-        }
+        float sum[3];
+        add_warp_sums<NW>(s_red, lane, sum);
 
         if (valid)
         {
@@ -637,46 +538,13 @@ namespace ibl
   // Two statements of the per-pair arithmetic follow.  The first (direction_pair, gather_pair,
   // pair_same_face, pair_general: PROJ = false) is round 2's first cut — three-term directions, an
   // integer record index whose bias kMagicBits*(ws+1) is folded into the record pointer, four weight
-  // products — kept for the A/B variants of the tools build.  The second (…_proj: what ships) is the
-  // projective form described at its head.
+  // products — kept for the A/B variants of the tools build.  The second (gather_pair_proj with the
+  // coordinates of prefilter_pair.cuh: what ships) is the projective form described there.
 
-  struct PairEntry
-  {
-    f32x2 lx, ly, lz, wh;   // each: (sample a, sample b)
-  };
-
-  template<bool SMEM_TABLE>
-  __device__ __forceinline__ PairEntry load_pair(float4 const *t)
-  {
-    ulonglong2 const *q = reinterpret_cast<ulonglong2 const*>(t);
-    ulonglong2 lo = SMEM_TABLE ? q[0] : __ldg(q);
-    ulonglong2 hi = SMEM_TABLE ? q[1] : __ldg(q + 1);
-    return PairEntry{ lo.x, lo.y, hi.x, hi.y };
-  }
-
-  struct Frame
-  {
-    Vec3f T, B, N;
-  };
-
-  // record `idx` (unsigned 32-bit, bias included): one IMAD.WIDE.U32 as long as `base` is an opaque
-  // register pair (see opaque()); otherwise the compiler re-associates the 64-bit sum into four adds
+  // record `idx` (unsigned 32-bit, bias included) of an opaque() `base`
   __device__ __forceinline__ uint4 load_record(uint4 const *base, uint32_t idx)
   {
     return __ldg(base + idx);
-  }
-
-  __device__ __forceinline__ uint4 const *opaque(uint4 const *ptr)
-  {
-    asm volatile("" : "+l"(ptr));
-    return ptr;
-  }
-
-  __device__ __forceinline__ f32x2 neg2(f32x2 a)
-  {
-    float lo, hi;
-    unpack2(a, lo, hi);
-    return pack2(-lo, -hi);
   }
 
   // reflected directions of both samples in the frame's coordinates, the kernel above's operation order
@@ -780,23 +648,6 @@ namespace ibl
     gather_pair<EXP_ALU, RHI>(p, base, fa * p.geom.face_size, fb * p.geom.face_size, fu, fv, e, acc);
   }
 
-
-  // ---- projective form (ibl_math.cuh: face_footprint_proj, cube_footprint_proj, footprint_weights_diff) ----
-  //
-  // Entries hold (lx/lz, ly/lz): a direction is two packed multiply-adds per component.  On the texel's
-  // own face the rows arrive folded (fold_face_row), so integer part and fraction of a texel coordinate
-  // are one FFMA2 each straight from the quotient; the record index is formed in the fp32 adder
-  // (magic + i + j*ws, exact) and its bits go into IMAD.WIDE as they are.  The right-hand taps' weights
-  // are differences.  Per pair of samples: 32 packed fp32 operations and 10 integer multiply-adds where
-  // the form above needs 37 and 12.
-
-  __device__ __forceinline__ void direction_pair_proj(Frame const &t, PairEntry const &e, f32x2 &x, f32x2 &y, f32x2 &z)
-  {
-    x = fma2(e.lx, bcast2(t.T.x), fma2(e.ly, bcast2(t.B.x), bcast2(t.N.x)));
-    y = fma2(e.lx, bcast2(t.T.y), fma2(e.ly, bcast2(t.B.y), bcast2(t.N.y)));
-    z = fma2(e.lx, bcast2(t.T.z), fma2(e.ly, bcast2(t.B.z), bcast2(t.N.z)));
-  }
-
   // idx = raw index bits of both samples (what `base` has been moved back by), du/dv = fraction - 0.5
   template<int EXP_ALU>
   __device__ __forceinline__ void gather_pair_proj(PrefilterDnParams const &p, uint4 const *base, uint32_t idx_a, uint32_t idx_b, f32x2 du, f32x2 dv, PairEntry const &e, Sums &acc)
@@ -846,56 +697,20 @@ namespace ibl
   template<int EXP_ALU>
   __device__ __forceinline__ void pair_same_face_proj(PrefilterDnParams const &p, Frame const &t, uint4 const *base, PairEntry const &e, Sums &acc)
   {
-    f32x2 la, lb, lm;
-    direction_pair_proj(t, e, la, lb, lm);
-
-    float ma, mb;
-    unpack2(lm, ma, mb);
-    f32x2 r = pack2(rcp_fast(ma), rcp_fast(mb));
-
-    f32x2 mu = fma2(la, r, bcast2(kMagic));
-    f32x2 mv = fma2(lb, r, bcast2(kMagic));
-    f32x2 niu = add2(neg2(mu), bcast2(kMagic));
-    f32x2 niv = add2(neg2(mv), bcast2(kMagic));
-    f32x2 du = fma2(la, r, niu);
-    f32x2 dv = fma2(lb, r, niv);
-
-    float ia, ib;
-    unpack2(fma2(niv, bcast2(p.geom.neg_ws), mu), ia, ib);
-
-    gather_pair_proj<EXP_ALU>(p, base, f2u(ia), f2u(ib), du, dv, e, acc);
+    uint32_t ia, ib;
+    f32x2 du, dv;
+    pair_taps_same_face(p.geom, t, e, ia, ib, du, dv);
+    gather_pair_proj<EXP_ALU>(p, base, ia, ib, du, dv, e, acc);
   }
 
   // frame rows in world coordinates; `base` = records moved back by geom.bias_general
   template<int EXP_ALU>
   __device__ __forceinline__ void pair_general_proj(PrefilterDnParams const &p, Frame const &t, uint4 const *base, PairEntry const &e, Sums &acc)
   {
-    f32x2 x, y, z;
-    direction_pair_proj(t, e, x, y, z);
-
-    float xa, xb, ya, yb, za, zb;
-    unpack2(x, xa, xb);
-    unpack2(y, ya, yb);
-    unpack2(z, za, zb);
-
-    float qua, qva, qub, qvb;
-    uint32_t fa, fb;
-    cube_select_unshrunk(xa, ya, za, qua, qva, fa);
-    cube_select_unshrunk(xb, yb, zb, qub, qvb, fb);
-
-    // the two-ulp shrink of the reciprocal (cube_select) rides in the scale
-    f32x2 qu = pack2(qua, qub), qv = pack2(qva, qvb);
-    f32x2 mu = fma2(qu, bcast2(p.geom.hw_shrunk), bcast2(p.geom.hwm_magic));
-    f32x2 mv = fma2(qv, bcast2(p.geom.hh_shrunk), bcast2(p.geom.hhm_magic));
-    f32x2 cu = add2(neg2(mu), bcast2(p.geom.hwm_magic));
-    f32x2 cv = add2(neg2(mv), bcast2(p.geom.hhm_magic));
-    f32x2 du = fma2(qu, bcast2(p.geom.hw_shrunk), cu);
-    f32x2 dv = fma2(qv, bcast2(p.geom.hh_shrunk), cv);
-
-    float ia, ib;
-    unpack2(fma2(cv, bcast2(p.geom.neg_ws), mu), ia, ib);
-
-    gather_pair_proj<EXP_ALU>(p, base, fa * p.geom.face_size + f2u(ia), fb * p.geom.face_size + f2u(ib), du, dv, e, acc);
+    uint32_t ia, ib;
+    f32x2 du, dv;
+    pair_taps_general(p.geom, t, e, ia, ib, du, dv);
+    gather_pair_proj<EXP_ALU>(p, base, ia, ib, du, dv, e, acc);
   }
 
   template<int NW, int MINB, bool SMEM_TABLE, bool QUEUES, int EXP_ALU, int DEPTH = 1, bool RHI = false, bool PLAIN_QUEUE = false, bool LEAN = false, bool PROJ = true, int VW = 1>
@@ -1006,58 +821,7 @@ namespace ibl
       {
         if (PROJ)
         {
-          // the texel's frame from the per-level planes (launch_build_frames)
-          float const *f = p.frames + ((size_t)row * p.wd + x);
-          const size_t plane = (size_t)6 * p.hd * p.wd;
-          st.T = Vec3f{ __ldg(f + 0 * plane), __ldg(f + 1 * plane), __ldg(f + 2 * plane) };
-          st.B = Vec3f{ __ldg(f + 3 * plane), __ldg(f + 4 * plane), __ldg(f + 5 * plane) };
-          st.N = Vec3f{ __ldg(f + 6 * plane), __ldg(f + 7 * plane), __ldg(f + 8 * plane) };
-
-          // this warp reads ONE azimuth sector of every band: how far out its samples may lie before one of them
-          // can leave some texel's face (sector_rho_limits, kept as the minimum over the texels of every 8x4 tile
-          // of the level; a slab that starts between two such tile rows looks at both; the eight 45-degree sectors
-          // pair up for four warps)
-          float limit, limit_second = 0.0f;
-          {
-            const int tiles_x = (p.wd + 7) >> 3, tile_rows = (6 * p.hd + 3) >> 2;
-            const int top = __shfl_sync(0xffffffffu, row, 0), left = __shfl_sync(0xffffffffu, x, 0);     // lane 0 is always inside the slab
-            const int t0 = top >> 2, t1 = min((top + 3) >> 2, tile_rows - 1);
-            float const *tile = p.frames + 9 * plane + (left >> 3);
-            const size_t sector = (size_t)tile_rows * tiles_x;
-            const int first = NW == 8 ? warp : 2 * warp;
-
-            limit = fminf(__ldg(tile + first * sector + (size_t)t0 * tiles_x), __ldg(tile + first * sector + (size_t)t1 * tiles_x));
-            if (NW != 8)
-            {
-              float second = fminf(__ldg(tile + (first + 1) * sector + (size_t)t0 * tiles_x), __ldg(tile + (first + 1) * sector + (size_t)t1 * tiles_x));
-              if (VW == 2)
-                limit_second = second;
-              else
-                limit = fminf(limit, second);
-            }
-          }
-
-          // leading bands whose share of this sector stays inside it (sector_rho increases with the band): the lanes
-          // look at 32 bands at a time
-          #pragma unroll
-          for(int pass = 0; pass < VW; ++pass)
-          {
-            float const *rho = p.sector_rho[SECTORS] + (VW * warp + pass) * bands;
-            const float within_limit = pass == 0 ? limit : limit_second;
-            int count = 0;
-            for(int base = 0; base < bands; base += 32)
-            {
-              int k = base + lane;
-              unsigned within = __ballot_sync(0xffffffffu, k < bands && __ldg(rho + k) <= within_limit);
-              count += __popc(within);
-              if (within != 0xffffffffu)
-                break;
-            }
-            if (pass == 0)
-              n_same = count;
-            else
-              n_same_second = count;
-          }
+          tile_frame_bands<NW, VW>(p, x, row, warp, lane, bands, st, n_same, n_same_second);
         }
         else
         {
@@ -1155,28 +919,13 @@ namespace ibl
         }
       }
 
-      // ---- reduction over the CTA's warps: s_red[(warp*3 + c)*32 + lane] ----
-      float a[4];
-      unpack2(acc.rg, a[0], a[1]);
-      unpack2(acc.bb, a[2], a[3]);
-      a[2] += a[3];
-
-      #pragma unroll
-      for(int c = 0; c < 3; ++c)
-        s_red[(warp * 3 + c) * 32 + lane] = a[c];
-
+      store_warp_sums(acc, s_red, warp, lane);
       __syncthreads();
 
       if (warp == 0)
       {
-        float sum[3] = { 0.0f, 0.0f, 0.0f };
-        #pragma unroll
-        for(int w = 0; w < NW; ++w)
-        {
-          #pragma unroll
-          for(int c = 0; c < 3; ++c)
-            sum[c] += s_red[(w * 3 + c) * 32 + lane];
-        }
+        float sum[3];
+        add_warp_sums<NW>(s_red, lane, sum);
 
         if (valid)
         {
@@ -1364,27 +1113,17 @@ namespace ibl
       p.probes = 1;
     p.texels_per_probe = texels;
 
-    // warps per texel: enough CTAs to cover the machine first, then depth; never more lanes than samples.
-    // Chosen from ONE probe's texels also when a launch carries several: the shape decides the order of
-    // the sums, and a batch must give the words of single calls.
+    // warps per texel (tail_warps) chosen from ONE probe's texels also when a launch carries several: the
+    // shape decides the order of the sums, and a batch must give the words of single calls
     (void)sm_count;
     int grid = texels * p.probes;
     const bool proj = p.table_proj != nullptr && proj_usable(p.geom.ws, p.geom.hs);
-    if (texels >= 4096 || p.table_count <= 128)
+    switch (tail_warps(texels, p.table_count))
     {
-      if (proj) prefilter_tail_kernel<4, true><<<grid, 128, 0, stream>>>(p); else prefilter_tail_kernel<4, false><<<grid, 128, 0, stream>>>(p);
-    }
-    else if (texels >= 1024 || p.table_count <= 256)
-    {
-      if (proj) prefilter_tail_kernel<8, true><<<grid, 256, 0, stream>>>(p); else prefilter_tail_kernel<8, false><<<grid, 256, 0, stream>>>(p);
-    }
-    else if (texels >= 256 || p.table_count <= 512)
-    {
-      if (proj) prefilter_tail_kernel<16, true><<<grid, 512, 0, stream>>>(p); else prefilter_tail_kernel<16, false><<<grid, 512, 0, stream>>>(p);
-    }
-    else
-    {
-      if (proj) prefilter_tail_kernel<32, true><<<grid, 1024, 0, stream>>>(p); else prefilter_tail_kernel<32, false><<<grid, 1024, 0, stream>>>(p);
+      case 4: if (proj) prefilter_tail_kernel<4, true><<<grid, 128, 0, stream>>>(p); else prefilter_tail_kernel<4, false><<<grid, 128, 0, stream>>>(p); break;
+      case 8: if (proj) prefilter_tail_kernel<8, true><<<grid, 256, 0, stream>>>(p); else prefilter_tail_kernel<8, false><<<grid, 256, 0, stream>>>(p); break;
+      case 16: if (proj) prefilter_tail_kernel<16, true><<<grid, 512, 0, stream>>>(p); else prefilter_tail_kernel<16, false><<<grid, 512, 0, stream>>>(p); break;
+      default: if (proj) prefilter_tail_kernel<32, true><<<grid, 1024, 0, stream>>>(p); else prefilter_tail_kernel<32, false><<<grid, 1024, 0, stream>>>(p); break;
     }
 
     return cudaGetLastError();
@@ -1423,90 +1162,75 @@ namespace ibl
     return cudaGetLastError();
   }
 
-  namespace
+  // The occupancy query costs more host time than the launch itself: its answer is remembered per (kernel,
+  // device, size).  The kernel's ADDRESS is part of the key (round 1 keyed by size only: a hit recorded by one
+  // kernel skipped the opt-in of another).  The dynamic shared-memory opt-in is only ever raised, and only
+  // above the 48 KB every kernel may use without it: setting the attribute to a smaller value would LOWER the
+  // kernel's limit.
+  cudaError_t resident_ctas(void const *kernel, int threads, size_t smem, int *resident)
   {
-    // Resident CTAs per SM of one kernel for one dynamic shared-memory size, remembered per (kernel,
-    // device, size): the occupancy query costs more host time than the launch itself.  Every kernel
-    // instantiation here has the same function-pointer type, so the kernel's ADDRESS is part of the key
-    // (round 1 keyed by size only: a hit recorded by one kernel skipped the opt-in of another).  The
-    // dynamic shared-memory opt-in is only ever raised, and only above the 48 KB every kernel may use
-    // without it: setting the attribute to a smaller value would LOWER the kernel's limit.
-    cudaError_t resident_ctas(void (*kernel)(PrefilterDnParams), int threads, size_t smem, int *resident)
-    {
-      struct Entry { void (*kernel)(PrefilterDnParams); int device; size_t smem; int resident; };
-      thread_local static std::vector<Entry> cache;
-      struct OptIn { void (*kernel)(PrefilterDnParams); int device; size_t smem; };
-      thread_local static std::vector<OptIn> opted;
+    struct Entry { void const *kernel; int device; size_t smem; int resident; };
+    thread_local static std::vector<Entry> cache;
+    struct OptIn { void const *kernel; int device; size_t smem; };
+    thread_local static std::vector<OptIn> opted;
 
-      int device = 0;
-      cudaError_t err = cudaGetDevice(&device);
-      if (err != cudaSuccess)
-        return err;
+    int device = 0;
+    cudaError_t err = cudaGetDevice(&device);
+    if (err != cudaSuccess)
+      return err;
 
-      for(auto const &e : cache)
-        if (e.kernel == kernel && e.device == device && e.smem == smem)
-        {
-          *resident = e.resident;
-          return cudaSuccess;
-        }
-
-      if (smem > 48 * 1024)
+    for(auto const &e : cache)
+      if (e.kernel == kernel && e.device == device && e.smem == smem)
       {
-        OptIn *mine = nullptr;
-        for(auto &o : opted)
-          if (o.kernel == kernel && o.device == device)
-            mine = &o;
-
-        if (!mine || mine->smem < smem)
-        {
-          err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-          if (err != cudaSuccess)
-            return err;
-          if (mine)
-            mine->smem = smem;
-          else
-            opted.push_back(OptIn{ kernel, device, smem });
-        }
+        *resident = e.resident;
+        return cudaSuccess;
       }
 
-      err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(resident, kernel, threads, smem);
-      if (err != cudaSuccess)
-        return err;
-      if (*resident < 1)
-        return cudaErrorLaunchOutOfResources;
+    if (smem > 48 * 1024)
+    {
+      OptIn *mine = nullptr;
+      for(auto &o : opted)
+        if (o.kernel == kernel && o.device == device)
+          mine = &o;
 
-      if (cache.size() >= 256)
-        cache.clear();
-      cache.push_back(Entry{ kernel, device, smem, *resident });
-
-      return cudaSuccess;
+      if (!mine || mine->smem < smem)
+      {
+        err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (err != cudaSuccess)
+          return err;
+        if (mine)
+          mine->smem = smem;
+        else
+          opted.push_back(OptIn{ kernel, device, smem });
+      }
     }
 
+    err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(resident, kernel, threads, smem);
+    if (err != cudaSuccess)
+      return err;
+    if (*resident < 1)
+      return cudaErrorLaunchOutOfResources;
+
+    if (cache.size() >= 256)
+      cache.clear();
+    cache.push_back(Entry{ kernel, device, smem, *resident });
+
+    return cudaSuccess;
+  }
+
+  namespace
+  {
     template<int NW, int UNROLL, int MINB, bool SMEM_TABLE, bool QUEUES>
     cudaError_t launch_dn(PrefilterDnParams p, int sm_count, cudaStream_t stream, int *launched_grid)
     {
       auto kernel = prefilter_dn_kernel<NW, UNROLL, MINB, SMEM_TABLE, QUEUES>;
 
-      int rows = p.row_end - p.row_begin;
-      int tiles_x = (p.wd + 7) / 8, tiles_y = (rows + 3) / 4;
-      p.blocks_x = (tiles_x + 3) / 4;
-      p.tiles = p.blocks_x * ((tiles_y + 3) / 4) * 16;
-
       size_t smem = (SMEM_TABLE ? (size_t)p.table_count * sizeof(float4) : 0) + (size_t)NW * 3 * 32 * sizeof(float) + sizeof(int);
 
-      int resident = 0;
-      cudaError_t err = resident_ctas(kernel, 32 * NW, smem, &resident);
+      int grid = 0;
+      cudaError_t err = plan_tiles(p, kernel, 32 * NW, smem, 1, sm_count, &grid);
       if (err != cudaSuccess)
         return err;
-
-      int grid = p.tiles < sm_count * resident ? p.tiles : sm_count * resident;
-      if (grid < 1)
-        grid = 1;
-
-      // queues: 7/8 of the tiles in per-SM chunks, the rest in the common pool
-      p.queues = sm_count;
-      p.chunk = (p.tiles - p.tiles / 8) / sm_count;
-      p.queued = p.chunk * sm_count;
 
       kernel<<<grid, 32 * NW, smem, stream>>>(p);
 
@@ -1515,44 +1239,25 @@ namespace ibl
 
       return cudaGetLastError();
     }
-  }
 
-  namespace
-  {
     template<int NW, int MINB, bool SMEM_TABLE, bool QUEUES, int EXP_ALU = 0, int DEPTH = 1, bool RHI = false, bool PLAIN_QUEUE = false, bool LEAN = false, bool PROJ = true, int VW = 1>
     cudaError_t launch_dp(PrefilterDnParams p, int sm_count, cudaStream_t stream, int *launched_grid)
     {
       auto kernel = prefilter_dp_kernel<NW, MINB, SMEM_TABLE, QUEUES, EXP_ALU, DEPTH, RHI, PLAIN_QUEUE, LEAN, PROJ, VW>;
 
-      int rows = p.row_end - p.row_begin;
-      int tiles_x = (p.wd + 7) / 8, tiles_y = (rows + 3) / 4;
-      p.blocks_x = (tiles_x + 3) / 4;
-      p.tiles_per_probe = p.blocks_x * ((tiles_y + 3) / 4) * 16;
-      if (p.probes < 1)
-        p.probes = 1;
-      p.tiles = p.tiles_per_probe * p.probes;
-
       const int table_bands = PROJ ? p.sector_bands[NW * VW == 8 ? 1 : 0] : p.bands;
       const int band_entries = PROJ ? kSectorShare * NW * VW : kSampleBand;
       size_t smem = (SMEM_TABLE ? (size_t)table_bands * band_entries * sizeof(float4) : 0) + (size_t)NW * 3 * 32 * sizeof(float) + sizeof(int);
 
-      int resident = 0;
-      cudaError_t err = resident_ctas(kernel, 32 * NW, smem, &resident);
+      // (Cutting the common pool's tiles, or every tile of a slab too small to fill the machine, into 2-8
+      // shares of their bands was measured and dropped: profiles/r2_summary.md.)
+      if (p.probes < 1)
+        p.probes = 1;
+      int grid = 0;
+      cudaError_t err = plan_tiles(p, kernel, 32 * NW, smem, p.probes, sm_count, &grid);
       if (err != cudaSuccess)
         return err;
-
-      const int slots = sm_count * resident;
-
-      int grid = p.tiles < slots ? p.tiles : slots;
-      if (grid < 1)
-        grid = 1;
-
-      // queues: 7/8 of the tiles in per-SM chunks, the rest in the common pool that evens out the end of
-      // the launch.  (Cutting the pool's tiles, or every tile of a slab too small to fill the machine,
-      // into 2-8 shares of their bands was measured and dropped: profiles/r2_summary.md.)
-      p.queues = sm_count;
-      p.chunk = (p.tiles - p.tiles / 8) / sm_count;
-      p.queued = p.chunk * sm_count;
+      p.tiles_per_probe = p.tiles / p.probes;
 
       kernel<<<grid, 32 * NW, smem, stream>>>(p);
 
@@ -1570,11 +1275,6 @@ namespace ibl
     }
   }
 
-  // slabs of at least this many texels take their tiles from per-SM queues
-  constexpr size_t kQueuedTexels = 32u * 148u * 8u;
-  // ... and of at least this many run 4 warps per tile instead of 8
-  constexpr size_t kFourWarpTexels = 160000u;
-
   bool prefilter_batchable(int ws, int hs)
   {
     PrefilterDnParams p = {};
@@ -1590,12 +1290,11 @@ namespace ibl
     if (rows <= 0 || p.wd <= 0)
       return cudaSuccess;
 
-    // Automatic choice by slab size (measured on C2, tools/level_times.py).  A table beyond ~1100
-    // entries (4096-sample bakes) would cost too much shared memory per CTA: read it through L1.
+    // Automatic choice by slab size (measured on C2, tools/level_times.py) and table size (kBigTableEntries).
     if (variant == 0)
     {
       size_t texels = (size_t)rows * p.wd;
-      bool big_table = p.table_count > 1100;
+      bool big_table = p.table_count > kBigTableEntries;
 
       // the two biggest classes work on two samples at a time (prefilter_dp_kernel; measured on C2:
       // level 1 885 -> 862 us, level 2 277 -> 262, level 3 96 -> 88); launch_prefilter_dn falls back to

@@ -14,11 +14,13 @@
 //     texels of a footprint read straight from the source level.  Small slabs, levels narrower than a
 //     tile, and every source the pair kernel cannot address (!proj_usable: odd sizes, faces above 2048^2).
 //
-// The device helpers below restate those of prefilter_dn.cu instead of sharing them: the rgbe kernels
-// are sensitive to everything compiled into their bodies (DESIGN.md §4.1), and they stay untouched.
+// The pair kernel shares its device helpers with prefilter_dn.cu (prefilter_pair.cuh): packed fp32 ops, pair
+// entries, projective footprint coordinates, tile hand-out, per-tile frame and same-face band count, CTA
+// reduction.  The launchers share resident_ctas, plan_tiles, the slab-size classes and tail_warps (prefilter.h).
 
 #include "prefilter.h"
 #include "prefilter_f.h"
+#include "prefilter_pair.cuh"
 #include "ibl_math.cuh"
 
 #include <cuda_runtime.h>
@@ -27,32 +29,8 @@ namespace ibl
 {
   namespace
   {
-    typedef unsigned long long f32x2;
-
-    __device__ __forceinline__ f32x2 pack2(float lo, float hi) { f32x2 r; asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi)); return r; }
-    __device__ __forceinline__ void unpack2(f32x2 a, float &lo, float &hi) { asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(a)); }
-    __device__ __forceinline__ f32x2 fma2(f32x2 a, f32x2 b, f32x2 c) { f32x2 d; asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c)); return d; }
-    __device__ __forceinline__ f32x2 mul2(f32x2 a, f32x2 b) { f32x2 d; asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
-    __device__ __forceinline__ f32x2 add2(f32x2 a, f32x2 b) { f32x2 d; asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
-    __device__ __forceinline__ f32x2 bcast2(float v) { return pack2(v, v); }
-
-    __device__ __forceinline__ f32x2 neg2(f32x2 a)
-    {
-      float lo, hi;
-      unpack2(a, lo, hi);
-      return pack2(-lo, -hi);
-    }
-
     template<int FMT> struct RecordOf { typedef F32Record type; };
     template<> struct RecordOf<kFloatFormatF16> { typedef F16Record type; };
-
-    // a record pointer the compiler cannot re-associate: the index goes into one IMAD.WIDE
-    template<typename R>
-    __device__ __forceinline__ R const *opaque(R const *ptr)
-    {
-      asm volatile("" : "+l"(ptr));
-      return ptr;
-    }
 
     // ---- records --------------------------------------------------------------------------
 
@@ -139,37 +117,6 @@ namespace ibl
       }
     }
 
-    struct Sums
-    {
-      f32x2 rg, bb;       // (r, g) and the b sums of the two samples of a pair
-    };
-
-    struct PairEntry
-    {
-      f32x2 lx, ly, lz, wh;   // each: (sample a, sample b)
-    };
-
-    template<bool SMEM_TABLE>
-    __device__ __forceinline__ PairEntry load_pair(float4 const *t)
-    {
-      ulonglong2 const *q = reinterpret_cast<ulonglong2 const*>(t);
-      ulonglong2 lo = SMEM_TABLE ? q[0] : __ldg(q);
-      ulonglong2 hi = SMEM_TABLE ? q[1] : __ldg(q + 1);
-      return PairEntry{ lo.x, lo.y, hi.x, hi.y };
-    }
-
-    struct Frame
-    {
-      Vec3f T, B, N;
-    };
-
-    __device__ __forceinline__ void direction_pair_proj(Frame const &t, PairEntry const &e, f32x2 &x, f32x2 &y, f32x2 &z)
-    {
-      x = fma2(e.lx, bcast2(t.T.x), fma2(e.ly, bcast2(t.B.x), bcast2(t.N.x)));
-      y = fma2(e.lx, bcast2(t.T.y), fma2(e.ly, bcast2(t.B.y), bcast2(t.N.y)));
-      z = fma2(e.lx, bcast2(t.T.z), fma2(e.ly, bcast2(t.B.z), bcast2(t.N.z)));
-    }
-
     // idx = raw index bits of both samples (what `base` has been moved back by), du/dv = fraction - 0.5;
     // the weights of footprint_weights_diff (ibl.cpp:40 times the sample weight), taps as floats
     template<typename R>
@@ -204,108 +151,20 @@ namespace ibl
     template<typename R>
     __device__ __forceinline__ void pair_same_face(PrefilterFloatParams const &p, Frame const &t, R const *base, PairEntry const &e, Sums &acc)
     {
-      f32x2 la, lb, lm;
-      direction_pair_proj(t, e, la, lb, lm);
-
-      float ma, mb;
-      unpack2(lm, ma, mb);
-      f32x2 r = pack2(rcp_fast(ma), rcp_fast(mb));
-
-      f32x2 mu = fma2(la, r, bcast2(kMagic));
-      f32x2 mv = fma2(lb, r, bcast2(kMagic));
-      f32x2 niu = add2(neg2(mu), bcast2(kMagic));
-      f32x2 niv = add2(neg2(mv), bcast2(kMagic));
-      f32x2 du = fma2(la, r, niu);
-      f32x2 dv = fma2(lb, r, niv);
-
-      float ia, ib;
-      unpack2(fma2(niv, bcast2(p.geom.neg_ws), mu), ia, ib);
-
-      gather_pair(base, f2u(ia), f2u(ib), du, dv, e, acc);
+      uint32_t ia, ib;
+      f32x2 du, dv;
+      pair_taps_same_face(p.geom, t, e, ia, ib, du, dv);
+      gather_pair(base, ia, ib, du, dv, e, acc);
     }
 
     // frame rows in world coordinates; `base` = records moved back by geom.bias_general
     template<typename R>
     __device__ __forceinline__ void pair_general(PrefilterFloatParams const &p, Frame const &t, R const *base, PairEntry const &e, Sums &acc)
     {
-      f32x2 x, y, z;
-      direction_pair_proj(t, e, x, y, z);
-
-      float xa, xb, ya, yb, za, zb;
-      unpack2(x, xa, xb);
-      unpack2(y, ya, yb);
-      unpack2(z, za, zb);
-
-      float qua, qva, qub, qvb;
-      uint32_t fa, fb;
-      cube_select_unshrunk(xa, ya, za, qua, qva, fa);
-      cube_select_unshrunk(xb, yb, zb, qub, qvb, fb);
-
-      f32x2 qu = pack2(qua, qub), qv = pack2(qva, qvb);
-      f32x2 mu = fma2(qu, bcast2(p.geom.hw_shrunk), bcast2(p.geom.hwm_magic));
-      f32x2 mv = fma2(qv, bcast2(p.geom.hh_shrunk), bcast2(p.geom.hhm_magic));
-      f32x2 cu = add2(neg2(mu), bcast2(p.geom.hwm_magic));
-      f32x2 cv = add2(neg2(mv), bcast2(p.geom.hhm_magic));
-      f32x2 du = fma2(qu, bcast2(p.geom.hw_shrunk), cu);
-      f32x2 dv = fma2(qv, bcast2(p.geom.hh_shrunk), cv);
-
-      float ia, ib;
-      unpack2(fma2(cv, bcast2(p.geom.neg_ws), mu), ia, ib);
-
-      gather_pair(base, fa * p.geom.face_size + f2u(ia), fb * p.geom.face_size + f2u(ib), du, dv, e, acc);
-    }
-
-    // ---- tiles (prefilter_dn.cu: steal_tile, next_tile_plain, tile_texel) -------------------------------
-
-    __device__ __noinline__ int steal_tile(int *counters, int queues, int chunk, uint32_t smid, int lane)
-    {
-      const int own = (int)(smid % (uint32_t)queues);
-
-      for(int base = 1; base < queues; base += 32)
-      {
-        int i = base + lane;
-        int q = own + i;
-        if (q >= queues)
-          q -= queues;
-
-        bool holds = i < queues && *(volatile int const *)(counters + q) < chunk;
-
-        for(unsigned candidates = __ballot_sync(0xffffffffu, holds); candidates != 0u; candidates &= candidates - 1u)
-        {
-          int src = __ffs(candidates) - 1;
-          int k = -1;
-          if (lane == src)
-            k = atomicAdd(counters + q, 1);
-          k = __shfl_sync(0xffffffffu, k, src);
-
-          if (k < chunk)
-            return __shfl_sync(0xffffffffu, q, src) * chunk + k;
-        }
-      }
-
-      return -1;
-    }
-
-    __device__ __forceinline__ int next_tile_plain(PrefilterFloatParams const &p, uint32_t smid)
-    {
-      if ((int)smid < p.queues)
-      {
-        int k = atomicAdd(p.counters + smid, 1);
-        if (k < p.chunk)
-          return (int)smid * p.chunk + k;
-      }
-
-      int tile = p.queued + atomicAdd(p.counters + p.queues, 1);
-      return tile < p.tiles ? tile : -1;
-    }
-
-    __device__ __forceinline__ bool tile_texel(PrefilterFloatParams const &p, int tile, int lane, int &x, int &row)
-    {
-      int block = tile >> 4, in = tile & 15;
-      int bx = block % p.blocks_x, by = block / p.blocks_x;
-      x = (bx * 4 + (in & 3)) * 8 + (lane & 7);
-      row = p.row_begin + (by * 4 + (in >> 2)) * 4 + (lane >> 3);
-      return x < p.wd && row < p.row_end;
+      uint32_t ia, ib;
+      f32x2 du, dv;
+      pair_taps_general(p.geom, t, e, ia, ib, du, dv);
+      gather_pair(base, ia, ib, du, dv, e, acc);
     }
 
     // ---- epilogue ---------------------------------------------------------------------------
@@ -424,41 +283,8 @@ namespace ibl
         int face = row / p.hd;
 
         Frame st;
-        int n_same;
-        {
-          float const *f = p.frames + ((size_t)row * p.wd + x);
-          const size_t plane = (size_t)6 * p.hd * p.wd;
-          st.T = Vec3f{ __ldg(f + 0 * plane), __ldg(f + 1 * plane), __ldg(f + 2 * plane) };
-          st.B = Vec3f{ __ldg(f + 3 * plane), __ldg(f + 4 * plane), __ldg(f + 5 * plane) };
-          st.N = Vec3f{ __ldg(f + 6 * plane), __ldg(f + 7 * plane), __ldg(f + 8 * plane) };
-
-          // this warp's sector limit over the tile rows the slab's first row touches (prefilter_dp_kernel)
-          float limit;
-          {
-            const int tiles_x = (p.wd + 7) >> 3, tile_rows = (6 * p.hd + 3) >> 2;
-            const int top = __shfl_sync(0xffffffffu, row, 0), left = __shfl_sync(0xffffffffu, x, 0);
-            const int t0 = top >> 2, t1 = min((top + 3) >> 2, tile_rows - 1);
-            float const *tl = p.frames + 9 * plane + (left >> 3);
-            const size_t sector = (size_t)tile_rows * tiles_x;
-            const int first = NW == 8 ? warp : 2 * warp;
-
-            limit = fminf(__ldg(tl + first * sector + (size_t)t0 * tiles_x), __ldg(tl + first * sector + (size_t)t1 * tiles_x));
-            if (NW != 8)
-              limit = fminf(limit, fminf(__ldg(tl + (first + 1) * sector + (size_t)t0 * tiles_x), __ldg(tl + (first + 1) * sector + (size_t)t1 * tiles_x)));
-          }
-
-          float const *rho = p.sector_rho[SECTORS] + warp * bands;
-          int count = 0;
-          for(int base = 0; base < bands; base += 32)
-          {
-            int k = base + lane;
-            unsigned within = __ballot_sync(0xffffffffu, k < bands && __ldg(rho + k) <= limit);
-            count += __popc(within);
-            if (within != 0xffffffffu)
-              break;
-          }
-          n_same = count;
-        }
+        int n_same, n_same_second;
+        tile_frame_bands<NW, 1>(p, x, row, warp, lane, bands, st, n_same, n_same_second);
 
         Sums acc;
         acc.rg = 0ull;
@@ -495,28 +321,13 @@ namespace ibl
           }
         }
 
-        // ---- reduction over the CTA's warps: s_red[(warp*3 + c)*32 + lane] ----
-        float a[4];
-        unpack2(acc.rg, a[0], a[1]);
-        unpack2(acc.bb, a[2], a[3]);
-        a[2] += a[3];
-
-        #pragma unroll
-        for(int c = 0; c < 3; ++c)
-          s_red[(warp * 3 + c) * 32 + lane] = a[c];
-
+        store_warp_sums(acc, s_red, warp, lane);
         __syncthreads();
 
         if (warp == 0)
         {
-          float sum[3] = { 0.0f, 0.0f, 0.0f };
-          #pragma unroll
-          for(int w = 0; w < NW; ++w)
-          {
-            #pragma unroll
-            for(int c = 0; c < 3; ++c)
-              sum[c] += s_red[(w * 3 + c) * 32 + lane];
-          }
+          float sum[3];
+          add_warp_sums<NW>(s_red, lane, sum);
 
           if (valid)
             store_texel<FMT>(p, (size_t)row * p.wd + x, sum[0] * p.norm, sum[1] * p.norm, sum[2] * p.norm);
@@ -630,61 +441,29 @@ namespace ibl
       }
     }
 
-    // resident CTAs per SM for one kernel and dynamic shared-memory size (opt-in above 48 KB)
-    cudaError_t resident_ctas(void (*kernel)(PrefilterFloatParams), int threads, size_t smem, int *resident)
-    {
-      if (smem > 48 * 1024)
-      {
-        cudaError_t err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (err != cudaSuccess)
-          return err;
-      }
-
-      cudaError_t err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(resident, kernel, threads, smem);
-      if (err != cudaSuccess)
-        return err;
-      return *resident < 1 ? cudaErrorLaunchOutOfResources : cudaSuccess;
-    }
-
     template<int FMT, int NW, int MINB, bool SMEM_TABLE, bool QUEUES>
     cudaError_t launch_pair(PrefilterFloatParams p, int sm_count, cudaStream_t stream)
     {
       auto kernel = prefilter_float_pair_kernel<FMT, NW, MINB, SMEM_TABLE, QUEUES>;
 
-      int rows = p.row_end - p.row_begin;
-      int tiles_x = (p.wd + 7) / 8, tiles_y = (rows + 3) / 4;
-      p.blocks_x = (tiles_x + 3) / 4;
-      p.tiles = p.blocks_x * ((tiles_y + 3) / 4) * 16;
-
       const int table_bands = p.sector_bands[NW == 8 ? 1 : 0];
       size_t smem = (SMEM_TABLE ? (size_t)table_bands * kSectorShare * NW * sizeof(float4) : 0) + (size_t)NW * 3 * 32 * sizeof(float) + sizeof(int);
 
-      int resident = 0;
-      cudaError_t err = resident_ctas(kernel, 32 * NW, smem, &resident);
+      int grid = 0;
+      cudaError_t err = plan_tiles(p, kernel, 32 * NW, smem, 1, sm_count, &grid);
       if (err != cudaSuccess)
         return err;
-
-      int grid = p.tiles < sm_count * resident ? p.tiles : sm_count * resident;
-      if (grid < 1)
-        grid = 1;
-
-      // queues: 7/8 of the tiles in per-SM chunks, the rest in the common pool
-      p.queues = sm_count;
-      p.chunk = (p.tiles - p.tiles / 8) / sm_count;
-      p.queued = p.chunk * sm_count;
 
       kernel<<<grid, 32 * NW, smem, stream>>>(p);
       return cudaGetLastError();
     }
 
+    // the slab-size classes of launch_prefilter_dn
     template<int FMT>
     cudaError_t launch_pair_for(PrefilterFloatParams const &p, int sm_count, cudaStream_t stream)
     {
-      // the slab-size classes of launch_prefilter_dn: 4 warps per tile for the biggest slabs, 8 below;
-      // tile queues from kQueuedTexels up; a table beyond ~1100 entries is read through L1
       const size_t texels = (size_t)(p.row_end - p.row_begin) * p.wd;
-      const bool big_table = p.table_count > 1100;
-      const size_t kQueuedTexels = 32u * 148u * 8u, kFourWarpTexels = 160000u;
+      const bool big_table = p.table_count > kBigTableEntries;
 
       if (texels >= kFourWarpTexels)
         return big_table ? launch_pair<FMT, 4, 8, false, true>(p, sm_count, stream) : launch_pair<FMT, 4, 8, true, true>(p, sm_count, stream);
@@ -696,15 +475,13 @@ namespace ibl
     template<int FMT, bool PROJ>
     cudaError_t launch_tail_for(PrefilterFloatParams const &p, int texels, cudaStream_t stream)
     {
-      // warps per texel as in launch_prefilter_tail: cover the machine first, then depth
-      if (texels >= 4096 || p.table_count <= 128)
-        prefilter_float_tail_kernel<FMT, 4, PROJ><<<texels, 128, 0, stream>>>(p);
-      else if (texels >= 1024 || p.table_count <= 256)
-        prefilter_float_tail_kernel<FMT, 8, PROJ><<<texels, 256, 0, stream>>>(p);
-      else if (texels >= 256 || p.table_count <= 512)
-        prefilter_float_tail_kernel<FMT, 16, PROJ><<<texels, 512, 0, stream>>>(p);
-      else
-        prefilter_float_tail_kernel<FMT, 32, PROJ><<<texels, 1024, 0, stream>>>(p);
+      switch (tail_warps(texels, p.table_count))
+      {
+        case 4: prefilter_float_tail_kernel<FMT, 4, PROJ><<<texels, 128, 0, stream>>>(p); break;
+        case 8: prefilter_float_tail_kernel<FMT, 8, PROJ><<<texels, 256, 0, stream>>>(p); break;
+        case 16: prefilter_float_tail_kernel<FMT, 16, PROJ><<<texels, 512, 0, stream>>>(p); break;
+        default: prefilter_float_tail_kernel<FMT, 32, PROJ><<<texels, 1024, 0, stream>>>(p); break;
+      }
       return cudaGetLastError();
     }
   }
