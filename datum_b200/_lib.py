@@ -64,6 +64,8 @@ SIGNATURES = {
     "datum_ibl_buildmips_cube_float": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "datum_ibl_buildmips_cube_float_device": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
     "datum_ibl_prefilter_level_float_device": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "datum_ibl_bake_probes_float": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, ctypes.POINTER(c_void_p), c_void_p]),
+    "datum_ibl_multi_bake_probes_float": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, ctypes.POINTER(c_void_p), c_void_p]),
 }
 
 

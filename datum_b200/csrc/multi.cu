@@ -12,7 +12,7 @@
 //       handles) and whose last CTA bumps the peers' arrival counters; the streams wait on the counters.
 //       The host thread only enqueues: all devices run concurrently, nothing blocks until the end.
 //   probe batches (config 4)              probe p on device p % ndev, one host thread per device around
-//       datum_ibl_bake_probes; no data-path exchange.
+//       datum_ibl_bake_probes or datum_ibl_bake_probes_float; no data-path exchange.
 //   SH9 of one cube (config 5)            rows split, 28 partial sums per device added on the host.
 //
 // A device may appear more than once in the list (two contexts on one GPU): that is how the exchange
@@ -107,6 +107,55 @@ namespace
 
   uint32_t *chain_of(datum_ibl_multi *m, size_t d) { return reinterpret_cast<uint32_t*>(m->shared[d] + DATUM_IBL_PEER_FLAG_BYTES); }
   uint32_t *flags_of(datum_ibl_multi *m, size_t d) { return reinterpret_cast<uint32_t*>(m->shared[d]); }
+
+  // Probe batches (config 4): probe p on device p % ndev; each device's share is one synchronous batched call
+  // bake(ctx, n, payloads, sh) on its own host thread.  One device, or at most one probe: the first device's call.
+  template<typename Bake>
+  int shard_probes(datum_ibl_multi *m, const char *who, int count, void *const *payloads, float *sh, Bake bake)
+  {
+    if (!m || (count > 0 && !payloads))
+      return fail(std::string(who) + ": null argument");
+    if (count < 0)
+      return fail(std::string(who) + ": bad count");
+
+    const int world = (int)m->devices.size();
+
+    if (world == 1 || count <= 1)
+      return bake(m->ctx[0], count, payloads, sh);
+
+    std::vector<std::vector<void*>> mine(world);
+    for(int p = 0; p < count; ++p)
+      mine[p % world].push_back(payloads[p]);
+
+    std::vector<std::vector<float>> mine_sh(world);
+    std::vector<std::string> errors(world);
+    std::vector<std::thread> workers;
+
+    for(int d = 0; d < world; ++d)
+    {
+      if (sh)
+        mine_sh[d].resize(mine[d].size() * 27);
+
+      workers.emplace_back([&, d] {
+        if (mine[d].empty())
+          return;
+        if (bake(m->ctx[d], (int)mine[d].size(), mine[d].data(), sh ? mine_sh[d].data() : nullptr))
+          errors[d] = datum_ibl_last_error();       // thread-local text of the worker
+      });
+    }
+
+    for(auto &w : workers)
+      w.join();
+
+    for(int d = 0; d < world; ++d)
+      if (!errors[d].empty())
+        return fail(std::string(who) + ": device " + std::to_string(m->devices[d]) + ": " + errors[d]);
+
+    for(int p = 0; sh && p < count; ++p)
+      std::memcpy(sh + (size_t)p * 27, mine_sh[p % world].data() + (size_t)(p / world) * 27, 27 * sizeof(float));
+
+    return 0;
+  }
 }
 
 extern "C"
@@ -335,49 +384,18 @@ extern "C"
 
   int datum_ibl_multi_bake_probes(datum_ibl_multi *m, int count, int width, int height, int levels, int samples, void *const *bits, float *sh)
   {
-    if (!m || (count > 0 && !bits))
-      return fail("datum_ibl_multi_bake_probes: null argument");
-    if (count < 0)
-      return fail("datum_ibl_multi_bake_probes: bad count");
-
-    const int world = (int)m->devices.size();
-
-    if (world == 1 || count <= 1)
-      return datum_ibl_bake_probes(m->ctx[0], count, width, height, levels, samples, bits, sh);
-
-    // probe p on device p % world; each device's share is one synchronous batched call on its own host thread
-    std::vector<std::vector<void*>> mine(world);
-    for(int p = 0; p < count; ++p)
-      mine[p % world].push_back(bits[p]);
-
-    std::vector<std::vector<float>> mine_sh(world);
-    std::vector<std::string> errors(world);
-    std::vector<std::thread> workers;
-
-    for(int d = 0; d < world; ++d)
+    return shard_probes(m, "datum_ibl_multi_bake_probes", count, bits, sh, [&](datum_ibl_ctx *ctx, int n, void *const *mine, float *mine_sh)
     {
-      if (sh)
-        mine_sh[d].resize(mine[d].size() * 27);
+      return datum_ibl_bake_probes(ctx, n, width, height, levels, samples, mine, mine_sh);
+    });
+  }
 
-      workers.emplace_back([&, d] {
-        if (mine[d].empty())
-          return;
-        if (datum_ibl_bake_probes(m->ctx[d], (int)mine[d].size(), width, height, levels, samples, mine[d].data(), sh ? mine_sh[d].data() : nullptr))
-          errors[d] = datum_ibl_last_error();       // thread-local text of the worker
-      });
-    }
-
-    for(auto &w : workers)
-      w.join();
-
-    for(int d = 0; d < world; ++d)
-      if (!errors[d].empty())
-        return fail("datum_ibl_multi_bake_probes: device " + std::to_string(m->devices[d]) + ": " + errors[d]);
-
-    for(int p = 0; sh && p < count; ++p)
-      std::memcpy(sh + (size_t)p * 27, mine_sh[p % world].data() + (size_t)(p / world) * 27, 27 * sizeof(float));
-
-    return 0;
+  int datum_ibl_multi_bake_probes_float(datum_ibl_multi *m, int format, int count, int width, int height, int levels, int samples, void *const *chains, float *sh)
+  {
+    return shard_probes(m, "datum_ibl_multi_bake_probes_float", count, chains, sh, [&](datum_ibl_ctx *ctx, int n, void *const *mine, float *mine_sh)
+    {
+      return datum_ibl_bake_probes_float(ctx, format, n, width, height, levels, samples, mine, mine_sh);
+    });
   }
 
   int datum_ibl_multi_project_sh9(datum_ibl_multi *m, void const *level0, int format, int width, int height, float *sh)

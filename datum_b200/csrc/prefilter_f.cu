@@ -17,6 +17,12 @@
 // The pair kernel shares its device helpers with prefilter_dn.cu (prefilter_pair.cuh): packed fp32 ops, pair
 // entries, projective footprint coordinates, tile hand-out, per-tile frame and same-face band count, CTA
 // reduction.  The launchers share resident_ctas, plan_tiles, the slab-size classes and tail_warps (prefilter.h).
+//
+// Batches (datum_ibl_bake_probes_float): the record pass, the pair kernel and the tail kernel also compute the
+// same level of several chains in one launch, like the rgbe kernels, in instantiations of their own (BATCH):
+// the single-probe kernels compile none of the batch code.  Launch shapes that decide the order of the sums
+// (warps per tile, warps per texel) follow ONE probe's slab, so every probe of a batch gets the bytes of a
+// single call; only the tile queues and the grid follow the whole launch.
 
 #include "prefilter.h"
 #include "prefilter_f.h"
@@ -34,15 +40,22 @@ namespace ibl
 
     // ---- records --------------------------------------------------------------------------
 
-    template<int FMT>
-    __global__ void __launch_bounds__(256) build_float_records_kernel(void const *__restrict__ src, void *__restrict__ rec, int ws, int hs, int *__restrict__ counters, int ncounters)
+    // BATCH: blockIdx.y = probe, source levels src_stride texels apart, their records back to back
+    template<int FMT, bool BATCH>
+    __device__ __forceinline__ void build_float_records(void const *__restrict__ src, void *__restrict__ rec, int ws, int hs, size_t src_stride, int *__restrict__ counters, int ncounters)
     {
       // the prefilter launch that follows on the stream takes its tiles from these queues
-      if (blockIdx.x == 0)
+      if (blockIdx.x == 0 && (!BATCH || blockIdx.y == 0))
         for(int i = threadIdx.x; i < ncounters; i += blockDim.x)
           counters[i] = 0;
 
       const uint32_t level = 6u * (uint32_t)ws * (uint32_t)hs;
+
+      if (BATCH)
+      {
+        src = static_cast<unsigned char const*>(src) + (size_t)blockIdx.y * src_stride * float_texel_bytes(FMT);
+        rec = static_cast<unsigned char*>(rec) + (size_t)blockIdx.y * level * sizeof(typename RecordOf<FMT>::type);
+      }
 
       for(uint32_t idx = blockIdx.x * blockDim.x + threadIdx.x; idx < level; idx += gridDim.x * blockDim.x)
       {
@@ -70,6 +83,20 @@ namespace ibl
           r[2] = make_float4(t2.z, t3.x, t3.y, t3.z);
         }
       }
+    }
+
+    // one chain, and the same level of several chains (separate kernels: the single-probe one compiles none of
+    // the batch code)
+    template<int FMT>
+    __global__ void __launch_bounds__(256) build_float_records_kernel(void const *__restrict__ src, void *__restrict__ rec, int ws, int hs, int *__restrict__ counters, int ncounters)
+    {
+      build_float_records<FMT, false>(src, rec, ws, hs, 0, counters, ncounters);
+    }
+
+    template<int FMT>
+    __global__ void __launch_bounds__(256) build_float_records_batch_kernel(void const *__restrict__ src, void *__restrict__ rec, int ws, int hs, size_t src_stride, int *__restrict__ counters, int ncounters)
+    {
+      build_float_records<FMT, true>(src, rec, ws, hs, src_stride, counters, ncounters);
     }
 
     // ---- taps -----------------------------------------------------------------------------
@@ -199,7 +226,9 @@ namespace ibl
     //
     // CTA = NW warps sharing one 8x4 tile; warp w reads azimuth sector w of every band of the sector table,
     // its leading bands without face selection as long as they provably stay on the texel's face.
-    template<int FMT, int NW, int MINB, bool SMEM_TABLE, bool QUEUES>
+    // BATCH: the same level of p.probes chains, tiles numbered probe by probe (prefilter_dp_kernel's batches).
+    // The single-probe instantiations compile none of the batch code.
+    template<int FMT, int NW, int MINB, bool SMEM_TABLE, bool QUEUES, bool BATCH = false>
     __global__ void __launch_bounds__(32 * NW, MINB) prefilter_float_pair_kernel(PrefilterFloatParams p)
     {
       typedef typename RecordOf<FMT>::type R;
@@ -268,8 +297,16 @@ namespace ibl
         if (tile < 0)
           break;
 
+        // a batch: which probe, and the tile within that probe's slab
+        int probe = 0, ltile = tile;
+        if (BATCH)
+        {
+          probe = tile / p.tiles_per_probe;
+          ltile = tile - probe * p.tiles_per_probe;
+        }
+
         int x, row;
-        bool valid = tile_texel(p, tile, lane, x, row);
+        bool valid = tile_texel(p, ltile, lane, x, row);
 
         if (__ballot_sync(0xffffffffu, valid) == 0u)
         {
@@ -292,8 +329,11 @@ namespace ibl
 
         float4 const *tw = table + warp * PER;
 
+        // this probe's records (a batch: the probes' records back to back)
+        R const *biased_probe = BATCH ? opaque(biased + (size_t)probe * p.record_stride) : biased;
+
         {
-          R const *base = opaque(biased + (size_t)face * p.geom.face_size);
+          R const *base = opaque(biased_probe + (size_t)face * p.geom.face_size);
 
           #pragma unroll BAND_UNROLL
           for(int band = 0; band < n_same; ++band)
@@ -310,7 +350,7 @@ namespace ibl
           st.B = from_face_local(face, unfold_face_row(p.geom, st.B));
           st.N = from_face_local(face, unfold_face_row(p.geom, st.N));
 
-          R const *general = opaque(biased + (size_t)(kMagicBits - p.geom.bias_general));
+          R const *general = opaque(biased_probe + (size_t)(kMagicBits - p.geom.bias_general));
 
           #pragma unroll BAND_UNROLL
           for(int band = n_same; band < bands; ++band)
@@ -330,7 +370,7 @@ namespace ibl
           add_warp_sums<NW>(s_red, lane, sum);
 
           if (valid)
-            store_texel<FMT>(p, (size_t)row * p.wd + x, sum[0] * p.norm, sum[1] * p.norm, sum[2] * p.norm);
+            store_texel<FMT>(p, (size_t)row * p.wd + x + (BATCH ? (size_t)probe * p.dst_stride : (size_t)0), sum[0] * p.norm, sum[1] * p.norm, sum[2] * p.norm);
         }
 
         __syncthreads();
@@ -338,7 +378,9 @@ namespace ibl
     }
 
     // ---- the tail kernel: one CTA per texel, lanes are samples (prefilter_tail_kernel) ----------------
-    template<int FMT, int NW, bool PROJ>
+    // BATCH: the same level of p.probes chains, blockIdx.x runs over the texels probe by probe (batches run only
+    // where every source is proj_usable, prefilter_batchable: PROJ)
+    template<int FMT, int NW, bool PROJ, bool BATCH = false>
     __global__ void __launch_bounds__(32 * NW) prefilter_float_tail_kernel(PrefilterFloatParams p)
     {
       __shared__ float s_red[NW][3];
@@ -346,7 +388,14 @@ namespace ibl
 
       const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 
-      const int texel = blockIdx.x;
+      int texel = blockIdx.x, probe = 0;
+      if (BATCH)
+      {
+        probe = texel / p.texels_per_probe;
+        texel -= probe * p.texels_per_probe;
+      }
+      void const *src = BATCH ? static_cast<unsigned char const*>(p.src) + (size_t)probe * p.src_stride * float_texel_bytes(FMT) : p.src;
+
       const int row = p.row_begin + texel / p.wd;
       const int x = texel - (texel / p.wd) * p.wd;
       const int face = row / p.hd;
@@ -408,7 +457,7 @@ namespace ibl
         for(int k = 0; k < 4; ++k)
         {
           float c[3];
-          load_texel<FMT>(p.src, tap[k], c);
+          load_texel<FMT>(src, tap[k], c);
           float_accumulate_tap(c[0], c[1], c[2], w[k], acc);
         }
       }
@@ -437,79 +486,116 @@ namespace ibl
             sum[c] += s_red[w][c];
         }
 
-        store_texel<FMT>(p, (size_t)row * p.wd + x, sum[0] * p.norm, sum[1] * p.norm, sum[2] * p.norm);
+        store_texel<FMT>(p, (size_t)row * p.wd + x + (BATCH ? (size_t)probe * p.dst_stride : (size_t)0), sum[0] * p.norm, sum[1] * p.norm, sum[2] * p.norm);
       }
     }
 
-    template<int FMT, int NW, int MINB, bool SMEM_TABLE, bool QUEUES>
+    template<int FMT, int NW, int MINB, bool SMEM_TABLE, bool QUEUES, bool BATCH>
     cudaError_t launch_pair(PrefilterFloatParams p, int sm_count, cudaStream_t stream)
     {
-      auto kernel = prefilter_float_pair_kernel<FMT, NW, MINB, SMEM_TABLE, QUEUES>;
+      auto kernel = prefilter_float_pair_kernel<FMT, NW, MINB, SMEM_TABLE, QUEUES, BATCH>;
 
       const int table_bands = p.sector_bands[NW == 8 ? 1 : 0];
       size_t smem = (SMEM_TABLE ? (size_t)table_bands * kSectorShare * NW * sizeof(float4) : 0) + (size_t)NW * 3 * 32 * sizeof(float) + sizeof(int);
 
       int grid = 0;
-      cudaError_t err = plan_tiles(p, kernel, 32 * NW, smem, 1, sm_count, &grid);
+      cudaError_t err = plan_tiles(p, kernel, 32 * NW, smem, p.probes, sm_count, &grid);
       if (err != cudaSuccess)
         return err;
+      p.tiles_per_probe = p.tiles / p.probes;
 
       kernel<<<grid, 32 * NW, smem, stream>>>(p);
       return cudaGetLastError();
     }
 
-    // the slab-size classes of launch_prefilter_dn
+    template<int FMT, int NW, int MINB, bool QUEUES, bool BATCH>
+    cudaError_t launch_pair_table(PrefilterFloatParams const &p, int sm_count, cudaStream_t stream)
+    {
+      return p.table_count > kBigTableEntries ? launch_pair<FMT, NW, MINB, false, QUEUES, BATCH>(p, sm_count, stream) : launch_pair<FMT, NW, MINB, true, QUEUES, BATCH>(p, sm_count, stream);
+    }
+
+    // The slab-size classes of launch_prefilter_dn.  Warps per tile follow ONE probe's slab (they decide the
+    // order of the sums: a batch must give the bytes of single calls), the tile queues the whole launch.
+    template<int FMT, bool BATCH>
+    cudaError_t launch_pair_shape(PrefilterFloatParams const &p, int sm_count, cudaStream_t stream)
+    {
+      const size_t texels = (size_t)(p.row_end - p.row_begin) * p.wd;
+
+      if (texels >= kFourWarpTexels)
+        return launch_pair_table<FMT, 4, 8, true, BATCH>(p, sm_count, stream);
+      if (texels * (size_t)p.probes >= kQueuedTexels)
+        return launch_pair_table<FMT, 8, 4, true, BATCH>(p, sm_count, stream);
+      return launch_pair_table<FMT, 8, 4, false, BATCH>(p, sm_count, stream);
+    }
+
     template<int FMT>
     cudaError_t launch_pair_for(PrefilterFloatParams const &p, int sm_count, cudaStream_t stream)
     {
-      const size_t texels = (size_t)(p.row_end - p.row_begin) * p.wd;
-      const bool big_table = p.table_count > kBigTableEntries;
-
-      if (texels >= kFourWarpTexels)
-        return big_table ? launch_pair<FMT, 4, 8, false, true>(p, sm_count, stream) : launch_pair<FMT, 4, 8, true, true>(p, sm_count, stream);
-      if (texels >= kQueuedTexels)
-        return big_table ? launch_pair<FMT, 8, 4, false, true>(p, sm_count, stream) : launch_pair<FMT, 8, 4, true, true>(p, sm_count, stream);
-      return big_table ? launch_pair<FMT, 8, 4, false, false>(p, sm_count, stream) : launch_pair<FMT, 8, 4, true, false>(p, sm_count, stream);
+      return p.probes > 1 ? launch_pair_shape<FMT, true>(p, sm_count, stream) : launch_pair_shape<FMT, false>(p, sm_count, stream);
     }
 
+    template<int NW, int FMT, bool PROJ>
+    void launch_tail(PrefilterFloatParams const &p, int grid, cudaStream_t stream)
+    {
+      if (p.probes > 1)
+        prefilter_float_tail_kernel<FMT, NW, true, true><<<grid, 32 * NW, 0, stream>>>(p);
+      else
+        prefilter_float_tail_kernel<FMT, NW, PROJ><<<grid, 32 * NW, 0, stream>>>(p);
+    }
+
+    // warps per texel (tail_warps) chosen from ONE probe's texels also when a launch carries several
     template<int FMT, bool PROJ>
     cudaError_t launch_tail_for(PrefilterFloatParams const &p, int texels, cudaStream_t stream)
     {
+      const int grid = texels * p.probes;
       switch (tail_warps(texels, p.table_count))
       {
-        case 4: prefilter_float_tail_kernel<FMT, 4, PROJ><<<texels, 128, 0, stream>>>(p); break;
-        case 8: prefilter_float_tail_kernel<FMT, 8, PROJ><<<texels, 256, 0, stream>>>(p); break;
-        case 16: prefilter_float_tail_kernel<FMT, 16, PROJ><<<texels, 512, 0, stream>>>(p); break;
-        default: prefilter_float_tail_kernel<FMT, 32, PROJ><<<texels, 1024, 0, stream>>>(p); break;
+        case 4: launch_tail<4, FMT, PROJ>(p, grid, stream); break;
+        case 8: launch_tail<8, FMT, PROJ>(p, grid, stream); break;
+        case 16: launch_tail<16, FMT, PROJ>(p, grid, stream); break;
+        default: launch_tail<32, FMT, PROJ>(p, grid, stream); break;
       }
       return cudaGetLastError();
     }
   }
 
-  cudaError_t launch_build_float_records(int format, void const *src, void *records, int ws, int hs, int *counters, int ncounters, int sm_count, cudaStream_t stream)
+  cudaError_t launch_build_float_records(int format, void const *src, void *records, int ws, int hs, int probes, size_t src_stride, int *counters, int ncounters, int sm_count, cudaStream_t stream)
   {
+    if (probes < 1)
+      probes = 1;
+
     size_t level = (size_t)6 * ws * hs;
     size_t blocks = (level + 255) / 256;
-    size_t cap = (size_t)sm_count * 8;
+    size_t cap = ((size_t)sm_count * 8 + probes - 1) / probes;
     int grid = (int)(blocks < cap ? blocks : cap);
     if (grid < 1)
       grid = 1;
 
-    if (format == kFloatFormatF16)
+    const dim3 cubes(grid, probes);
+    if (format == kFloatFormatF16 && probes == 1)
       build_float_records_kernel<kFloatFormatF16><<<grid, 256, 0, stream>>>(src, records, ws, hs, counters, ncounters);
-    else if (format == kFloatFormatF32)
+    else if (format == kFloatFormatF32 && probes == 1)
       build_float_records_kernel<kFloatFormatF32><<<grid, 256, 0, stream>>>(src, records, ws, hs, counters, ncounters);
+    else if (format == kFloatFormatF16)
+      build_float_records_batch_kernel<kFloatFormatF16><<<cubes, 256, 0, stream>>>(src, records, ws, hs, src_stride, counters, ncounters);
+    else if (format == kFloatFormatF32)
+      build_float_records_batch_kernel<kFloatFormatF32><<<cubes, 256, 0, stream>>>(src, records, ws, hs, src_stride, counters, ncounters);
     else
       return cudaErrorInvalidValue;
     return cudaGetLastError();
   }
 
-  cudaError_t launch_prefilter_float(PrefilterFloatParams const &p, int sm_count, cudaStream_t stream)
+  cudaError_t launch_prefilter_float(PrefilterFloatParams const &params, int sm_count, cudaStream_t stream)
   {
+    PrefilterFloatParams p = params;
     if (p.row_end <= p.row_begin || p.wd <= 0)
       return cudaSuccess;
     if (!proj_usable(p.geom.ws, p.geom.hs) || !p.frames || !p.table_sector[0] || !p.table_sector[1])
       return cudaErrorInvalidValue;
+    if (p.probes < 1)
+      p.probes = 1;
+    if (p.probes > 1 && p.dst_f32)
+      return cudaErrorNotSupported;       // batches store the format's texels only
 
     if (p.format == kFloatFormatF16)
       return launch_pair_for<kFloatFormatF16>(p, sm_count, stream);
@@ -518,13 +604,21 @@ namespace ibl
     return cudaErrorInvalidValue;
   }
 
-  cudaError_t launch_prefilter_float_tail(PrefilterFloatParams const &p, cudaStream_t stream)
+  cudaError_t launch_prefilter_float_tail(PrefilterFloatParams const &params, cudaStream_t stream)
   {
+    PrefilterFloatParams p = params;
     int texels = (p.row_end - p.row_begin) * p.wd;
     if (texels <= 0)
       return cudaSuccess;
 
+    if (p.probes < 1)
+      p.probes = 1;
+    p.texels_per_probe = texels;
+
     const bool proj = proj_usable(p.geom.ws, p.geom.hs);
+    if (p.probes > 1 && (p.dst_f32 || !proj))
+      return cudaErrorNotSupported;       // batches: texels of the format, proj_usable sources (prefilter_batchable)
+
     if (p.format == kFloatFormatF16)
       return proj ? launch_tail_for<kFloatFormatF16, true>(p, texels, stream) : launch_tail_for<kFloatFormatF16, false>(p, texels, stream);
     if (p.format == kFloatFormatF32)

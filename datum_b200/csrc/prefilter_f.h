@@ -141,15 +141,23 @@ namespace ibl
     int *counters;              // queues+1 tile queue heads, zeroed by launch_build_float_records
     int blocks_x, tiles;        // filled by the launcher
     int queues, chunk, queued;
+
+    // the same level of `probes` chains in one launch (datum_ibl_bake_probes_float); 0 or 1: one chain.
+    // Strides in units of the format: src_stride and dst_stride in TEXELS between the probes' source and
+    // destination levels, record_stride in RECORDS (F16Record / F32Record) between their record sets
+    // (launch_build_float_records writes them back to back: 6*ws*hs).  dst_f32 must be null.
+    int probes, tiles_per_probe, texels_per_probe;    // the last two filled by the launchers
+    size_t src_stride, record_stride, dst_stride;
   };
 
-  // records of a ws x hs source level; also zeroes the `ncounters` tile queue heads
-  cudaError_t launch_build_float_records(int format, void const *src, void *records, int ws, int hs, int *counters, int ncounters, int sm_count, cudaStream_t stream);
+  // records of the ws x hs source levels of `probes` chains (src_stride texels apart; records back to back);
+  // also zeroes the `ncounters` tile queue heads
+  cudaError_t launch_build_float_records(int format, void const *src, void *records, int ws, int hs, int probes, size_t src_stride, int *counters, int ncounters, int sm_count, cudaStream_t stream);
 
   // pair kernel (proj_usable sources, slabs above kTailTexels, levels at least 8 wide)
   cudaError_t launch_prefilter_float(PrefilterFloatParams const &p, int sm_count, cudaStream_t stream);
 
-  // one CTA per destination texel, lanes are samples; any source size
+  // one CTA per destination texel, lanes are samples; any source size (a batch: proj_usable sources only)
   cudaError_t launch_prefilter_float_tail(PrefilterFloatParams const &p, cudaStream_t stream);
 #endif
 }

@@ -4,8 +4,8 @@
 // What both chains compute alike lives here: the packed fp32 ops, the pair table entries and the projective
 // footprint coordinates of two samples, the tile hand-out, and the per-tile frame, same-face band count and
 // CTA reduction.  What differs between the chains stays in each kernel: the record layout, the tap fetch and
-// decode, the store and (rgbe only) batches, peers and the arrival signal.  Nothing here depends on which chain
-// calls it.
+// decode, the store, the batch addressing (probe strides) and (rgbe only) peers and the arrival signal.  Nothing
+// here depends on which chain calls it.
 //
 // The rgbe kernels are sensitive to everything compiled into their bodies (DESIGN.md §4.1): these helpers keep
 // the statement order of the code they replace, and take output references rather than returning structs,

@@ -90,6 +90,20 @@ def _check_dtype(buf, dtype, what):
         raise ValueError("%s must hold %s texels, not %s" % (what, dtype.name, got))
 
 
+def _float_chain_pointers(fmt, width, height, levels, chains):
+    """ctypes array of the host chains of a float batch, every one checked for dtype and size."""
+    dtype = _float_dtype(fmt)
+    need = float_chain_texels(width, height, levels) * _texel_bytes(fmt)
+    pointers = (ctypes.c_void_p * max(len(chains), 1))()
+    for i, chain in enumerate(chains):
+        what = "chains[%d]" % i
+        if hasattr(chain, "is_cuda") and chain.is_cuda:
+            raise ValueError("%s must be a host buffer" % what)
+        _check_dtype(chain, dtype, what)
+        pointers[i] = _host_pointer(chain, need, what)
+    return pointers
+
+
 def _host_pointer(buf, min_bytes, what):
     """Address of a writable, contiguous host buffer (numpy array or CPU torch tensor)."""
     if isinstance(buf, np.ndarray):
@@ -277,6 +291,17 @@ class IblContext:
             _check_dtype(chain, _float_dtype(fmt), "chain")
         ptr = _host_pointer(chain, float_chain_texels(width, height, levels) * _texel_bytes(fmt), "chain")
         self._check(self._lib.datum_ibl_buildmips_cube_float(self._handle, fmt, width, height, levels, samples, ptr))
+
+    def bake_probes_float(self, fmt, width, height, levels, chains, samples=1024, sh9=False):
+        """A batch of float chains (datum_ibl_bake_probes_float): every chain is a host array of the format's
+        dtype used like the `chain` of buildmips_cube_float, and ends with the same bytes; small probes share
+        launches, and uploads, kernels and downloads of consecutive probes overlap (fully when the chains are
+        pinned).  With sh9=True returns the SH9 projection of every level 0 as a (count, 9, 3) float32 array."""
+        count = len(chains)
+        pointers = _float_chain_pointers(fmt, width, height, levels, chains)
+        sh = np.zeros((count, 9, 3), np.float32) if sh9 else None
+        self._check(self._lib.datum_ibl_bake_probes_float(self._handle, fmt, count, width, height, levels, samples, pointers, sh.ctypes.data if sh9 and count else None))
+        return sh
 
     def buildmips_cube_float_device(self, fmt, width, height, levels, d_chain, samples=1024, d_f32=None):
         """The same chain on a device-resident CUDA tensor of the format's dtype; asynchronous on the
@@ -512,6 +537,14 @@ class MultiContext:
             pointers[i] = _host_pointer(payload, need, "payloads[%d]" % i)
         sh = np.zeros((count, 9, 3), np.float32) if sh9 else None
         self._check(self._lib.datum_ibl_multi_bake_probes(self._handle, count, width, height, levels, samples, pointers, sh.ctypes.data if sh9 and count else None))
+        return sh
+
+    def bake_probes_float(self, fmt, width, height, levels, chains, samples=1024, sh9=False):
+        """IblContext.bake_probes_float with probe p on devices[p % ndev]."""
+        count = len(chains)
+        pointers = _float_chain_pointers(fmt, width, height, levels, chains)
+        sh = np.zeros((count, 9, 3), np.float32) if sh9 else None
+        self._check(self._lib.datum_ibl_multi_bake_probes_float(self._handle, fmt, count, width, height, levels, samples, pointers, sh.ctypes.data if sh9 and count else None))
         return sh
 
     def project_sh9(self, level0, fmt, width, height):

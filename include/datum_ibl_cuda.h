@@ -321,6 +321,19 @@ int datum_ibl_buildmips_cube_float_device(datum_ibl_ctx *ctx, int format, int wi
 /* One level of a float chain, rows [row_begin, row_end) of the destination; device pointers, asynchronous. */
 int datum_ibl_prefilter_level_float_device(datum_ibl_ctx *ctx, int format, void const *d_src, int ws, int hs, int level, int levels, int samples, int row_begin, int row_end, void *d_dst, float *d_dst_f32);
 
+/*
+ * datum_ibl_bake_probes for float chains: chains[i] is the i-th host chain (pageable or pinned), all of the same
+ * format, width/height/levels, laid out and level 0 pre-filled as for datum_ibl_buildmips_cube_float.  `sh`
+ * (optional, may be NULL) receives the SH9 projection of every level 0 as read in the chain's format,
+ * count x float[9][3].  Every chain's bytes are those of a single datum_ibl_buildmips_cube_float call; small
+ * probes share launches and the uploads, kernels and downloads of consecutive groups overlap as in
+ * datum_ibl_bake_probes.  Synchronous.
+ */
+int datum_ibl_bake_probes_float(datum_ibl_ctx *ctx, int format, int count, int width, int height, int levels, int samples, void *const *chains, float *sh);
+
+/* datum_ibl_bake_probes_float with probe p on devices[p % ndev] (see datum_ibl_multi_bake_probes); results identical to one device's */
+int datum_ibl_multi_bake_probes_float(datum_ibl_multi *multi, int format, int count, int width, int height, int levels, int samples, void *const *chains, float *sh);
+
 #ifdef __cplusplus
 }
 #endif
