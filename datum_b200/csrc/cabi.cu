@@ -318,11 +318,12 @@ namespace
     return slot;
   }
 
-  // the GPUs sharing a probe: where this slab's words also go, and whom to tell when all are stored
+  // the GPUs sharing a probe: where this slab's texels also go (the destination level in each peer's chain: rgbe
+  // words or texels of a float chain's format), and whom to tell when all are stored
   struct PeerTargets
   {
     int count = 0;
-    uint32_t *words[ibl::kMaxPeers] = {};
+    void *dst[ibl::kMaxPeers] = {};
     unsigned int *arrive[ibl::kMaxPeers] = {};   // null: no signal from the kernel
   };
 
@@ -497,7 +498,7 @@ namespace
     p.dst_f32 = d_dst_f32;
     p.peers = peers.count;
     for(int k = 0; k < peers.count; ++k)
-      p.peer_words[k] = peers.words[k];
+      p.peer_words[k] = static_cast<uint32_t*>(peers.dst[k]);
     if (fill_signal(ctx, peers, p.signal))
       return 1;
     p.wd = wd;
@@ -558,7 +559,7 @@ namespace
       p.dst_f32 = d_dst_f32;
       p.peers = peers.count;
       for(int k = 0; k < peers.count; ++k)
-        p.peer_words[k] = peers.words[k];
+        p.peer_words[k] = static_cast<uint32_t*>(peers.dst[k]);
       if (fill_signal(ctx, peers, p.signal))
         return 1;
       p.wd = wd;
@@ -983,8 +984,9 @@ namespace
 
   // one level of a float chain on the context's stream.  The pair kernel takes slabs above kTailTexels of
   // levels at least a tile wide whose source it can address (proj_usable); everything else runs the tail kernel.
-  // A batch computes the level of batch.probes chains in one launch (no d_dst_f32).
-  int run_level_float(datum_ibl_ctx *ctx, int format, void const *d_src, int ws, int hs, DeviceTable const &table, int row_begin, int row_end, void *d_dst, float *d_dst_f32, bool record_dominant, Batch const &batch = Batch())
+  // Peers: the slab also goes into their chains and the launch signals them (no d_dst_f32).  A batch computes the
+  // level of batch.probes chains in one launch (no d_dst_f32, no peers).
+  int run_level_float(datum_ibl_ctx *ctx, int format, void const *d_src, int ws, int hs, DeviceTable const &table, int row_begin, int row_end, void *d_dst, float *d_dst_f32, bool record_dominant, PeerTargets const &peers = PeerTargets(), Batch const &batch = Batch())
   {
     int wd = ws >> 1, hd = hs >> 1;
 
@@ -1014,6 +1016,11 @@ namespace
     p.src_stride = batch.stride;
     p.dst_stride = batch.stride;
     p.record_stride = (size_t)6 * ws * hs;
+    p.peers = peers.count;
+    for(int k = 0; k < peers.count; ++k)
+      p.peer_dst[k] = peers.dst[k];
+    if (fill_signal(ctx, peers, p.signal))
+      return 1;
 
     const bool tail = (size_t)(row_end - row_begin) * wd <= (size_t)ibl::kTailTexels || wd < 8 || !ibl::proj_usable(ws, hs);
     cudaError_t err = cudaSuccess;
@@ -1075,7 +1082,7 @@ namespace
     {
       int hd = height >> 1;
 
-      if (run_level_float(ctx, format, src, width, height, (*tables)[level], 0, 6 * hd, dst, d_f32, level == 1, batch))
+      if (run_level_float(ctx, format, src, width, height, (*tables)[level], 0, 6 * hd, dst, d_f32, level == 1, PeerTargets(), batch))
         return 1;
 
       size_t outcount = (size_t)(width >> 1) * hd * 6;
@@ -1822,7 +1829,7 @@ extern "C"
         return fail("datum_ibl_prefilter_level_peers: null pointer for a rank");
       if (r != rank)
       {
-        peers.words[peers.count] = d_dst_words[r];
+        peers.dst[peers.count] = d_dst_words[r];
         peers.arrive[peers.count] = d_flags ? reinterpret_cast<unsigned int*>(d_flags[r] + (epoch & 1u)) : nullptr;
         peers.count += 1;
       }
@@ -1841,6 +1848,55 @@ extern "C"
         return 1;
     }
     else if (run_level(ctx, d_src, ws, hs, (*tables)[level], row_begin, row_end, d_dst_words[rank], nullptr, false, peers))
+      return 1;
+
+    return d_flags ? wait_for_arrivals(ctx, d_flags[rank], epoch, world) : 0;
+  }
+
+  int datum_ibl_prefilter_level_float_peers(datum_ibl_ctx *ctx, int format, void const *d_src, int ws, int hs, int level, int levels, int samples, int row_begin, int row_end, int rank, int world, void *const *d_dst, uint32_t *const *d_flags, uint32_t epoch)
+  {
+    if (!ctx || !d_src || !d_dst)
+      return fail("datum_ibl_prefilter_level_float_peers: null argument");
+    if (!float_format(format))
+      return fail("datum_ibl_prefilter_level_float_peers: unknown format " + std::to_string(format) + " (DATUM_IBL_FORMAT_F32 or DATUM_IBL_FORMAT_F16)");
+    if (levels < 2 || levels > 16 || level < 1 || level >= levels || samples < 1 || samples > kFloatMaxSamples)
+      return fail("datum_ibl_prefilter_level_float_peers: bad level/levels/samples");
+    if (world < 1 || world > DATUM_IBL_MAX_PEERS + 1 || rank < 0 || rank >= world)
+      return fail("datum_ibl_prefilter_level_float_peers: bad rank/world (at most 8 GPUs share a probe)");
+    if (d_flags && epoch == 0)
+      return fail("datum_ibl_prefilter_level_float_peers: epochs start at 1");
+
+    const uintptr_t align = (uintptr_t)ibl::float_texel_bytes(format);
+    PeerTargets peers;
+    for(int r = 0; r < world; ++r)
+    {
+      if (!d_dst[r] || (d_flags && !d_flags[r]))
+        return fail("datum_ibl_prefilter_level_float_peers: null pointer for a rank");
+      if (reinterpret_cast<uintptr_t>(d_dst[r]) % align != 0)
+        return fail("datum_ibl_prefilter_level_float_peers: misaligned source or destination");
+      if (r != rank)
+      {
+        peers.dst[peers.count] = d_dst[r];
+        peers.arrive[peers.count] = d_flags ? reinterpret_cast<unsigned int*>(d_flags[r] + (epoch & 1u)) : nullptr;
+        peers.count += 1;
+      }
+    }
+    if (reinterpret_cast<uintptr_t>(d_src) % align != 0)
+      return fail("datum_ibl_prefilter_level_float_peers: misaligned source or destination");
+
+    DeviceGuard guard(ctx->device);
+
+    std::vector<DeviceTable> *tables = nullptr;
+    if (get_tables(ctx, levels, samples, &tables))
+      return 1;
+
+    if (row_begin == row_end && d_flags)
+    {
+      // an empty slab still has to arrive
+      if (signal_arrival(ctx, rank, world, d_flags, epoch))
+        return 1;
+    }
+    else if (run_level_float(ctx, format, d_src, ws, hs, (*tables)[level], row_begin, row_end, d_dst[rank], nullptr, false, peers))
       return 1;
 
     return d_flags ? wait_for_arrivals(ctx, d_flags[rank], epoch, world) : 0;

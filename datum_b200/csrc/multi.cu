@@ -7,10 +7,11 @@
 // per-device entry points of cabi.cu:
 //
 //   one probe split (BASELINE config 3)   every device holds the payload; per level each device computes a
-//       slab of rows with datum_ibl_prefilter_level_peers, whose kernel epilogue stores the slab into all
-//       payloads over NVLink (plain peer access inside one process: cudaDeviceEnablePeerAccess, no IPC
-//       handles) and whose last CTA bumps the peers' arrival counters; the streams wait on the counters.
-//       The host thread only enqueues: all devices run concurrently, nothing blocks until the end.
+//       slab of rows with datum_ibl_prefilter_level_peers (rgbe) or datum_ibl_prefilter_level_float_peers
+//       (F32, F16), whose kernel epilogue stores the slab into all payloads over NVLink (plain peer access
+//       inside one process: cudaDeviceEnablePeerAccess, no IPC handles) and whose last CTA bumps the peers'
+//       arrival counters; the streams wait on the counters.  The host thread only enqueues: all devices run
+//       concurrently, nothing blocks until the end.
 //   probe batches (config 4)              probe p on device p % ndev, one host thread per device around
 //       datum_ibl_bake_probes or datum_ibl_bake_probes_float; no data-path exchange.
 //   SH9 of one cube (config 5)            rows split, 28 partial sums per device added on the host.
@@ -40,7 +41,7 @@ struct datum_ibl_multi
 
   // one shared-probe payload per device: [flag block][chain], grow-only
   std::vector<unsigned char*> shared;
-  size_t shared_words = 0;
+  size_t shared_bytes = 0;
   uint32_t epoch = 0;
 
   std::vector<unsigned char*> sh_staging;   // per device: 28 doubles + its slab of the cube
@@ -68,12 +69,13 @@ namespace
         cudaFree(m->shared[d]);
         m->shared[d] = nullptr;
       }
-    m->shared_words = 0;
+    m->shared_bytes = 0;
   }
 
-  int reserve_shared(datum_ibl_multi *m, size_t words)
+  // chain bytes of every device's payload (rgbe words or float texels)
+  int reserve_shared(datum_ibl_multi *m, size_t bytes)
   {
-    if (words <= m->shared_words)
+    if (bytes <= m->shared_bytes)
       return 0;
 
     // nothing of a previous bake may still be in flight towards the old buffers
@@ -87,7 +89,7 @@ namespace
     {
       DeviceScope scope(m->devices[d]);
       void *ptr = nullptr;
-      cudaError_t err = cudaMalloc(&ptr, DATUM_IBL_PEER_FLAG_BYTES + words * sizeof(uint32_t));
+      cudaError_t err = cudaMalloc(&ptr, DATUM_IBL_PEER_FLAG_BYTES + bytes);
       if (err == cudaSuccess)
         err = cudaMemset(ptr, 0, DATUM_IBL_PEER_FLAG_BYTES);
       if (err != cudaSuccess)
@@ -100,13 +102,144 @@ namespace
       m->shared[d] = static_cast<unsigned char*>(ptr);
     }
 
-    m->shared_words = words;
+    m->shared_bytes = bytes;
     m->epoch = 0;
     return 0;
   }
 
-  uint32_t *chain_of(datum_ibl_multi *m, size_t d) { return reinterpret_cast<uint32_t*>(m->shared[d] + DATUM_IBL_PEER_FLAG_BYTES); }
+  unsigned char *chain_of(datum_ibl_multi *m, size_t d) { return m->shared[d] + DATUM_IBL_PEER_FLAG_BYTES; }
   uint32_t *flags_of(datum_ibl_multi *m, size_t d) { return reinterpret_cast<uint32_t*>(m->shared[d]); }
+
+  // One probe shared by the devices (BASELINE config 3), rgbe or float chains of `texel` bytes per texel: every
+  // device holds the chain; per level each device computes a slab of rows and stores it into every chain (split),
+  // or the whole level into its own.  bake_level(d, split, ws, hs, level, row_begin, row_end, src, dst, flags)
+  // enqueues device d's part; dst[r] is the destination level in device r's chain, src the source level in d's,
+  // flags the devices' flag blocks (epoch m->epoch).
+  template<typename BakeLevel>
+  int share_probe(datum_ibl_multi *m, const char *who, size_t texel, int width, int height, int levels, void *host, BakeLevel bake_level)
+  {
+    const int world = (int)m->devices.size();
+    const std::string name = who;
+
+    size_t texels = datum_ibl_chain_bytes(width, height, levels) / sizeof(uint32_t);
+    size_t level0 = (size_t)width * height * 6;
+
+    if (reserve_shared(m, texels * texel))
+      return 1;
+
+    // level 0: every device uploads ONE slice of it over its own PCIe link, then fetches the other slices from its
+    // peers over NVLink (one upload to the first device and copies from there took 2.8 ms for the 100 MB of a
+    // 2048^2 rgbe cube: 2 ms on one PCIe link + 0.8 ms out of one GPU's NVLink ports)
+    std::vector<cudaStream_t> streams(world);
+    for(int d = 0; d < world; ++d)
+      streams[d] = (cudaStream_t)datum_ibl_stream(m->ctx[d]);
+
+    // slices in texels, multiples of 64
+    auto slice_begin = [&](size_t count, int d) { size_t per = ((count + world - 1) / world + 63) & ~(size_t)63; size_t b = per * (size_t)d; return b < count ? b : count; };
+
+    std::vector<cudaEvent_t> uploaded(world, nullptr);
+    int failed = 0;
+
+    for(int d = 0; d < world && !failed; ++d)
+    {
+      DeviceScope scope(m->devices[d]);
+      size_t begin = slice_begin(level0, d), end = slice_begin(level0, d + 1);
+      cudaError_t err = cudaSuccess;
+      if (end > begin)
+        err = cudaMemcpyAsync(chain_of(m, d) + begin * texel, static_cast<unsigned char const*>(host) + begin * texel, (end - begin) * texel, cudaMemcpyHostToDevice, streams[d]);
+      if (err == cudaSuccess)
+        err = cudaEventCreateWithFlags(&uploaded[d], cudaEventDisableTiming);
+      if (err == cudaSuccess)
+        err = cudaEventRecord(uploaded[d], streams[d]);
+      if (err != cudaSuccess)
+        failed = fail_cuda((name + ": upload").c_str(), err);
+    }
+
+    for(int d = 0; d < world && !failed; ++d)
+    {
+      DeviceScope scope(m->devices[d]);
+      for(int k = 1; k < world && !failed; ++k)
+      {
+        int s = (d + k) % world;      // every device starts with another peer
+        size_t begin = slice_begin(level0, s), end = slice_begin(level0, s + 1);
+        if (end <= begin)
+          continue;
+        cudaError_t err = cudaStreamWaitEvent(streams[d], uploaded[s], 0);
+        if (err == cudaSuccess)
+          err = cudaMemcpyPeerAsync(chain_of(m, d) + begin * texel, m->devices[d], chain_of(m, s) + begin * texel, m->devices[s], (end - begin) * texel, streams[d]);
+        if (err != cudaSuccess)
+          failed = fail_cuda((name + ": level 0 from peer").c_str(), err);
+      }
+    }
+
+    std::vector<uint32_t*> flags(world);
+    for(int d = 0; d < world; ++d)
+      flags[d] = flags_of(m, d);
+
+    // every device has level 0 before anybody stores level 1 into it, and nobody still reads the previous probe
+    if (!failed)
+    {
+      m->epoch += 1;
+      for(int d = 0; d < world && !failed; ++d)
+        failed = datum_ibl_peer_barrier(m->ctx[d], d, world, flags.data(), m->epoch);
+    }
+
+    // tools/ibl.cpp:247-278, rows of every big level shared out
+    size_t src_off = 0, dst_off = level0;
+    int ws = width, hs = height;
+
+    for(int level = 1; level < levels && !failed; ++level)
+    {
+      int wd = ws >> 1, hd = hs >> 1;
+      int rows = 6 * hd;
+      bool split = rows % world == 0 && (long long)rows * wd > kMinSplitTexels;
+
+      if (split)
+        m->epoch += 1;
+
+      std::vector<void*> dst(world);
+      for(int r = 0; r < world; ++r)
+        dst[r] = chain_of(m, r) + dst_off * texel;
+
+      for(int d = 0; d < world && !failed; ++d)
+      {
+        int per = rows / world;
+        failed = bake_level(d, split, ws, hs, level, split ? d * per : 0, split ? (d + 1) * per : rows, chain_of(m, d) + src_off * texel, dst.data(), flags.data());
+      }
+
+      src_off = dst_off;
+      dst_off += (size_t)wd * hd * 6;
+      ws = wd;
+      hs = hd;
+    }
+
+    // every device now holds the whole chain: each hands one slice of the baked levels back
+    for(int d = 0; d < world && !failed; ++d)
+    {
+      DeviceScope scope(m->devices[d]);
+      size_t begin = level0 + slice_begin(texels - level0, d), end = level0 + slice_begin(texels - level0, d + 1);
+      if (end <= begin)
+        continue;
+      cudaError_t err = cudaMemcpyAsync(static_cast<unsigned char*>(host) + begin * texel, chain_of(m, d) + begin * texel, (end - begin) * texel, cudaMemcpyDeviceToHost, streams[d]);
+      if (err != cudaSuccess)
+        failed = fail_cuda((name + ": download").c_str(), err);
+    }
+
+    // also after a failure: nothing may stay in flight
+    std::string first_error = failed ? datum_ibl_last_error() : "";
+    for(int d = 0; d < world; ++d)
+      if (datum_ibl_synchronize(m->ctx[d]) && !failed)
+      {
+        failed = 1;
+        first_error = datum_ibl_last_error();
+      }
+
+    for(cudaEvent_t e : uploaded)
+      if (e)
+        cudaEventDestroy(e);
+
+    return failed ? fail(first_error) : 0;
+  }
 
   // Probe batches (config 4): probe p on device p % ndev; each device's share is one synchronous batched call
   // bake(ctx, n, payloads, sh) on its own host thread.  One device, or at most one probe: the first device's call.
@@ -258,128 +391,43 @@ extern "C"
     if (width < 1 || height < 1 || levels < 1 || levels > 16 || (width >> (levels - 1)) < 1 || (height >> (levels - 1)) < 1 || samples < 1)
       return fail("datum_ibl_multi_buildmips_cube_ibl: bad width/height/levels/samples");
 
-    size_t words = datum_ibl_chain_bytes(width, height, levels) / sizeof(uint32_t);
-    size_t level0 = (size_t)width * height * 6;
-
-    if (reserve_shared(m, words))
-      return 1;
-
-    // level 0: every device uploads ONE slice of it over its own PCIe link, then fetches the other slices from its
-    // peers over NVLink (one upload to the first device and copies from there took 2.8 ms for the 100 MB of a
-    // 2048^2 cube: 2 ms on one PCIe link + 0.8 ms out of one GPU's NVLink ports)
-    std::vector<cudaStream_t> streams(world);
-    for(int d = 0; d < world; ++d)
-      streams[d] = (cudaStream_t)datum_ibl_stream(m->ctx[d]);
-
-    auto slice_begin = [&](size_t count, int d) { size_t per = ((count + world - 1) / world + 63) & ~(size_t)63; size_t b = per * (size_t)d; return b < count ? b : count; };
-
-    std::vector<cudaEvent_t> uploaded(world, nullptr);
-    int failed = 0;
-
-    for(int d = 0; d < world && !failed; ++d)
-    {
-      DeviceScope scope(m->devices[d]);
-      size_t begin = slice_begin(level0, d), end = slice_begin(level0, d + 1);
-      cudaError_t err = cudaSuccess;
-      if (end > begin)
-        err = cudaMemcpyAsync(chain_of(m, d) + begin, static_cast<uint32_t const*>(bits) + begin, (end - begin) * sizeof(uint32_t), cudaMemcpyHostToDevice, streams[d]);
-      if (err == cudaSuccess)
-        err = cudaEventCreateWithFlags(&uploaded[d], cudaEventDisableTiming);
-      if (err == cudaSuccess)
-        err = cudaEventRecord(uploaded[d], streams[d]);
-      if (err != cudaSuccess)
-        failed = fail_cuda("datum_ibl_multi_buildmips_cube_ibl: upload", err);
-    }
-
-    for(int d = 0; d < world && !failed; ++d)
-    {
-      DeviceScope scope(m->devices[d]);
-      for(int k = 1; k < world && !failed; ++k)
+    return share_probe(m, "datum_ibl_multi_buildmips_cube_ibl", sizeof(uint32_t), width, height, levels, bits,
+      [&](int d, bool split, int ws, int hs, int level, int row_begin, int row_end, unsigned char *src, void *const *dst, uint32_t *const *flags)
       {
-        int s = (d + k) % world;      // every device starts with another peer
-        size_t begin = slice_begin(level0, s), end = slice_begin(level0, s + 1);
-        if (end <= begin)
-          continue;
-        cudaError_t err = cudaStreamWaitEvent(streams[d], uploaded[s], 0);
-        if (err == cudaSuccess)
-          err = cudaMemcpyPeerAsync(chain_of(m, d) + begin, m->devices[d], chain_of(m, s) + begin, m->devices[s], (end - begin) * sizeof(uint32_t), streams[d]);
-        if (err != cudaSuccess)
-          failed = fail_cuda("datum_ibl_multi_buildmips_cube_ibl: level 0 from peer", err);
-      }
-    }
+        if (!split)
+          return datum_ibl_prefilter_level_device(m->ctx[d], reinterpret_cast<uint32_t const*>(src), ws, hs, level, levels, samples, row_begin, row_end, static_cast<uint32_t*>(dst[d]), nullptr);
 
-    std::vector<uint32_t*> flags(world);
-    for(int d = 0; d < world; ++d)
-      flags[d] = flags_of(m, d);
+        std::vector<uint32_t*> words(world);
+        for(int r = 0; r < world; ++r)
+          words[r] = static_cast<uint32_t*>(dst[r]);
+        return datum_ibl_prefilter_level_peers(m->ctx[d], reinterpret_cast<uint32_t const*>(src), ws, hs, level, levels, samples, row_begin, row_end, d, world, words.data(), flags, m->epoch);
+      });
+  }
 
-    // every device has level 0 before anybody stores level 1 into it, and nobody still reads the previous probe
-    if (!failed)
-    {
-      m->epoch += 1;
-      for(int d = 0; d < world && !failed; ++d)
-        failed = datum_ibl_peer_barrier(m->ctx[d], d, world, flags.data(), m->epoch);
-    }
+  int datum_ibl_multi_buildmips_cube_float(datum_ibl_multi *m, int format, int width, int height, int levels, int samples, void *chain)
+  {
+    if (!m || !chain)
+      return fail("datum_ibl_multi_buildmips_cube_float: null argument");
 
-    // tools/ibl.cpp:247-278, rows of every big level shared out
-    size_t src_off = 0, dst_off = level0;
-    int ws = width, hs = height;
+    const int world = (int)m->devices.size();
 
-    for(int level = 1; level < levels && !failed; ++level)
-    {
-      int wd = ws >> 1, hd = hs >> 1;
-      int rows = 6 * hd;
-      bool split = rows % world == 0 && (long long)rows * wd > kMinSplitTexels;
+    if (world == 1)
+      return datum_ibl_buildmips_cube_float(m->ctx[0], format, width, height, levels, samples, chain);
 
-      if (split)
-        m->epoch += 1;
+    if (format != DATUM_IBL_FORMAT_F32 && format != DATUM_IBL_FORMAT_F16)
+      return fail("datum_ibl_multi_buildmips_cube_float: unknown format " + std::to_string(format) + " (DATUM_IBL_FORMAT_F32 or DATUM_IBL_FORMAT_F16)");
+    if (width < 1 || height < 1 || levels < 1 || levels > 16 || (width >> (levels - 1)) < 1 || (height >> (levels - 1)) < 1 || samples < 1 || samples > 4096)
+      return fail("datum_ibl_multi_buildmips_cube_float: bad width/height/levels/samples");
 
-      for(int d = 0; d < world && !failed; ++d)
+    const size_t texel = format == DATUM_IBL_FORMAT_F16 ? 8 : 16;
+
+    return share_probe(m, "datum_ibl_multi_buildmips_cube_float", texel, width, height, levels, chain,
+      [&](int d, bool split, int ws, int hs, int level, int row_begin, int row_end, unsigned char *src, void *const *dst, uint32_t *const *flags)
       {
-        if (split)
-        {
-          std::vector<uint32_t*> dst(world);
-          for(int r = 0; r < world; ++r)
-            dst[r] = chain_of(m, r) + dst_off;
-
-          int per = rows / world;
-          failed = datum_ibl_prefilter_level_peers(m->ctx[d], chain_of(m, d) + src_off, ws, hs, level, levels, samples, d * per, (d + 1) * per, d, world, dst.data(), flags.data(), m->epoch);
-        }
-        else
-          failed = datum_ibl_prefilter_level_device(m->ctx[d], chain_of(m, d) + src_off, ws, hs, level, levels, samples, 0, rows, chain_of(m, d) + dst_off, nullptr);
-      }
-
-      src_off = dst_off;
-      dst_off += (size_t)wd * hd * 6;
-      ws = wd;
-      hs = hd;
-    }
-
-    // every device now holds the whole chain: each hands one slice of the baked levels back
-    for(int d = 0; d < world && !failed; ++d)
-    {
-      DeviceScope scope(m->devices[d]);
-      size_t begin = level0 + slice_begin(words - level0, d), end = level0 + slice_begin(words - level0, d + 1);
-      if (end <= begin)
-        continue;
-      cudaError_t err = cudaMemcpyAsync(static_cast<uint32_t*>(bits) + begin, chain_of(m, d) + begin, (end - begin) * sizeof(uint32_t), cudaMemcpyDeviceToHost, streams[d]);
-      if (err != cudaSuccess)
-        failed = fail_cuda("datum_ibl_multi_buildmips_cube_ibl: download", err);
-    }
-
-    // also after a failure: nothing may stay in flight
-    std::string first_error = failed ? datum_ibl_last_error() : "";
-    for(int d = 0; d < world; ++d)
-      if (datum_ibl_synchronize(m->ctx[d]) && !failed)
-      {
-        failed = 1;
-        first_error = datum_ibl_last_error();
-      }
-
-    for(cudaEvent_t e : uploaded)
-      if (e)
-        cudaEventDestroy(e);
-
-    return failed ? fail(first_error) : 0;
+        if (!split)
+          return datum_ibl_prefilter_level_float_device(m->ctx[d], format, src, ws, hs, level, levels, samples, row_begin, row_end, dst[d], nullptr);
+        return datum_ibl_prefilter_level_float_peers(m->ctx[d], format, src, ws, hs, level, levels, samples, row_begin, row_end, d, world, dst, flags, m->epoch);
+      });
   }
 
   int datum_ibl_multi_bake_probes(datum_ibl_multi *m, int count, int width, int height, int levels, int samples, void *const *bits, float *sh)

@@ -117,34 +117,6 @@ namespace ibl
   }
 
 
-  // ---- "this launch has stored everything" -----------------------------------------------------
-  //
-  // One probe shared by several GPUs: the epilogues above store every word into the peers' chains.
-  // The CTA that finishes LAST (ticket counter) bumps an arrival counter in every peer's flag block
-  // with a system-scope release; the peers' streams wait on their own counter (a stream memory
-  // operation, no kernel) before the next level reads the words.  Every thread fences its own
-  // stores before the ticket, the last CTA fences again behind it (cumulativity).
-  __device__ __forceinline__ void signal_peers_when_last(PeerSignal const &s)
-  {
-    if (s.count <= 0)
-      return;
-
-    __threadfence_system();
-    __syncthreads();
-
-    if (threadIdx.x == 0)
-    {
-      unsigned int ticket = atomicAdd(s.ticket, 1u);
-      if (ticket == gridDim.x - 1)
-      {
-        __threadfence_system();
-        for(int k = 0; k < s.count; ++k)
-          asm volatile("red.release.sys.global.add.u32 [%0], 1;" :: "l"(s.arrive[k]) : "memory");
-        *s.ticket = 0;        // ready for the next launch on this stream
-      }
-    }
-  }
-
   // ---- one sample of one texel -------------------------------------------------------
 
   struct TexelFrame

@@ -23,6 +23,12 @@
 // the single-probe kernels compile none of the batch code.  Launch shapes that decide the order of the sums
 // (warps per tile, warps per texel) follow ONE probe's slab, so every probe of a batch gets the bytes of a
 // single call; only the tile queues and the grid follow the whole launch.
+//
+// Shared probes (datum_ibl_prefilter_level_float_peers, datum_ibl_multi_buildmips_cube_float): one probe split
+// over up to 8 GPUs by rows, like the rgbe chain's.  The pair kernel and the tail kernel (both forms of PROJ)
+// have instantiations of their own (SHARED) whose epilogue stores every texel (8 B for F16, 16 B for F32) into
+// this GPU's chain and into every peer's over NVLink, and whose CTAs then run signal_peers_when_last
+// (prefilter_pair.cuh): the last one to finish bumps the peers' arrival counters.  One chain, no dst_f32.
 
 #include "prefilter.h"
 #include "prefilter_f.h"
@@ -222,13 +228,35 @@ namespace ibl
       }
     }
 
+    // one probe shared by several GPUs: the texel goes to this GPU's chain and, over NVLink, into every peer's
+    template<int FMT>
+    __device__ __forceinline__ void store_texel_peers(PrefilterFloatParams const &p, size_t o, float r, float g, float b)
+    {
+      if (FMT == kFloatFormatF16)
+      {
+        uint32_t hr = float_to_half_rn(r), hg = float_to_half_rn(g), hb = float_to_half_rn(b);
+        const uint2 texel = make_uint2(hg << 16 | hr, 0x3C00u << 16 | hb);
+        reinterpret_cast<uint2*>(p.dst)[o] = texel;
+        for(int k = 0; k < p.peers; ++k)
+          reinterpret_cast<uint2*>(p.peer_dst[k])[o] = texel;
+      }
+      else
+      {
+        const float4 texel = make_float4(r, g, b, 1.0f);
+        reinterpret_cast<float4*>(p.dst)[o] = texel;
+        for(int k = 0; k < p.peers; ++k)
+          reinterpret_cast<float4*>(p.peer_dst[k])[o] = texel;
+      }
+    }
+
     // ---- the pair kernel ------------------------------------------------------------------------
     //
     // CTA = NW warps sharing one 8x4 tile; warp w reads azimuth sector w of every band of the sector table,
     // its leading bands without face selection as long as they provably stay on the texel's face.
     // BATCH: the same level of p.probes chains, tiles numbered probe by probe (prefilter_dp_kernel's batches).
-    // The single-probe instantiations compile none of the batch code.
-    template<int FMT, int NW, int MINB, bool SMEM_TABLE, bool QUEUES, bool BATCH = false>
+    // SHARED: one probe shared by several GPUs, a slab stored into every peer's chain and the peers told when it
+    // is complete (prefilter_dp_kernel's peer stores).  The single-probe instantiations compile none of either.
+    template<int FMT, int NW, int MINB, bool SMEM_TABLE, bool QUEUES, bool BATCH = false, bool SHARED = false>
     __global__ void __launch_bounds__(32 * NW, MINB) prefilter_float_pair_kernel(PrefilterFloatParams p)
     {
       typedef typename RecordOf<FMT>::type R;
@@ -370,17 +398,26 @@ namespace ibl
           add_warp_sums<NW>(s_red, lane, sum);
 
           if (valid)
-            store_texel<FMT>(p, (size_t)row * p.wd + x + (BATCH ? (size_t)probe * p.dst_stride : (size_t)0), sum[0] * p.norm, sum[1] * p.norm, sum[2] * p.norm);
+          {
+            if (SHARED)
+              store_texel_peers<FMT>(p, (size_t)row * p.wd + x, sum[0] * p.norm, sum[1] * p.norm, sum[2] * p.norm);
+            else
+              store_texel<FMT>(p, (size_t)row * p.wd + x + (BATCH ? (size_t)probe * p.dst_stride : (size_t)0), sum[0] * p.norm, sum[1] * p.norm, sum[2] * p.norm);
+          }
         }
 
         __syncthreads();
       }
+
+      if (SHARED)
+        signal_peers_when_last(p.signal);
     }
 
     // ---- the tail kernel: one CTA per texel, lanes are samples (prefilter_tail_kernel) ----------------
     // BATCH: the same level of p.probes chains, blockIdx.x runs over the texels probe by probe (batches run only
-    // where every source is proj_usable, prefilter_batchable: PROJ)
-    template<int FMT, int NW, bool PROJ, bool BATCH = false>
+    // where every source is proj_usable, prefilter_batchable: PROJ).  SHARED: one probe's slab stored into every
+    // peer's chain, the peers told when it is complete (either form of PROJ: odd sources and faces above 2048^2).
+    template<int FMT, int NW, bool PROJ, bool BATCH = false, bool SHARED = false>
     __global__ void __launch_bounds__(32 * NW) prefilter_float_tail_kernel(PrefilterFloatParams p)
     {
       __shared__ float s_red[NW][3];
@@ -486,14 +523,20 @@ namespace ibl
             sum[c] += s_red[w][c];
         }
 
-        store_texel<FMT>(p, (size_t)row * p.wd + x + (BATCH ? (size_t)probe * p.dst_stride : (size_t)0), sum[0] * p.norm, sum[1] * p.norm, sum[2] * p.norm);
+        if (SHARED)
+          store_texel_peers<FMT>(p, (size_t)row * p.wd + x, sum[0] * p.norm, sum[1] * p.norm, sum[2] * p.norm);
+        else
+          store_texel<FMT>(p, (size_t)row * p.wd + x + (BATCH ? (size_t)probe * p.dst_stride : (size_t)0), sum[0] * p.norm, sum[1] * p.norm, sum[2] * p.norm);
       }
+
+      if (SHARED)
+        signal_peers_when_last(p.signal);
     }
 
-    template<int FMT, int NW, int MINB, bool SMEM_TABLE, bool QUEUES, bool BATCH>
+    template<int FMT, int NW, int MINB, bool SMEM_TABLE, bool QUEUES, bool BATCH, bool SHARED>
     cudaError_t launch_pair(PrefilterFloatParams p, int sm_count, cudaStream_t stream)
     {
-      auto kernel = prefilter_float_pair_kernel<FMT, NW, MINB, SMEM_TABLE, QUEUES, BATCH>;
+      auto kernel = prefilter_float_pair_kernel<FMT, NW, MINB, SMEM_TABLE, QUEUES, BATCH, SHARED>;
 
       const int table_bands = p.sector_bands[NW == 8 ? 1 : 0];
       size_t smem = (SMEM_TABLE ? (size_t)table_bands * kSectorShare * NW * sizeof(float4) : 0) + (size_t)NW * 3 * 32 * sizeof(float) + sizeof(int);
@@ -508,30 +551,34 @@ namespace ibl
       return cudaGetLastError();
     }
 
-    template<int FMT, int NW, int MINB, bool QUEUES, bool BATCH>
+    template<int FMT, int NW, int MINB, bool QUEUES, bool BATCH, bool SHARED>
     cudaError_t launch_pair_table(PrefilterFloatParams const &p, int sm_count, cudaStream_t stream)
     {
-      return p.table_count > kBigTableEntries ? launch_pair<FMT, NW, MINB, false, QUEUES, BATCH>(p, sm_count, stream) : launch_pair<FMT, NW, MINB, true, QUEUES, BATCH>(p, sm_count, stream);
+      return p.table_count > kBigTableEntries ? launch_pair<FMT, NW, MINB, false, QUEUES, BATCH, SHARED>(p, sm_count, stream) : launch_pair<FMT, NW, MINB, true, QUEUES, BATCH, SHARED>(p, sm_count, stream);
     }
 
     // The slab-size classes of launch_prefilter_dn.  Warps per tile follow ONE probe's slab (they decide the
     // order of the sums: a batch must give the bytes of single calls), the tile queues the whole launch.
-    template<int FMT, bool BATCH>
+    template<int FMT, bool BATCH, bool SHARED>
     cudaError_t launch_pair_shape(PrefilterFloatParams const &p, int sm_count, cudaStream_t stream)
     {
       const size_t texels = (size_t)(p.row_end - p.row_begin) * p.wd;
 
       if (texels >= kFourWarpTexels)
-        return launch_pair_table<FMT, 4, 8, true, BATCH>(p, sm_count, stream);
+        return launch_pair_table<FMT, 4, 8, true, BATCH, SHARED>(p, sm_count, stream);
       if (texels * (size_t)p.probes >= kQueuedTexels)
-        return launch_pair_table<FMT, 8, 4, true, BATCH>(p, sm_count, stream);
-      return launch_pair_table<FMT, 8, 4, false, BATCH>(p, sm_count, stream);
+        return launch_pair_table<FMT, 8, 4, true, BATCH, SHARED>(p, sm_count, stream);
+      return launch_pair_table<FMT, 8, 4, false, BATCH, SHARED>(p, sm_count, stream);
     }
+
+    bool shared_probe(PrefilterFloatParams const &p) { return p.peers > 0 || p.signal.count > 0; }
 
     template<int FMT>
     cudaError_t launch_pair_for(PrefilterFloatParams const &p, int sm_count, cudaStream_t stream)
     {
-      return p.probes > 1 ? launch_pair_shape<FMT, true>(p, sm_count, stream) : launch_pair_shape<FMT, false>(p, sm_count, stream);
+      if (p.probes > 1)
+        return launch_pair_shape<FMT, true, false>(p, sm_count, stream);
+      return shared_probe(p) ? launch_pair_shape<FMT, false, true>(p, sm_count, stream) : launch_pair_shape<FMT, false, false>(p, sm_count, stream);
     }
 
     template<int NW, int FMT, bool PROJ>
@@ -539,6 +586,8 @@ namespace ibl
     {
       if (p.probes > 1)
         prefilter_float_tail_kernel<FMT, NW, true, true><<<grid, 32 * NW, 0, stream>>>(p);
+      else if (shared_probe(p))
+        prefilter_float_tail_kernel<FMT, NW, PROJ, false, true><<<grid, 32 * NW, 0, stream>>>(p);
       else
         prefilter_float_tail_kernel<FMT, NW, PROJ><<<grid, 32 * NW, 0, stream>>>(p);
     }
@@ -596,6 +645,8 @@ namespace ibl
       p.probes = 1;
     if (p.probes > 1 && p.dst_f32)
       return cudaErrorNotSupported;       // batches store the format's texels only
+    if (shared_probe(p) && (p.probes > 1 || p.dst_f32))
+      return cudaErrorNotSupported;       // a shared probe: one chain, texels of the format
 
     if (p.format == kFloatFormatF16)
       return launch_pair_for<kFloatFormatF16>(p, sm_count, stream);
@@ -618,6 +669,8 @@ namespace ibl
     const bool proj = proj_usable(p.geom.ws, p.geom.hs);
     if (p.probes > 1 && (p.dst_f32 || !proj))
       return cudaErrorNotSupported;       // batches: texels of the format, proj_usable sources (prefilter_batchable)
+    if (shared_probe(p) && (p.probes > 1 || p.dst_f32))
+      return cudaErrorNotSupported;       // a shared probe: one chain, texels of the format
 
     if (p.format == kFloatFormatF16)
       return proj ? launch_tail_for<kFloatFormatF16, true>(p, texels, stream) : launch_tail_for<kFloatFormatF16, false>(p, texels, stream);

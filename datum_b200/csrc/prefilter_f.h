@@ -10,6 +10,8 @@
 #include <cstdint>
 
 #if defined(__CUDACC__)
+#include "prefilter.h"
+
 #include <cuda_runtime.h>
 #endif
 
@@ -148,6 +150,12 @@ namespace ibl
     // (launch_build_float_records writes them back to back: 6*ws*hs).  dst_f32 must be null.
     int probes, tiles_per_probe, texels_per_probe;    // the last two filled by the launchers
     size_t src_stride, record_stride, dst_stride;
+
+    // one probe shared by several GPUs (datum_ibl_prefilter_level_float_peers): the epilogue stores every texel
+    // into dst and into the same destination level of each peer's chain; probes == 1 and dst_f32 null
+    void *peer_dst[kMaxPeers];
+    int peers;
+    PeerSignal signal;        // whom to tell when the whole slab is stored
   };
 
   // records of the ws x hs source levels of `probes` chains (src_stride texels apart; records back to back);
@@ -157,7 +165,8 @@ namespace ibl
   // pair kernel (proj_usable sources, slabs above kTailTexels, levels at least 8 wide)
   cudaError_t launch_prefilter_float(PrefilterFloatParams const &p, int sm_count, cudaStream_t stream);
 
-  // one CTA per destination texel, lanes are samples; any source size (a batch: proj_usable sources only)
+  // one CTA per destination texel, lanes are samples; any source size (a batch: proj_usable sources only).
+  // Both launchers run their shared-probe instantiations when p.peers > 0 or p.signal.count > 0.
   cudaError_t launch_prefilter_float_tail(PrefilterFloatParams const &p, cudaStream_t stream);
 #endif
 }

@@ -2,16 +2,17 @@
 // float chains (prefilter_f.cu); internal to libdatum_ibl_cuda.
 //
 // What both chains compute alike lives here: the packed fp32 ops, the pair table entries and the projective
-// footprint coordinates of two samples, the tile hand-out, and the per-tile frame, same-face band count and
-// CTA reduction.  What differs between the chains stays in each kernel: the record layout, the tap fetch and
-// decode, the store, the batch addressing (probe strides) and (rgbe only) peers and the arrival signal.  Nothing
-// here depends on which chain calls it.
+// footprint coordinates of two samples, the tile hand-out, the per-tile frame, same-face band count and
+// CTA reduction, and the arrival signal of a probe shared by several GPUs.  What differs between the chains
+// stays in each kernel: the record layout, the tap fetch and decode, the store (peer stores included) and the
+// batch addressing (probe strides).  Nothing here depends on which chain calls it.
 //
 // The rgbe kernels are sensitive to everything compiled into their bodies (DESIGN.md §4.1): these helpers keep
 // the statement order of the code they replace, and take output references rather than returning structs,
 // so that every kernel of both files compiles to the same SASS as before they were shared.
 #pragma once
 
+#include "prefilter.h"
 #include "ibl_math.cuh"
 
 #include <cuda_runtime.h>
@@ -304,6 +305,34 @@ namespace ibl
       #pragma unroll
       for(int c = 0; c < 3; ++c)
         sum[c] += s_red[(w * 3 + c) * 32 + lane];
+    }
+  }
+
+  // ---- "this launch has stored everything" -----------------------------------------------------
+  //
+  // One probe shared by several GPUs: the kernels' epilogues store every texel into the peers' chains.
+  // The CTA that finishes LAST (ticket counter) bumps an arrival counter in every peer's flag block
+  // with a system-scope release; the peers' streams wait on their own counter (a stream memory
+  // operation, no kernel) before the next level reads the texels.  Every thread fences its own
+  // stores before the ticket, the last CTA fences again behind it (cumulativity).
+  __device__ __forceinline__ void signal_peers_when_last(PeerSignal const &s)
+  {
+    if (s.count <= 0)
+      return;
+
+    __threadfence_system();
+    __syncthreads();
+
+    if (threadIdx.x == 0)
+    {
+      unsigned int ticket = atomicAdd(s.ticket, 1u);
+      if (ticket == gridDim.x - 1)
+      {
+        __threadfence_system();
+        for(int k = 0; k < s.count; ++k)
+          asm volatile("red.release.sys.global.add.u32 [%0], 1;" :: "l"(s.arrive[k]) : "memory");
+        *s.ticket = 0;        // ready for the next launch on this stream
+      }
     }
   }
 }

@@ -152,11 +152,17 @@ class PeerChain:
     torch.distributed (all_gather_object: plumbing, not data path), and every rank
     maps its peers' allocations.  bake() then needs no collective: the prefilter
     kernel's epilogue stores each slab into all chains over NVLink and a one-CTA
-    stream memory wait on the arrival counters separates the levels."""
+    stream memory wait on the arrival counters separates the levels.
+
+    `fmt`: ibl.FORMAT_RGBE (the default: `chain` is a flat int32 tensor of rgbe
+    words) or a float chain's ibl.FORMAT_F32 / ibl.FORMAT_F16 (`chain` is a
+    (texels, 4) float32 / float16 tensor, baked without rgbe re-quantisation)."""
 
     FLAG_BYTES = 256
 
-    def __init__(self, ctx, width, height, levels, group=None):
+    _TYPESTR = {ibl.FORMAT_RGBE: "<i4", ibl.FORMAT_F32: "<f4", ibl.FORMAT_F16: "<f2"}
+
+    def __init__(self, ctx, width, height, levels, group=None, fmt=ibl.FORMAT_RGBE):
         import torch
         self.torch = torch
         self.ctx = ctx
@@ -164,13 +170,17 @@ class PeerChain:
         self.dist, self.rank, self.world = _world(group)
         if self.world > 8:
             raise ValueError("a probe is shared by at most 8 GPUs (one NVSwitch domain)")
+        if fmt not in self._TYPESTR:
+            raise ValueError("unknown texel format %r" % (fmt,))
         self.width, self.height, self.levels = width, height, levels
+        self.fmt = fmt
+        self.texel_bytes = ibl.TEXEL_BYTES[fmt]
         self.offs = ibl.level_offsets(width, height, levels)
-        self.words = self.offs[-1]
+        self.words = self.offs[-1]          # texels of the chain (rgbe: words)
         self.epoch = 0
 
         # flags first (256 B), then the chain
-        self.local, handle = ctx.peer_alloc(self.FLAG_BYTES + 4 * self.words)
+        self.local, handle = ctx.peer_alloc(self.FLAG_BYTES + self.texel_bytes * self.words)
         self.bases = [None] * self.world
         self.bases[self.rank] = self.local
         if self.world > 1:
@@ -179,7 +189,10 @@ class PeerChain:
             for r in range(self.world):
                 if r != self.rank:
                     self.bases[r] = ctx.peer_open(handles[r])
-        self.chain = torch.as_tensor(_DeviceArray(self.local + self.FLAG_BYTES, self.words), device=torch.device("cuda", ctx.device))
+        if fmt == ibl.FORMAT_RGBE:
+            self.chain = torch.as_tensor(_DeviceArray(self.local + self.FLAG_BYTES, self.words), device=torch.device("cuda", ctx.device))
+        else:
+            self.chain = torch.as_tensor(_DeviceArray(self.local + self.FLAG_BYTES, 4 * self.words, self._TYPESTR[fmt]), device=torch.device("cuda", ctx.device)).view(self.words, 4)
 
     def chain_address(self, rank):
         return self.bases[rank] + self.FLAG_BYTES
@@ -199,20 +212,27 @@ class PeerChain:
         if self.world > 1:
             self.barrier()
 
+        tb = self.texel_bytes
         for step in plan:
             level = step["level"]
-            src = self.chain_address(self.rank) + 4 * self.offs[level - 1]
+            src = self.chain_address(self.rank) + tb * self.offs[level - 1]
             begin, end = step["ranges"][self.rank]
 
             if step["split"]:
                 self.epoch += 1
-                dst = [self.chain_address(r) + 4 * self.offs[level] for r in range(self.world)]
-                self.ctx.prefilter_level_peers(src, step["ws"], step["hs"], level, self.levels, samples, begin, end, self.rank, self.world, dst, self.bases, self.epoch)
+                dst = [self.chain_address(r) + tb * self.offs[level] for r in range(self.world)]
+                self._level(src, step, level, samples, begin, end, self.rank, self.world, dst, self.bases, self.epoch)
             else:
-                dst = self.chain_address(self.rank) + 4 * self.offs[level]
-                self.ctx.prefilter_level_peers(src, step["ws"], step["hs"], level, self.levels, samples, begin, end, 0, 1, [dst])
+                dst = self.chain_address(self.rank) + tb * self.offs[level]
+                self._level(src, step, level, samples, begin, end, 0, 1, [dst])
 
         return self.chain
+
+    def _level(self, src, step, level, samples, begin, end, rank, world, dst, flags=None, epoch=0):
+        if self.fmt == ibl.FORMAT_RGBE:
+            self.ctx.prefilter_level_peers(src, step["ws"], step["hs"], level, self.levels, samples, begin, end, rank, world, dst, flags, epoch)
+        else:
+            self.ctx.prefilter_level_float_peers(self.fmt, src, step["ws"], step["hs"], level, self.levels, samples, begin, end, rank, world, dst, flags, epoch)
 
     def close(self):
         self.ctx.synchronize()

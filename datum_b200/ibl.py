@@ -364,6 +364,13 @@ class IblContext:
         flags = (ctypes.c_void_p * world)(*flag_addresses) if flag_addresses is not None else None
         self._check(self._lib.datum_ibl_prefilter_level_peers(self._handle, ctypes.c_void_p(src_address), ws, hs, level, levels, samples, row_begin, row_end, rank, world, dst, flags, epoch))
 
+    def prefilter_level_float_peers(self, fmt, src_address, ws, hs, level, levels, samples, row_begin, row_end, rank, world, dst_addresses, flag_addresses=None, epoch=0):
+        """prefilter_level_peers for a float chain of format `fmt` (FORMAT_F32 or FORMAT_F16): raw device addresses,
+        aligned to the texel size; every texel of the slab goes to the destination level of each rank's chain."""
+        dst = (ctypes.c_void_p * world)(*dst_addresses)
+        flags = (ctypes.c_void_p * world)(*flag_addresses) if flag_addresses is not None else None
+        self._check(self._lib.datum_ibl_prefilter_level_float_peers(self._handle, fmt, ctypes.c_void_p(src_address), ws, hs, level, levels, samples, row_begin, row_end, rank, world, dst, flags, epoch))
+
     def peer_barrier(self, rank, world, flag_addresses, epoch):
         """Barrier of the GPUs sharing a probe, on the context's stream (flag blocks by rank)."""
         flags = (ctypes.c_void_p * world)(*flag_addresses)
@@ -527,6 +534,16 @@ class MultiContext:
         """tools/ibl.h:9 with ONE probe shared by the devices (rows of every big level split, NVLink peer stores)."""
         ptr = _host_pointer(bits, image_datasize(width, height, 6, levels), "bits")
         self._check(self._lib.datum_ibl_multi_buildmips_cube_ibl(self._handle, width, height, levels, samples, ptr))
+
+    def buildmips_cube_float(self, fmt, width, height, levels, chain, samples=1024):
+        """IblContext.buildmips_cube_float with ONE probe shared by the devices (rows of every big level split,
+        NVLink peer stores).  Level 0 stays the caller's; the other levels equal the one-device chain's up to the
+        re-cut tiles.  Synchronous."""
+        if hasattr(chain, "is_cuda") and chain.is_cuda:
+            raise ValueError("chain must be a host buffer")
+        _check_dtype(chain, _float_dtype(fmt), "chain")
+        ptr = _host_pointer(chain, float_chain_texels(width, height, levels) * _texel_bytes(fmt), "chain")
+        self._check(self._lib.datum_ibl_multi_buildmips_cube_float(self._handle, fmt, width, height, levels, samples, ptr))
 
     def bake_probes(self, width, height, levels, payloads, samples=1024, sh9=False):
         """IblContext.bake_probes with probe p on devices[p % ndev]."""

@@ -334,6 +334,25 @@ int datum_ibl_bake_probes_float(datum_ibl_ctx *ctx, int format, int count, int w
 /* datum_ibl_bake_probes_float with probe p on devices[p % ndev] (see datum_ibl_multi_bake_probes); results identical to one device's */
 int datum_ibl_multi_bake_probes_float(datum_ibl_multi *multi, int format, int count, int width, int height, int levels, int samples, void *const *chains, float *sh);
 
+/*
+ * datum_ibl_prefilter_level_peers for a float chain: rank `rank` of `world` (<= 8) GPUs sharing the probe
+ * computes rows [row_begin, row_end) of the level and stores every texel of the format into d_dst[r], the START
+ * of the destination level in rank r's chain as mapped HERE (r == rank: the local one).  With d_flags (flag
+ * blocks by rank, may be NULL: no signal, no wait) and epoch > 0 the launch signals its completion to the peers
+ * (an empty slab still arrives) and the context's stream then waits for the arrivals of all peers.  Pointers
+ * aligned to the texel size, `samples` 1..4096.  Asynchronous.
+ */
+int datum_ibl_prefilter_level_float_peers(datum_ibl_ctx *ctx, int format, void const *d_src, int ws, int hs, int level, int levels, int samples, int row_begin, int row_end, int rank, int world, void *const *d_dst, uint32_t *const *d_flags, uint32_t epoch);
+
+/*
+ * datum_ibl_buildmips_cube_float with ONE probe shared by the devices, the float counterpart of
+ * datum_ibl_multi_buildmips_cube_ibl: the same split of rows, peer stores, arrival counters and uploads.  Level 0
+ * of the result is the caller's; the other levels equal the single-device chain's up to the re-cut tiles
+ * (F32 within 1e-4 of a texel's largest channel, F16 within 1 ulp).  One device: datum_ibl_buildmips_cube_float.
+ * Host chain, synchronous.
+ */
+int datum_ibl_multi_buildmips_cube_float(datum_ibl_multi *multi, int format, int width, int height, int levels, int samples, void *chain);
+
 #ifdef __cplusplus
 }
 #endif
