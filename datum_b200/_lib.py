@@ -68,6 +68,10 @@ SIGNATURES = {
     "datum_ibl_multi_bake_probes_float": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, ctypes.POINTER(c_void_p), c_void_p]),
     "datum_ibl_prefilter_level_float_peers": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, ctypes.POINTER(c_void_p), ctypes.POINTER(c_void_p), ctypes.c_uint32]),
     "datum_ibl_multi_buildmips_cube_float": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
+    "datum_ibl_pack_cube_float": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int, c_void_p]),
+    "datum_ibl_pack_cube_float_ibl": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
+    "datum_ibl_ingest_cube_argb32_float": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "datum_ibl_ingest_cube_argb32_float_ibl": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
 }
 
 

@@ -1105,6 +1105,54 @@ namespace
 
 namespace
 {
+  // Levels >= 1 of a float chain whose level 0 is at d_chain on the device, then the chain home: `chain` is the
+  // caller's host chain, `pinned` says whether it is page-locked (if not, the download goes through the pinned
+  // staging, reserved by the caller for the whole chain, and is moved on after the sync).  With send_level0 level
+  // 0 travels too, on the download stream under the level-1 kernels; without it the caller's level 0 is untouched.
+  int finish_float_chain(datum_ibl_ctx *ctx, int format, int width, int height, int levels, int samples, unsigned char *d_chain, void *chain, bool pinned, bool send_level0, const char *who)
+  {
+    const size_t texel = (size_t)ibl::float_texel_bytes(format);
+    const size_t bytes = datum_ibl_chain_bytes(width, height, levels) / sizeof(uint32_t) * texel;
+    const size_t level0 = (size_t)width * height * 6 * texel;
+    const size_t first = send_level0 ? 0 : level0;
+
+    unsigned char *host = pinned ? static_cast<unsigned char*>(chain) : static_cast<unsigned char*>(ctx->host_stage);
+
+    int failed = send_level0 ? ensure_pipeline(ctx) : 0;
+    if (!failed && send_level0)
+    {
+      cudaError_t err = send_level(ctx, 0, reinterpret_cast<uint32_t*>(host), reinterpret_cast<uint32_t const*>(d_chain), level0 / sizeof(uint32_t));
+      if (err != cudaSuccess)
+        failed = fail_cuda("cudaMemcpyAsync(level 0)", err);
+    }
+
+    if (!failed)
+      failed = run_chain_float(ctx, format, width, height, levels, samples, d_chain, nullptr);
+
+    if (!failed && bytes > level0)
+    {
+      cudaError_t err = cudaMemcpyAsync(host + level0, d_chain + level0, bytes - level0, cudaMemcpyDeviceToHost, ctx->stream);
+      if (err != cudaSuccess)
+        failed = fail_cuda("cudaMemcpyAsync(levels)", err);
+    }
+
+    // also after a failure: nothing may stay in flight that reads or writes the caller's chain
+    cudaError_t err = cudaStreamSynchronize(ctx->stream);
+    cudaError_t err2 = send_level0 && ctx->copy_out ? cudaStreamSynchronize(ctx->copy_out) : cudaSuccess;
+    if (failed)
+      return 1;
+    if (err != cudaSuccess || err2 != cudaSuccess)
+      return fail_cuda(who, err != cudaSuccess ? err : err2);
+
+    if (!pinned && bytes > first)
+      copy_parallel(static_cast<unsigned char*>(chain) + first, host + first, bytes - first);
+
+    return 0;
+  }
+}
+
+namespace
+{
   // Level 0 is already in ctx->chain (six-image ingest, equirect pack): send it home at once — it travels
   // under the level-1 kernels — then the chain with every level following as soon as it is complete.
   // `bits` receives the whole payload; pageable payloads go through the pinned staging.
@@ -1759,8 +1807,6 @@ extern "C"
     if (!pinned && reserve_host_stage(ctx, bytes))
       return 1;
 
-    unsigned char *host = pinned ? static_cast<unsigned char*>(chain) : static_cast<unsigned char*>(ctx->host_stage);
-
     err = upload_host(ctx, ctx->staging.ptr, chain, level0, pinned, ctx->host_stage);
     if (err != cudaSuccess)
     {
@@ -1768,26 +1814,7 @@ extern "C"
       return fail_cuda("cudaMemcpyAsync(level 0)", err);
     }
 
-    int failed = run_chain_float(ctx, format, width, height, levels, samples, ctx->staging.ptr, nullptr);
-
-    if (!failed && bytes > level0)
-    {
-      err = cudaMemcpyAsync(host + level0, ctx->staging.ptr + level0, bytes - level0, cudaMemcpyDeviceToHost, ctx->stream);
-      if (err != cudaSuccess)
-        failed = fail_cuda("cudaMemcpyAsync(levels)", err);
-    }
-
-    // also after a failure: nothing may stay in flight that reads or writes the caller's chain
-    err = cudaStreamSynchronize(ctx->stream);
-    if (failed)
-      return 1;
-    if (err != cudaSuccess)
-      return fail_cuda("datum_ibl_buildmips_cube_float", err);
-
-    if (!pinned && bytes > level0)
-      copy_parallel(static_cast<unsigned char*>(chain) + level0, host + level0, bytes - level0);
-
-    return 0;
+    return finish_float_chain(ctx, format, width, height, levels, samples, ctx->staging.ptr, chain, pinned, false, "datum_ibl_buildmips_cube_float");
   }
 
   int datum_ibl_prefilter_level_float_device(datum_ibl_ctx *ctx, int format, void const *d_src, int ws, int hs, int level, int levels, int samples, int row_begin, int row_end, void *d_dst, float *d_dst_f32)
@@ -2179,7 +2206,9 @@ extern "C"
 
   // ---- equirect image -> cube (+ chain) -------------------------------------------------
 
-  static int pack_cube_to_device(datum_ibl_ctx *ctx, int imgwidth, int imgheight, float const *pixels, int width, int height, uint32_t *d_level0)
+  // equirect image (host) -> level 0 at d_level0, texels of `format` (rgbe or a float chain's); the image goes
+  // through ctx->staging, so d_level0 must not live there
+  static int pack_cube_to_device(datum_ibl_ctx *ctx, int format, int imgwidth, int imgheight, float const *pixels, int width, int height, void *d_level0)
   {
     size_t image_bytes = (size_t)imgwidth * imgheight * sizeof(float4);
 
@@ -2212,13 +2241,13 @@ extern "C"
       p.quats[f] = ctx->quats[f];
     p.dst = d_level0;
 
-    err = ibl::launch_equirect_resample(p, ctx->stream);
+    err = ibl::launch_equirect_resample(p, format, ctx->stream);
     if (err != cudaSuccess)
       return fail_cuda("equirect_resample", err);
     ctx->launches += 1;
 
     // tools/hdr.cpp:358 -> 322-327 with levels == 1: image_buildmips_rgbe does nothing, then the edge blend
-    err = ibl::launch_blend_edges(d_level0, width, height, ctx->stream);
+    err = ibl::launch_blend_edges(d_level0, format, width, height, ctx->stream);
     if (err != cudaSuccess)
       return fail_cuda("blend_edges", err);
     if (width > 1 && height > 1)
@@ -2242,7 +2271,7 @@ extern "C"
     if (err != cudaSuccess)
       return fail_cuda("cudaMalloc(chain)", err);
 
-    if (pack_cube_to_device(ctx, imgwidth, imgheight, pixels, width, height, ctx->chain.ptr))
+    if (pack_cube_to_device(ctx, ibl::kFormatRgbe, imgwidth, imgheight, pixels, width, height, ctx->chain.ptr))
       return 1;
 
     err = cudaMemcpyAsync(bits, ctx->chain.ptr, level0 * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream);
@@ -2271,18 +2300,103 @@ extern "C"
       return 1;
 
     // tools/ibl.cpp:285, 287
-    if (pack_cube_to_device(ctx, imgwidth, imgheight, pixels, width, height, ctx->chain.ptr))
+    if (pack_cube_to_device(ctx, ibl::kFormatRgbe, imgwidth, imgheight, pixels, width, height, ctx->chain.ptr))
       return 1;
 
     return finish_chain_to_host(ctx, width, height, levels, samples, bits, "datum_ibl_pack_cube_ibl");
+  }
+
+  // ---- equirect image or six ARGB32 images -> level 0 (+ chain) of a float chain -------------------------
+  //
+  // Level 0 is computed in the texels of the format (resample.cu), never as rgbe words.  Device buffers: the
+  // equirect image and the ARGB32 pixels go to ctx->staging (pack_cube_to_device, ingest_to_device), so the float
+  // chain cannot live there as it does in datum_ibl_buildmips_cube_float; it lives in ctx->chain, reserved in
+  // words (a float chain is a whole number of words: 8 or 16 bytes per texel).
+
+  namespace
+  {
+    int check_float_source(const char *who, int format, int width, int height, int levels, int samples, bool chain)
+    {
+      if (!float_format(format))
+        return fail(std::string(who) + ": unknown format " + std::to_string(format) + " (DATUM_IBL_FORMAT_F32 or DATUM_IBL_FORMAT_F16)");
+      if (chain && (!valid_chain(width, height, levels) || samples < 1 || samples > kFloatMaxSamples))
+        return fail(std::string(who) + ": bad width/height/levels/samples");
+      if (!chain && (width < 1 || height < 1))
+        return fail(std::string(who) + ": bad width/height");
+      return 0;
+    }
+
+    // device chain of `levels` levels of the format in ctx->chain
+    int reserve_float_chain(datum_ibl_ctx *ctx, int format, int width, int height, int levels, size_t *bytes)
+    {
+      *bytes = datum_ibl_chain_bytes(width, height, levels) / sizeof(uint32_t) * ibl::float_texel_bytes(format);
+      cudaError_t err = ctx->chain.reserve(*bytes / sizeof(uint32_t));
+      return err == cudaSuccess ? 0 : fail_cuda("cudaMalloc(chain)", err);
+    }
+
+    // level 0 in ctx->chain -> the caller's host buffer, synchronously
+    int level0_home(datum_ibl_ctx *ctx, void *texels, size_t bytes, const char *who)
+    {
+      cudaError_t err = cudaMemcpyAsync(texels, ctx->chain.ptr, bytes, cudaMemcpyDeviceToHost, ctx->stream);
+      if (err == cudaSuccess)
+        err = cudaStreamSynchronize(ctx->stream);
+      return err == cudaSuccess ? 0 : fail_cuda(who, err);
+    }
+  }
+
+  int datum_ibl_pack_cube_float(datum_ibl_ctx *ctx, int format, int imgwidth, int imgheight, float const *pixels, int width, int height, void *texels)
+  {
+    if (!ctx || !pixels || !texels)
+      return fail("datum_ibl_pack_cube_float: null argument");
+    if (imgwidth < 1 || imgheight < 1)
+      return fail("datum_ibl_pack_cube_float: bad image size");
+    if (check_float_source("datum_ibl_pack_cube_float", format, width, height, 1, 1, false))
+      return 1;
+
+    DeviceGuard guard(ctx->device);
+
+    size_t bytes = 0;
+    if (reserve_float_chain(ctx, format, width, height, 1, &bytes))
+      return 1;
+    if (pack_cube_to_device(ctx, format, imgwidth, imgheight, pixels, width, height, ctx->chain.ptr))
+      return 1;
+
+    return level0_home(ctx, texels, bytes, "datum_ibl_pack_cube_float");
+  }
+
+  int datum_ibl_pack_cube_float_ibl(datum_ibl_ctx *ctx, int format, int imgwidth, int imgheight, float const *pixels, int width, int height, int levels, int samples, void *chain)
+  {
+    if (!ctx || !pixels || !chain)
+      return fail("datum_ibl_pack_cube_float_ibl: null argument");
+    if (imgwidth < 1 || imgheight < 1)
+      return fail("datum_ibl_pack_cube_float_ibl: bad image size");
+    if (check_float_source("datum_ibl_pack_cube_float_ibl", format, width, height, levels, samples, true))
+      return 1;
+
+    DeviceGuard guard(ctx->device);
+
+    size_t bytes = 0;
+    if (reserve_float_chain(ctx, format, width, height, levels, &bytes))
+      return 1;
+
+    // the pinned staging carries the image up and, for a pageable chain, the chain down: reserved for the larger
+    // of the two before the upload uses it
+    const bool pinned = host_is_pinned(chain);
+    if (!pinned && reserve_host_stage(ctx, std::max(bytes, (size_t)imgwidth * imgheight * sizeof(float4))))
+      return 1;
+
+    if (pack_cube_to_device(ctx, format, imgwidth, imgheight, pixels, width, height, ctx->chain.ptr))
+      return 1;
+
+    return finish_float_chain(ctx, format, width, height, levels, samples, reinterpret_cast<unsigned char*>(ctx->chain.ptr), chain, pinned, true, "datum_ibl_pack_cube_float_ibl");
   }
 
   // ---- six ARGB32 face images -> level 0 (+ chain) -------------------------------------
 
   namespace
   {
-    // argb (host) -> ctx->chain level 0 on the context stream
-    int ingest_to_device(datum_ibl_ctx *ctx, int width, int height, uint32_t const *argb, uint32_t *d_level0)
+    // argb (host, through ctx->staging) -> level 0 at d_level0 in texels of `format`, on the context stream
+    int ingest_to_device(datum_ibl_ctx *ctx, int format, int width, int height, uint32_t const *argb, void *d_level0)
     {
       size_t level0 = (size_t)width * height * 6;
 
@@ -2319,7 +2433,7 @@ extern "C"
         return fail_cuda("cudaMemcpyAsync(argb)", err);
       }
 
-      err = ibl::launch_ingest_argb32((uint32_t const*)ctx->staging.ptr, ctx->srgb_lut.ptr, width, height, d_level0, ctx->sm_count, ctx->stream);
+      err = ibl::launch_ingest_argb32((uint32_t const*)ctx->staging.ptr, ctx->srgb_lut.ptr, width, height, format, d_level0, ctx->sm_count, ctx->stream);
       if (err != cudaSuccess)
         return fail_cuda("ingest_argb32", err);
       ctx->launches += 1;
@@ -2343,7 +2457,7 @@ extern "C"
     if (err != cudaSuccess)
       return fail_cuda("cudaMalloc(chain)", err);
 
-    if (ingest_to_device(ctx, width, height, argb, ctx->chain.ptr))
+    if (ingest_to_device(ctx, ibl::kFormatRgbe, width, height, argb, ctx->chain.ptr))
       return 1;
 
     err = cudaMemcpyAsync(bits, ctx->chain.ptr, level0 * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream);
@@ -2372,10 +2486,52 @@ extern "C"
       return 1;
 
     // tools/assetbuilder.cpp:443-462, then :465
-    if (ingest_to_device(ctx, width, height, argb, ctx->chain.ptr))
+    if (ingest_to_device(ctx, ibl::kFormatRgbe, width, height, argb, ctx->chain.ptr))
       return 1;
 
     return finish_chain_to_host(ctx, width, height, levels, samples, bits, "datum_ibl_ingest_cube_argb32_ibl");
+  }
+
+  int datum_ibl_ingest_cube_argb32_float(datum_ibl_ctx *ctx, int format, int width, int height, uint32_t const *argb, void *texels)
+  {
+    if (!ctx || !argb || !texels)
+      return fail("datum_ibl_ingest_cube_argb32_float: null argument");
+    if (check_float_source("datum_ibl_ingest_cube_argb32_float", format, width, height, 1, 1, false))
+      return 1;
+
+    DeviceGuard guard(ctx->device);
+
+    size_t bytes = 0;
+    if (reserve_float_chain(ctx, format, width, height, 1, &bytes))
+      return 1;
+    if (ingest_to_device(ctx, format, width, height, argb, ctx->chain.ptr))
+      return 1;
+
+    return level0_home(ctx, texels, bytes, "datum_ibl_ingest_cube_argb32_float");
+  }
+
+  int datum_ibl_ingest_cube_argb32_float_ibl(datum_ibl_ctx *ctx, int format, int width, int height, int levels, int samples, uint32_t const *argb, void *chain)
+  {
+    if (!ctx || !argb || !chain)
+      return fail("datum_ibl_ingest_cube_argb32_float_ibl: null argument");
+    if (check_float_source("datum_ibl_ingest_cube_argb32_float_ibl", format, width, height, levels, samples, true))
+      return 1;
+
+    DeviceGuard guard(ctx->device);
+
+    size_t bytes = 0;
+    if (reserve_float_chain(ctx, format, width, height, levels, &bytes))
+      return 1;
+
+    // the float chain is at least four times the ARGB32 pixels: reserving for it covers the upload too
+    const bool pinned = host_is_pinned(chain);
+    if (!pinned && reserve_host_stage(ctx, bytes))
+      return 1;
+
+    if (ingest_to_device(ctx, format, width, height, argb, ctx->chain.ptr))
+      return 1;
+
+    return finish_float_chain(ctx, format, width, height, levels, samples, reinterpret_cast<unsigned char*>(ctx->chain.ptr), chain, pinned, true, "datum_ibl_ingest_cube_argb32_float_ibl");
   }
 
   // ---- LUTs -----------------------------------------------------------------------

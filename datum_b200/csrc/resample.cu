@@ -9,8 +9,13 @@
 // the loops are reproduced with exactly-rounded adds (no FMA contraction).  The
 // stage is a gather over an image that fits L2 for typical inputs; it is <1 % of
 // the bake and is not tuned further.
+//
+// Every kernel here has one body and a texel policy (RgbeTexel, F32Texel, F16Texel)
+// that says how a texel of level 0 is stored and read back.  The rgbe instantiations
+// are the reference's arithmetic; the float ones swap rgbe() for the format's store.
 
 #include "resample.h"
+#include "prefilter_f.h"
 
 #include <cuda_runtime.h>
 
@@ -18,6 +23,37 @@ namespace ibl
 {
   namespace
   {
+    // ---- texel policies: encode rgb into the stored texel (alpha 1.0), decode it back ----
+
+    struct RgbeTexel
+    {
+      typedef uint32_t Word;
+      static __device__ __forceinline__ Word encode(float r, float g, float b) { return rgbe_encode(r, g, b); }
+      static __device__ __forceinline__ void decode(Word w, float &r, float &g, float &b) { rgbe_decode(w, r, g, b); }
+    };
+
+    struct F32Texel
+    {
+      typedef float4 Word;
+      static __device__ __forceinline__ Word encode(float r, float g, float b) { return make_float4(r, g, b, 1.0f); }
+      static __device__ __forceinline__ void decode(Word w, float &r, float &g, float &b) { r = w.x; g = w.y; b = w.z; }
+    };
+
+    // RGBA16F as two words (g<<16 | r, a<<16 | b), the layout of the float chains (prefilter_f.h, F16Record)
+    struct F16Texel
+    {
+      typedef uint2 Word;
+      static __device__ __forceinline__ Word encode(float r, float g, float b)
+      {
+        uint32_t hr = float_to_half_rn(r), hg = float_to_half_rn(g), hb = float_to_half_rn(b);
+        return make_uint2(hg << 16 | hr, 0x3C00u << 16 | hb);
+      }
+      static __device__ __forceinline__ void decode(Word w, float &r, float &g, float &b)
+      {
+        r = half_to_float(w.x & 0xFFFFu); g = half_to_float(w.x >> 16); b = half_to_float(w.y & 0xFFFFu);
+      }
+    };
+
     struct Rgba { float r, g, b, a; };
 
     __device__ __forceinline__ Rgba lerp_rn(Rgba x, Rgba y, float t)
@@ -54,6 +90,7 @@ namespace ibl
     }
   }
 
+  template<typename Texel>
   __global__ void __launch_bounds__(256) equirect_resample_kernel(ResampleParams p)
   {
     size_t total = (size_t)6 * p.width * p.height;
@@ -91,14 +128,16 @@ namespace ibl
       }
     }
 
-    p.dst[idx] = rgbe_encode(div_rn(sum.r, totalweight), div_rn(sum.g, totalweight), div_rn(sum.b, totalweight));
+    static_cast<typename Texel::Word*>(p.dst)[idx] = Texel::encode(div_rn(sum.r, totalweight), div_rn(sum.g, totalweight), div_rn(sum.b, totalweight));
   }
 
   // ---- edge blend --------------------------------------------------------------------
   //
   // One CTA walks the reference's twelve loops in order; texel k of a loop is
   // independent of the other k (hdr.cpp:181-311), later loops read what earlier
-  // loops wrote (the corner texels), hence the barrier between loops.
+  // loops wrote (the corner texels), hence the barrier between loops.  Every loop
+  // reads the texels as stored and stores its results in the format, so a corner
+  // is re-encoded (rgbe) or re-rounded (F16) once per loop that writes it.
 
   namespace
   {
@@ -114,19 +153,21 @@ namespace ibl
       short count; // 0: h, 1: w, 2: min(w, h)
     };
 
-    __device__ __forceinline__ uint32_t blend3(uint32_t a, uint32_t b, uint32_t c)
+    template<typename Texel>
+    __device__ __forceinline__ typename Texel::Word blend3(typename Texel::Word a, typename Texel::Word b, typename Texel::Word c)
     {
       float ar, ag, ab, br, bg, bb, cr, cg, cb;
-      rgbe_decode(a, ar, ag, ab);
-      rgbe_decode(b, br, bg, bb);
-      rgbe_decode(c, cr, cg, cb);
-      return rgbe_encode(add_rn(add_rn(mul_rn(0.3f, ar), mul_rn(0.4f, br)), mul_rn(0.3f, cr)),
+      Texel::decode(a, ar, ag, ab);
+      Texel::decode(b, br, bg, bb);
+      Texel::decode(c, cr, cg, cb);
+      return Texel::encode(add_rn(add_rn(mul_rn(0.3f, ar), mul_rn(0.4f, br)), mul_rn(0.3f, cr)),
                          add_rn(add_rn(mul_rn(0.3f, ag), mul_rn(0.4f, bg)), mul_rn(0.3f, cg)),
                          add_rn(add_rn(mul_rn(0.3f, ab), mul_rn(0.4f, bb)), mul_rn(0.3f, cb)));
     }
   }
 
-  __global__ void __launch_bounds__(1024) blend_edges_kernel(uint32_t *img, int w, int h)
+  template<typename Texel>
+  __global__ void __launch_bounds__(1024) blend_edges_kernel(typename Texel::Word *img, int w, int h)
   {
     // W = w-1, H = h-1 written symbolically: base codes 0 -> 0, 1 -> 1, 2 -> w-2, 3 -> w-1, 4 -> h-2, 5 -> h-1
     // each entry: {a, b, c, d} as (xcode, ycode, dx, dy), faces, count kind
@@ -170,36 +211,52 @@ namespace ibl
         size_t ic = ((size_t)e.fb * h + (base[e.cy] + k * e.cdy)) * w + (base[e.cx] + k * e.cdx);
         size_t id = ((size_t)e.fb * h + (base[e.dy] + k * e.ddy)) * w + (base[e.dx] + k * e.ddx);
 
-        uint32_t a = img[ia], b = img[ib], c = img[ic], d = img[id];
+        typename Texel::Word a = img[ia], b = img[ib], c = img[ic], d = img[id];
 
-        img[ib] = blend3(a, b, c);
-        img[ic] = blend3(b, c, d);
+        img[ib] = blend3<Texel>(a, b, c);
+        img[ic] = blend3<Texel>(b, c, d);
       }
 
       __syncthreads();
     }
   }
 
-  cudaError_t launch_equirect_resample(ResampleParams const &p, cudaStream_t stream)
+  cudaError_t launch_equirect_resample(ResampleParams const &p, int format, cudaStream_t stream)
   {
     size_t total = (size_t)6 * p.width * p.height;
-    equirect_resample_kernel<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(p);
+    unsigned grid = (unsigned)((total + 255) / 256);
+    if (format == kFormatRgbe)
+      equirect_resample_kernel<RgbeTexel><<<grid, 256, 0, stream>>>(p);
+    else if (format == kFloatFormatF32)
+      equirect_resample_kernel<F32Texel><<<grid, 256, 0, stream>>>(p);
+    else if (format == kFloatFormatF16)
+      equirect_resample_kernel<F16Texel><<<grid, 256, 0, stream>>>(p);
+    else
+      return cudaErrorInvalidValue;
     return cudaGetLastError();
   }
 
-  cudaError_t launch_blend_edges(uint32_t *level, int width, int height, cudaStream_t stream)
+  cudaError_t launch_blend_edges(void *level, int format, int width, int height, cudaStream_t stream)
   {
     // hdr.cpp:177: levels narrower than 2 texels are left alone
     if (width <= 1 || height <= 1)
       return cudaSuccess;
 
-    blend_edges_kernel<<<1, 1024, 0, stream>>>(level, width, height);
+    if (format == kFormatRgbe)
+      blend_edges_kernel<RgbeTexel><<<1, 1024, 0, stream>>>(static_cast<uint32_t*>(level), width, height);
+    else if (format == kFloatFormatF32)
+      blend_edges_kernel<F32Texel><<<1, 1024, 0, stream>>>(static_cast<float4*>(level), width, height);
+    else if (format == kFloatFormatF16)
+      blend_edges_kernel<F16Texel><<<1, 1024, 0, stream>>>(static_cast<uint2*>(level), width, height);
+    else
+      return cudaErrorInvalidValue;
     return cudaGetLastError();
   }
 
-  // ---- six ARGB32 images -> rgbe level 0 (tools/assetbuilder.cpp:443-462) ----
+  // ---- six ARGB32 images -> level 0 (tools/assetbuilder.cpp:443-462) ----
 
-  __global__ void __launch_bounds__(256) ingest_argb32_kernel(uint32_t const *__restrict__ argb, float const *__restrict__ lut, int width, int height, uint32_t *__restrict__ dst)
+  template<typename Texel>
+  __global__ void __launch_bounds__(256) ingest_argb32_kernel(uint32_t const *__restrict__ argb, float const *__restrict__ lut, int width, int height, typename Texel::Word *__restrict__ dst)
   {
     __shared__ float s_lut[256];
     s_lut[threadIdx.x] = __ldg(lut + threadIdx.x);
@@ -222,11 +279,11 @@ namespace ibl
       float b = s_lut[px & 0xFFu];
 
       // image.mirrored(): vertical flip (assetbuilder.cpp:458)
-      dst[face * face_size + (size_t)(height - 1 - y) * width + x] = rgbe_encode(r, g, b);
+      dst[face * face_size + (size_t)(height - 1 - y) * width + x] = Texel::encode(r, g, b);
     }
   }
 
-  cudaError_t launch_ingest_argb32(uint32_t const *argb, float const *lut, int width, int height, uint32_t *dst, int sm_count, cudaStream_t stream)
+  cudaError_t launch_ingest_argb32(uint32_t const *argb, float const *lut, int width, int height, int format, void *dst, int sm_count, cudaStream_t stream)
   {
     size_t total = (size_t)6 * width * height;
     size_t blocks = (total + 255) / 256;
@@ -235,7 +292,14 @@ namespace ibl
     if (grid < 1)
       grid = 1;
 
-    ingest_argb32_kernel<<<grid, 256, 0, stream>>>(argb, lut, width, height, dst);
+    if (format == kFormatRgbe)
+      ingest_argb32_kernel<RgbeTexel><<<grid, 256, 0, stream>>>(argb, lut, width, height, static_cast<uint32_t*>(dst));
+    else if (format == kFloatFormatF32)
+      ingest_argb32_kernel<F32Texel><<<grid, 256, 0, stream>>>(argb, lut, width, height, static_cast<float4*>(dst));
+    else if (format == kFloatFormatF16)
+      ingest_argb32_kernel<F16Texel><<<grid, 256, 0, stream>>>(argb, lut, width, height, static_cast<uint2*>(dst));
+    else
+      return cudaErrorInvalidValue;
 
     return cudaGetLastError();
   }

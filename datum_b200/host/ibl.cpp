@@ -19,6 +19,7 @@
 #ifdef DATUM_IBL_IN_REFERENCE_TREE
 void image_project_sh9_cube(int width, int height, void const *level0_rgbe, float *sh);
 void image_pack_cube_faces_ibl(unsigned int const *argb, int width, int height, int levels, void *bits);
+void image_pack_cube_float_ibl(HDRImage const &image, int width, int height, int levels, int format, void *chain);
 void image_set_ibl_samples(int samples);
 void image_buildmips_cube_ibl_batch(int count, int width, int height, int levels, void *const *bits, float *sh);
 void image_pack_irradiance_sh9(int width, int height, void const *level0_rgbe, void *bits);
@@ -150,6 +151,11 @@ void image_project_sh9_cube(int width, int height, void const *level0_rgbe, floa
 void image_pack_cube_faces_ibl(unsigned int const *argb, int width, int height, int levels, void *bits)
 {
   check(datum_ibl_ingest_cube_argb32_ibl(context(), width, height, levels, g_samples, argb, bits));
+}
+
+void image_pack_cube_float_ibl(HDRImage const &image, int width, int height, int levels, int format, void *chain)
+{
+  check(datum_ibl_pack_cube_float_ibl(context(), format, image.width, image.height, &image.bits[0].r, width, height, levels, g_samples, chain));
 }
 
 void image_buildmips_cube_ibl_batch(int count, int width, int height, int levels, void *const *bits, float *sh)

@@ -37,6 +37,12 @@ void image_pack_irradiance_cube(void const *sh9_bits, int width, int height, voi
 // convertToFormat, :445) in the caller's face order; per pixel rgbe(srgba(pixel)),
 // vertical mirror, then the prefilter chain.  `bits` = the whole payload.
 void image_pack_cube_faces_ibl(unsigned int const *argb, int width, int height, int levels, void *bits);
+
+// The .hdr flow of write_skybox_asset (tools/assetbuilder.cpp:473-491) producing a float probe: the resample
+// and edge blend of image_pack_cube_ibl with level 0 stored as RGBA32F or RGBA16F texels (`format` =
+// DATUM_IBL_FORMAT_F32 or DATUM_IBL_FORMAT_F16) instead of rgbe, then the float prefilter chain
+// (datum_ibl_pack_cube_float_ibl).  `chain` = the whole chain, 16 or 8 bytes per texel, levels of the payload.
+void image_pack_cube_float_ibl(HDRImage const &image, int width, int height, int levels, int format, void *chain);
 void image_set_ibl_samples(int samples);
 
 // `count` image_buildmips_cube_ibl calls as one: payloads of the same width/height/levels, their

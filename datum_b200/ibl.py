@@ -123,6 +123,28 @@ def _host_pointer(buf, min_bytes, what):
     raise TypeError("%s must be a numpy array or a torch tensor" % what)
 
 
+def _float_host_buffer(fmt, buf, texels, what):
+    """Address of a host buffer of `texels` texels of float format `fmt`, checked for dtype and size."""
+    if hasattr(buf, "is_cuda") and buf.is_cuda:
+        raise ValueError("%s must be a host buffer" % what)
+    _check_dtype(buf, _float_dtype(fmt), what)
+    return _host_pointer(buf, texels * _texel_bytes(fmt), what)
+
+
+def _equirect_image(image):
+    image = np.ascontiguousarray(image, dtype=np.float32)
+    if image.ndim != 3 or image.shape[2] != 4:
+        raise ValueError("image must be (H, W, 4) float32")
+    return image
+
+
+def _face_images(faces):
+    faces = np.ascontiguousarray(faces, dtype=np.uint32)
+    if faces.ndim != 3 or faces.shape[0] != 6:
+        raise ValueError("faces must be (6, H, W) uint32")
+    return faces
+
+
 def _device_pointer(t, min_bytes, what, device):
     if t is None:
         return None
@@ -454,9 +476,7 @@ class IblContext:
         fn = getattr(self._lib, "datum_ibl_pack_cube_ibl", None)
         if fn is None:
             raise IblError("libdatum_ibl_cuda was built without the equirect resample stage")
-        image = np.ascontiguousarray(image, dtype=np.float32)
-        if image.ndim != 3 or image.shape[2] != 4:
-            raise ValueError("image must be (H, W, 4) float32")
+        image = _equirect_image(image)
         ptr = _host_pointer(bits, image_datasize(width, height, 6, levels), "bits")
         self._check(fn(self._handle, image.shape[1], image.shape[0], image.ctypes.data, width, height, levels, samples, ptr))
 
@@ -465,9 +485,7 @@ class IblContext:
         fn = getattr(self._lib, "datum_ibl_pack_cube", None)
         if fn is None:
             raise IblError("libdatum_ibl_cuda was built without the equirect resample stage")
-        image = np.ascontiguousarray(image, dtype=np.float32)
-        if image.ndim != 3 or image.shape[2] != 4:
-            raise ValueError("image must be (H, W, 4) float32")
+        image = _equirect_image(image)
         ptr = _host_pointer(bits, width * height * 6 * 4, "bits")
         self._check(fn(self._handle, image.shape[1], image.shape[0], image.ctypes.data, width, height, ptr))
 
@@ -478,21 +496,52 @@ class IblContext:
         """The per-image loop of write_skybox_asset(fout, id, paths) (assetbuilder.cpp:443-462).
         `faces` is a (6, H, W) uint32 array of QImage::Format_ARGB32 pixels (0xAARRGGBB) in the
         caller's face order; `bits` receives level 0 (6*W*H rgbe words)."""
-        faces = np.ascontiguousarray(faces, dtype=np.uint32)
-        if faces.ndim != 3 or faces.shape[0] != 6:
-            raise ValueError("faces must be (6, H, W) uint32")
+        faces = _face_images(faces)
         height, width = faces.shape[1], faces.shape[2]
         ptr = _host_pointer(bits, width * height * 6 * 4, "bits")
         self._check(self._lib.datum_ibl_ingest_cube_argb32(self._handle, width, height, faces.ctypes.data, ptr))
 
     def skybox_from_argb32(self, faces, levels, bits, samples=1024):
         """assetbuilder.cpp:443-465: ingest + image_buildmips_cube_ibl, level 0 staying on the device."""
-        faces = np.ascontiguousarray(faces, dtype=np.uint32)
-        if faces.ndim != 3 or faces.shape[0] != 6:
-            raise ValueError("faces must be (6, H, W) uint32")
+        faces = _face_images(faces)
         height, width = faces.shape[1], faces.shape[2]
         ptr = _host_pointer(bits, image_datasize(width, height, 6, levels), "bits")
         self._check(self._lib.datum_ibl_ingest_cube_argb32_ibl(self._handle, width, height, levels, samples, faces.ctypes.data, ptr))
+
+    # ---- equirect HDR image or six ARGB32 face images -> float chain (RGBA32F / RGBA16F) ----
+
+    def pack_cube_float(self, fmt, image, width, height, out):
+        """Level 0 of a float chain from an (H, W, 4) float32 equirect image (HDRImage::bits): the resample and
+        edge blend of image_pack_cube with the format's texel stored in place of rgbe (F32: the fp32 rgb, F16:
+        min(x, 65504) rounded to nearest-even, alpha 1.0).  `out`: numpy array or CPU tensor of the format's
+        dtype holding 6*width*height texels.  Pixel rgb must be finite and non-negative (F32: below 2^52).
+        Synchronous."""
+        image = _equirect_image(image)
+        ptr = _float_host_buffer(fmt, out, 6 * width * height, "out")
+        self._check(self._lib.datum_ibl_pack_cube_float(self._handle, fmt, image.shape[1], image.shape[0], image.ctypes.data, width, height, ptr))
+
+    def pack_cube_float_ibl(self, fmt, image, width, height, levels, chain, samples=1024):
+        """pack_cube_float followed by buildmips_cube_float, level 0 staying on the device: `chain` (host, the
+        layout of buildmips_cube_float) receives every level, level 0 included.  Synchronous."""
+        image = _equirect_image(image)
+        ptr = _float_host_buffer(fmt, chain, float_chain_texels(width, height, levels), "chain")
+        self._check(self._lib.datum_ibl_pack_cube_float_ibl(self._handle, fmt, image.shape[1], image.shape[0], image.ctypes.data, width, height, levels, samples, ptr))
+
+    def ingest_cube_argb32_float(self, fmt, faces, out):
+        """ingest_cube_argb32 with level 0 stored in the float format: per pixel the linear rgb of srgba(pixel),
+        alpha 1.0, rows mirrored.  `faces` is (6, H, W) uint32; `out` holds 6*W*H texels of the format's dtype."""
+        faces = _face_images(faces)
+        height, width = faces.shape[1], faces.shape[2]
+        ptr = _float_host_buffer(fmt, out, 6 * width * height, "out")
+        self._check(self._lib.datum_ibl_ingest_cube_argb32_float(self._handle, fmt, width, height, faces.ctypes.data, ptr))
+
+    def skybox_float_from_argb32(self, fmt, faces, levels, chain, samples=1024):
+        """ingest_cube_argb32_float followed by buildmips_cube_float, level 0 staying on the device: `chain`
+        receives every level.  Synchronous."""
+        faces = _face_images(faces)
+        height, width = faces.shape[1], faces.shape[2]
+        ptr = _float_host_buffer(fmt, chain, float_chain_texels(width, height, levels), "chain")
+        self._check(self._lib.datum_ibl_ingest_cube_argb32_float_ibl(self._handle, fmt, width, height, levels, samples, faces.ctypes.data, ptr))
 
 
 class MultiContext:

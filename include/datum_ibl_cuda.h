@@ -353,6 +353,41 @@ int datum_ibl_prefilter_level_float_peers(datum_ibl_ctx *ctx, int format, void c
  */
 int datum_ibl_multi_buildmips_cube_float(datum_ibl_multi *multi, int format, int width, int height, int levels, int samples, void *chain);
 
+/* ---- equirect HDR image or six face images -> level 0 (+ chain) of a float chain ---------------- */
+
+/*
+ * datum_ibl_pack_cube with level 0 stored in `format` (DATUM_IBL_FORMAT_F32 or DATUM_IBL_FORMAT_F16) instead of
+ * rgbe words.  Per cube texel the arithmetic of the rgbe resample up to sum / totalweight (the same box of
+ * bilinear taps, fp32 loop counters), then the format's texel: F32 stores the fp32 rgb, F16 stores min(x, 65504)
+ * rounded to nearest-even; alpha is 1.0.  The edge blend then runs the reference's twelve loops in order with the
+ * same 0.3/0.4/0.3 arithmetic; each loop reads the texels as stored (halves widened, corners written by earlier
+ * loops included) and stores its results in the format, so an F16 corner is rounded once per loop that writes
+ * it, as an rgbe corner is re-encoded.  Pixel rgb must be finite and non-negative, and below 2^52 for F32 (the
+ * level-0 rules of datum_ibl_buildmips_cube_float; not checked); F16 clamps texels above 65504.  `pixels` =
+ * imgwidth*imgheight RGBA fp32 on the host; `texels` receives the 6*width*height texels of level 0 (host,
+ * pageable or pinned).  Synchronous.
+ */
+int datum_ibl_pack_cube_float(datum_ibl_ctx *ctx, int format, int imgwidth, int imgheight, float const *pixels, int width, int height, void *texels);
+
+/*
+ * The level 0 above followed by the chain of datum_ibl_buildmips_cube_float, level 0 never leaving the device in
+ * between.  `chain` (host, pageable or pinned) receives the whole chain, level 0 included, in the layout of
+ * datum_ibl_buildmips_cube_float; its levels >= 1 are those datum_ibl_buildmips_cube_float makes from that
+ * level 0.  `samples` 1..4096.  Synchronous.
+ */
+int datum_ibl_pack_cube_float_ibl(datum_ibl_ctx *ctx, int format, int imgwidth, int imgheight, float const *pixels, int width, int height, int levels, int samples, void *chain);
+
+/*
+ * datum_ibl_ingest_cube_argb32 with level 0 stored in `format`: per pixel the linear rgb of srgba(pixel)
+ * (pow(c/255, 2.2f), the same 256 values the rgbe ingest encodes) stored as F32 or F16 texels with alpha 1.0,
+ * rows mirrored vertically, faces in argument order.  `texels` receives 6*width*height texels (host, pageable
+ * or pinned).  Synchronous.
+ */
+int datum_ibl_ingest_cube_argb32_float(datum_ibl_ctx *ctx, int format, int width, int height, uint32_t const *argb, void *texels);
+
+/* The ingest above followed by the chain of datum_ibl_buildmips_cube_float, as datum_ibl_pack_cube_float_ibl. */
+int datum_ibl_ingest_cube_argb32_float_ibl(datum_ibl_ctx *ctx, int format, int width, int height, int levels, int samples, uint32_t const *argb, void *chain);
+
 #ifdef __cplusplus
 }
 #endif
